@@ -7,7 +7,10 @@ collective).  One step = one scoring pass over one batch.  `value` is timed with
 inputs already resident in HBM; `e2e` goes through the Python API with pinned host buffers
 (H2D of audio + encoding and D2H of the log-likelihood inside the timed region).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--workload ...] [--dump-outputs DIR]
+
+--dump-outputs DIR writes what the last timed step returned (rank 0) as DIR/<name>.npy, so that two builds run with
+the same arguments, and therefore the same seeded inputs, can be compared output for output.
 """
 import argparse
 import json
@@ -33,6 +36,7 @@ BYTES_PER_SAMPLE_ENC_LAYER = 512      # encoder layer launch: 16-bit image of re
 FLOP_PER_SAMPLE_ENC = 2949632         # GEMMs the encoder executes: 33280 (nc_conv) + 30*65536 (K=2 convs) + 29*32768 (1x1 residuals)
 METRIC = "audio samples/sec"
 UNIT = "samples/s"
+DUMP_LIMIT_BYTES = 64 * 10 ** 6       # all files of one --dump-outputs, headers included
 
 
 def load_peaks():
@@ -242,10 +246,30 @@ def run_reference(args, rank, world):
     print(json.dumps(line), flush=True)
 
 
+def dump_outputs(out_dir, arrays, limit=DUMP_LIMIT_BYTES):
+    """Writes name -> array (NumPy or torch) as out_dir/<name>.npy: float64 stays float64, everything else becomes
+    float32.  Each array gets an equal share of ``limit``; one larger than its share is replaced by a sample of its
+    flattened elements, drawn with a fixed seed and kept in index order, so equal shapes give the same sample."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    share = limit // len(arrays) - 4096            # room for the .npy header
+    for name, a in arrays.items():
+        if hasattr(a, "detach"):
+            a = a.detach().cpu().numpy()
+        a = np.asarray(a)
+        a = a.astype(np.float64 if a.dtype == np.float64 else np.float32)
+        if a.nbytes > share:
+            idx = np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False)
+            a = a.reshape(-1)[np.sort(idx)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=20)
+    ap.add_argument("--steps", type=int, default=20,
+                    help="timed steps of the workload (the `also` block times its extra configurations with a fixed "
+                         "3 steps, 2 for generation)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="teacher_nll", choices=["teacher_nll", "student", "generate", "distill", "encode"])
@@ -254,7 +278,12 @@ def main():
     ap.add_argument("--length", type=int, default=0)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-also", action="store_true", help="skip the extra configurations of the `also` block")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -368,7 +397,7 @@ def main():
     for a, b in ev:
         flush.fill_(1)                      # L2 flush between timed iterations (not timed)
         a.record()
-        step_device()
+        out = step_device()
         b.record()
         if args.workload == "encode":
             km, kern_launches, kern_name = model._enc_eng.last_ms(), len(dil) + 1, "enc::k_enc_layer"
@@ -383,6 +412,11 @@ def main():
     partition = list(model._eng.last_partition()) if args.workload in ("teacher_nll", "student") and prec == "fp16" else None
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = sum(step_ms)
+    if args.dump_outputs and rank == 0:
+        names = {"teacher_nll": ("nll",), "student": ("out",), "generate": ("audio",), "encode": ("encoding",),
+                 "distill": ("loss", "power_loss")}[args.workload]
+        dump_outputs(args.dump_outputs, dict(zip(names, out if isinstance(out, tuple) else (out,))))
+    del out
     shard.barrier()
 
     # end to end through the public API with pinned host buffers

@@ -1,12 +1,13 @@
 """Writes tests/golden/reference_*.npz by EXECUTING the reference's own ops.py / model.py (imported unmodified
-from /root/reference on top of the NumPy TensorFlow stand-in, tests/tf_shim) in float64 on seeded inputs.
+from a checkout of tachitachi/SR-WaveNet on top of the NumPy TensorFlow stand-in, tests/tf_shim) in float64 on
+seeded inputs.
 
 These are outputs of the reference's code path (its graph construction, operation order, variable naming), not of
-the oracle; the per-operation TensorFlow semantics are the stand-in's (see its docstring).  /root/reference does not
-travel to the GPU box, the fixtures do: tests/test_oracle_golden.py holds the oracle to them and
+the oracle; the per-operation TensorFlow semantics are the stand-in's (see its docstring).  The reference is not part
+of this repository, the fixtures are: tests/test_oracle_golden.py holds the oracle to them and
 tests/test_gpu_reference_golden.py the CUDA path.
 
-Run from the repo root in the build container:  python tests/golden/make_reference_golden.py
+Run from the repo root:  SRWN_REFERENCE_DIR=<reference checkout> python tests/golden/make_reference_golden.py
 """
 import os
 import sys
@@ -77,6 +78,6 @@ def make(tag, dil, B, T, P, C, F, M=5, ar_T=0, seeds=(42, 43)):
 
 
 if __name__ == '__main__':
-    assert refshim.available(), 'needs /root/reference'
+    assert refshim.available(), 'set SRWN_REFERENCE_DIR to a checkout of the reference'
     make('small', [1, 2, 4, 1, 2, 4], B=2, T=1024, P=16, C=8, F=2, ar_T=64, seeds=(11, 12))
     make('default', synth.DEFAULT_DILATIONS, B=2, T=1024, P=128, C=32, F=4)               # teacher.py:55-62

@@ -1,9 +1,9 @@
 """Writes tests/golden/reference_heads.npz by EXECUTING the reference's WaveNet (model.py:8-72) and SiameseWaveNet
-(model.py:660-798) classes, imported unmodified from /root/reference on top of the NumPy TensorFlow stand-in
-(tests/tf_shim), in float64 on seeded weights and inputs.  The fixture travels to the GPU box
-(tests/test_gpu_heads.py); tests/test_heads.py re-derives it here when /root/reference is present.
+(model.py:660-798) classes, imported unmodified from a checkout of tachitachi/SR-WaveNet on top of the NumPy
+TensorFlow stand-in (tests/tf_shim), in float64 on seeded weights and inputs.  The CUDA path is held to the fixture
+(tests/test_gpu_heads.py); tests/test_heads.py re-derives it when SRWN_REFERENCE_DIR names the checkout.
 
-Run from the repo root in the build container:  python tests/golden/make_reference_heads_golden.py
+Run from the repo root:  SRWN_REFERENCE_DIR=<reference checkout> python tests/golden/make_reference_heads_golden.py
 """
 import os
 import sys

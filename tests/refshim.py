@@ -1,7 +1,8 @@
-"""Loads the reference's own ops.py / model.py (UNMODIFIED, from /root/reference) on top of the NumPy
-TensorFlow stand-in in tests/tf_shim.  Test infrastructure; used by tests/test_reference_shim.py and
-tests/golden/make_reference_golden.py.  /root/reference exists only in the build container, so callers
-skip when ``available()`` is False (the GPU box gets the committed fixtures instead)."""
+"""Loads the reference's own ops.py / model.py (UNMODIFIED, from a checkout of tachitachi/SR-WaveNet named by the
+environment variable SRWN_REFERENCE_DIR) on top of the NumPy TensorFlow stand-in in tests/tf_shim.  Test
+infrastructure; used by tests/test_reference_shim.py and tests/golden/make_reference_*golden.py.  The reference is
+not part of this repository, so callers skip when ``available()`` is False; the committed fixtures
+tests/golden/reference_*.npz hold what it computed."""
 import contextlib
 import importlib
 import io
@@ -9,12 +10,13 @@ import os
 import sys
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REFERENCE = os.environ.get('SRWN_REFERENCE_DIR', '/root/reference')
+REFERENCE = os.environ.get('SRWN_REFERENCE_DIR', '')
 SHIM = os.path.join(HERE, 'tf_shim')
 
 
 def available():
-    return os.path.exists(os.path.join(REFERENCE, 'ops.py')) and os.path.exists(os.path.join(REFERENCE, 'model.py'))
+    return bool(REFERENCE) and os.path.exists(os.path.join(REFERENCE, 'ops.py')) and \
+        os.path.exists(os.path.join(REFERENCE, 'model.py'))
 
 
 _loaded = {}

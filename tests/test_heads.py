@@ -1,6 +1,6 @@
 """CPU side of the WaveNet / SiameseWaveNet heads (model.py:8-72, 660-798): the variable names and shapes this build creates
 are the ones the reference's graph creates (checked against the fixture, and against the reference itself when
-/root/reference is present), and the committed fixture is what the reference's source produces today."""
+SRWN_REFERENCE_DIR names a checkout of it), and the committed fixture is what the reference's source produces today."""
 import os
 import sys
 
@@ -55,7 +55,7 @@ def test_train_is_refused_loudly():
 def test_fixture_is_what_the_reference_produces():
     import refshim
     if not refshim.available():
-        pytest.skip("/root/reference is not present")
+        pytest.skip("SRWN_REFERENCE_DIR does not name a reference checkout")
     sys.path.insert(0, GOLDEN)
     import make_reference_heads_golden as mk
     fresh, g = mk.compute(), _fixture()
