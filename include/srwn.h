@@ -103,7 +103,7 @@ int srwn_set_weight(srwn_handle_t h, const char* name, const float* data,
  * with room for `count` floats. */
 int srwn_get_weight(srwn_handle_t h, const char* name, float* data, int64_t count);
 /* Checks that every live variable was set and builds the packed operand images the
- * kernels read (bf16 UMMA layouts, summed skip bias). Must follow any srwn_set_weight. */
+ * kernels read (fp16 UMMA layouts, summed skip bias). Must follow any srwn_set_weight. */
 int srwn_commit_weights(srwn_handle_t h, void* stream);
 
 /* Synchronises `stream` and reports whether the last fused-kernel call that used this workspace

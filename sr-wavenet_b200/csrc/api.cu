@@ -488,8 +488,8 @@ extern "C" int srwn_teacher_logits(srwn_handle_t h, const float* x, const float*
   if (rc) return rc;
   if (precision == SRWN_BF16) return reject_bf16();
   if (precision == SRWN_FP16)
-    return run_teacher_fused_bf16(h, x, enc, nullptr, nullptr, nullptr, logits, B, T,
-                                  precision == SRWN_FP16, workspace, workspace_bytes, (cudaStream_t)stream);
+    return run_teacher_fused(h, x, enc, nullptr, nullptr, nullptr, logits, B, T,
+                             workspace, workspace_bytes, (cudaStream_t)stream);
   if (precision != SRWN_FP32) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
   F32Ws w = carve_f32(h, SRWN_OP_TEACHER_LOGITS, B, T, workspace, workspace_bytes, false);
   if (!workspace || w.bytes > workspace_bytes)
@@ -507,8 +507,8 @@ extern "C" int srwn_teacher_nll(srwn_handle_t h, const float* x_in, const float*
   if (rc) return rc;
   if (precision == SRWN_BF16) return reject_bf16();
   if (precision == SRWN_FP16)
-    return run_teacher_fused_bf16(h, x_in, enc, x_scored, nll_out, nll_sum, logits_out, B, T,
-                                  precision == SRWN_FP16, workspace, workspace_bytes, (cudaStream_t)stream);
+    return run_teacher_fused(h, x_in, enc, x_scored, nll_out, nll_sum, logits_out, B, T,
+                             workspace, workspace_bytes, (cudaStream_t)stream);
   if (precision != SRWN_FP32) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
   F32Ws w = carve_f32(h, SRWN_OP_TEACHER_NLL, B, T, workspace, workspace_bytes, logits_out == nullptr);
   if (!workspace || w.bytes > workspace_bytes)
@@ -545,7 +545,7 @@ static int student_forward_impl(srwn_handle_t h, const float* z, NoiseSpec noise
   if (rc) return rc;
   if (precision == SRWN_BF16) return reject_bf16();
   if (precision == SRWN_FP16)
-    return run_student_fused_bf16(h, z, noise, z_out, enc, out, s_tot, mu_tot, x_last, B, T, 1, workspace, workspace_bytes, st);
+    return run_student_fused(h, z, noise, z_out, enc, out, s_tot, mu_tot, x_last, B, T, workspace, workspace_bytes, st);
   if (precision != SRWN_FP32) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
   F32Ws w = carve_f32(h, SRWN_OP_STUDENT_FORWARD, B, T, workspace, workspace_bytes, false);
   if (!workspace || w.bytes > workspace_bytes)

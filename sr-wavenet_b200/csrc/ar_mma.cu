@@ -23,7 +23,6 @@
 #include <cuda_fp16.h>
 #include <vector>
 #include <cstdio>
-#include <cstdlib>
 
 const float* srwn_host_weights(srwn_ctx* c);
 __global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ cond_k,
@@ -77,7 +76,6 @@ struct Params {
   float* logits_out;          // [B][T][4M] or null
   int* err;
   int B, T, L, P, frames, M, sum_d;
-  int dbg;                    // tuning experiments (SRWN_AR_DBG): wrong results, timing only
   int dil[kMaxL];
   int qoff[kMaxL];
 };
@@ -175,10 +173,6 @@ __device__ __forceinline__ void tmem_ld2(uint32_t taddr, float2& v) {
 __device__ __forceinline__ void tmem_wait_ld2(float2& v) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" : "+f"(v.x), "+f"(v.y) :: "memory");
 }
-#ifndef SRWN_AR_SPLIT_RES
-#define SRWN_AR_SPLIT_RES 1     // 1: chain warp j computes only n-tile j of the residual conv and the warps exchange the stream image
-#endif
-
 #ifdef SRWN_AR_TIMING
 __device__ __forceinline__ long long clk_after(uint32_t dep) {      // clock read ordered after the value `dep` is ready
   long long t;
@@ -254,7 +248,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
 
   if (warp == kProducerWarp) {
     // ================= producer: skip / head weights, L2 -> shared ring ===========================
-    if (lane == 0 && !(p.dbg & 16)) {
+    if (lane == 0) {
       long long it = 0;
       for (int t = 0; t < p.T; t++) {
         for (int i = 0; i < n_items; i++, it++) {
@@ -270,8 +264,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
     return;
   }
   if (warp < kChainWarps) {
-    // ================= chain warps: warp j owns channels 8j..8j+7 (n-tile j) of the filter conv and the gate;
-    // every warp then computes the whole residual conv and keeps the whole residual stream (no second exchange)
+    // ================= chain warps: warp j owns channels 8j..8j+7 (n-tile j) of the filter conv, the gate, the residual
+    // conv and the fp32 residual stream; the warps exchange the stream's 16-bit image once per layer
     const int j = warp;
     const int cpos = (j == 1 ? 2 : j == 2 ? 1 : j) * 4;   // n-tile j's word inside a lane's 16 bytes of a gate slot: order {0, 2, 1, 3}
     auto chain_sync = [&]() { asm volatile("bar.sync 1, 128;" ::: "memory"); };
@@ -282,7 +276,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
     volatile int* sq = reinterpret_cast<volatile int*>(smem + Smem::qofs);      // [2][kMaxL]: queue slot byte offsets, by step parity
     volatile float* sx = reinterpret_cast<volatile float*>(smem + Smem::xslot);
     float xm1 = 0.f, xm2 = 0.f;                         // x[t-1], x[t-2] of utterance g
-    float h[4][2];                                      // residual stream: n-tile i, columns 8i+2q, 8i+2q+1 of row g
+    float h[4][2];                                      // layer-0 input (front conv): n-tile i, columns 8i+2q, 8i+2q+1 of row g
     uint32_t hA[4];                                     // its fp16 image, n-tile i = channels 8i+2q, 8i+2q+1 (A fragments: kt0 (0,1), kt1 (2,3))
     uint32_t hB[2];                                     // second copy of hA[2], hA[3]: a0 / a2 of the k-tile 1 quad
     uint32_t dm[6];                                     // don't-care registers that complete the k-tile 1 quads
@@ -357,10 +351,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
 #pragma unroll
       for (int i = 0; i < 4; i++) hA[i] = pack_h2(h[i][0], h[i][1]);
       hB[0] = pack_h2(h[2][0], h[2][1]); hB[1] = pack_h2(h[3][0], h[3][1]);
-#if SRWN_AR_SPLIT_RES
       float hj0 = j == 0 ? h[0][0] : j == 1 ? h[1][0] : j == 2 ? h[2][0] : h[3][0];      // this warp's part of the fp32 stream
       float hj1 = j == 0 ? h[0][1] : j == 1 ? h[1][1] : j == 2 ? h[2][1] : h[3][1];
-#endif
       // filter-conv B fragments of this warp's n-tile: [taps k-tiles 0,1 | current k-tiles 2,3]
       uint4 wft = lds128_ro(sbase + Smem::chain + lane * 16 + (2 * j) * 512);
       uint4 wfc = lds128_ro(sbase + Smem::chain + lane * 16 + (2 * j + 1) * 512);
@@ -371,13 +363,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
       auto layer = [&](const int l, Pre& S) {
         const uint32_t wl = sbase + Smem::chain + l * kChainLayerBytes + lane * 16;
         AR_T(t_0, hA[0]);
-#if SRWN_AR_SPLIT_RES
         float2 cbj;                                      // term added after this layer (index l + 1), this warp's two channels
         if (l + 1 < L) tmem_ld2(tm + (l + 1) * 8 + 2 * j, cbj);
-#else
-        float2 cbn[4];                                   // term added after this layer (index l + 1)
-        tmem_ld8(tm + (l + 1) * 8, cbn);
-#endif
         // ---- filter conv (ops.py:6-10), n-tile j: taps (W[0] on h[t-d]) and current (W[1] on h[t]) as two
         //      independent accumulation chains
         float acc[4] = {0.f, 0.f, 0.f, 0.f}, acc2[4] = {0.f, 0.f, 0.f, 0.f};
@@ -387,13 +374,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
         mma8q(acc, S.tap.y, dm[2], S.tap.w, dm[3], wft.z, wft.w);
         AR_T(t_1, S.tap.x);
         AR_T(t_2, __float_as_uint(acc[0] + acc2[0]));
-#if SRWN_AR_SPLIT_RES
         const uint4 wrj = lds128_ro(wl + 4096 + j * 512); // residual B fragments of n-tile j: land while the gate runs
-#else
-        uint4 wr[4];                                     // residual B fragments: land while the gate runs
-#pragma unroll
-        for (int i = 0; i < 4; i++) wr[i] = lds128_ro(wl + 4096 + i * 512);
-#endif
         // push h[t] (the slot held h[t-d] until now); every chain warp holds the same image
         if (j == 0) *reinterpret_cast<uint4*>(qbase + S.ofs) = make_uint4(hA[0], hA[2], hA[1], hA[3]);
         if (l + 3 < L) prefetch(S, l + 3, sqt);          // this set's next use: layer l + 3
@@ -411,7 +392,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
         chain_sync();                                    // the four words of every lane's slot are in place
         AR_T(t_4, 0u);
         if (j == 0 && lane == 0) mbar_arrive(bar(B_CFULL + l));      // release: the skip warps may read the slot
-#if SRWN_AR_SPLIT_RES
         // The output of the last layer is not used (model.py:183-190: only the skips reach the head), so its residual conv
         // is skipped.  Otherwise warp j computes n-tile j of the residual conv (two dependent MMAs instead of eight),
         // updates its two channels of the fp32 stream and the four warps exchange the 16-bit image through one slot.
@@ -429,26 +409,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
           hA[0] = hq.x; hA[2] = hq.y; hA[1] = hq.z; hA[3] = hq.w; hB[0] = hq.y; hB[1] = hq.w;
         }
         AR_T(t_5, hA[0] ^ hA[3]);
-#else
-        const uint4 cA = lds128(sbase + Smem::cslots + l * kSlotBytes + lane * 16);     // {c n-tile 0, 2, 1, 3}
-        // ---- residual 1x1 (ops.py:39) and dense = (inputs + residual) * sqrt(1/2) (ops.py:40); the folded
-        //      term carries sqrt(1/2)*bias and the next layer's conditioning (model.py:183)
-        float r[4][4];
-#pragma unroll
-        for (int i = 0; i < 4; i++) { r[i][0] = r[i][1] = r[i][2] = r[i][3] = 0.f; mma8q(r[i], cA.x, cA.y, cA.z, cA.w, wr[i].x, wr[i].y); }
-#pragma unroll
-        for (int i = 0; i < 4; i++) mma8q(r[i], cA.y, dm[4], cA.w, dm[5], wr[i].z, wr[i].w);
-        tmem_wait_ld(cbn);
-#pragma unroll
-        for (int i = 0; i < 4; i++) {
-          h[i][0] = fmaf(h[i][0] + r[i][0], SRWN_SQRT_HALF, cbn[i].x);
-          h[i][1] = fmaf(h[i][1] + r[i][1], SRWN_SQRT_HALF, cbn[i].y);
-        }
-#pragma unroll
-        for (int i = 0; i < 4; i++) hA[i] = pack_h2(h[i][0], h[i][1]);
-        hB[0] = pack_h2(h[2][0], h[2][1]); hB[1] = pack_h2(h[3][0], h[3][1]);
-        AR_T(t_5, hA[0] ^ hA[3]);
-#endif
         AR_ACC(tl_top, t_1 - t_0); AR_ACC(tl_conv, t_2 - t_1); AR_ACC(tl_gate, t_3 - t_2); AR_ACC(tl_sync, t_4 - t_3); AR_ACC(tl_res, t_5 - t_4);
       };
       {
@@ -470,7 +430,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
       const long long c1 = clock64();
       long long c2 = c1;
       if (j < 3) {
-        ok = ok && ((p.dbg & 32) || mbar_wait(bar(B_HID2), (uint32_t)(t & 1), abort_flag));
+        ok = ok && mbar_wait(bar(B_HID2), (uint32_t)(t & 1), abort_flag);
         c2 = clock64();
         float lgA[4] = {0.f, 0.f, 0.f, 0.f}, lgB[4] = {0.f, 0.f, 0.f, 0.f};      // two accumulation chains
         const uint32_t hb = sbase + Smem::cslots + (hid_slot + 8) * kSlotBytes + lane * 8;   // hid2 tiles
@@ -546,7 +506,6 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
   // half the tensor-pipe work of the row-major form, on pipes the chain warps share.  The B fragment of c^T is the same
   // register pair as the A fragment of c (b0 = a0, b1 = a2), so the gate slot is read as it is.
   const int sw = warp - 5;                                // warps 5..8 -> 0..3: skip / hidden channels 32 sw .. 32 sw + 31
-  if (p.dbg & 32) return;
   const float* shb = reinterpret_cast<const float*>(smem + Smem::hbias);
   long long it = 0;
   uint4 h1a[2][8];                                        // H1^T A fragments of this warp's two m-tiles, resident: [m-tile][k-tile]
@@ -564,7 +523,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
     bool ok = true;
     for (int l = 0; l < L && ok; l++, it++) {
       const int st = (int)(it % kStages);
-      ok = ((p.dbg & 16) || mbar_wait(bar(B_WFULL + st), (uint32_t)((it / kStages) & 1), abort_flag)) &&
+      ok = mbar_wait(bar(B_WFULL + st), (uint32_t)((it / kStages) & 1), abort_flag) &&
            mbar_wait(bar(B_CFULL + l), (uint32_t)(t & 1), abort_flag);      // suspended, not spinning: the chain warps share the SMSPs
       if (!ok) break;
       const uint4 c = lds128(sbase + Smem::cslots + l * kSlotBytes + lane * 16);   // gate output, n-tiles {0, 2, 1, 3}
@@ -765,7 +724,6 @@ int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, 
     if (c->dilations[l] & (c->dilations[l] - 1)) pow2 = false;
   }
   p.sum_d = pow2 ? -c->sum_dilation : c->sum_dilation;
-  p.dbg = getenv("SRWN_AR_DBG") ? atoi(getenv("SRWN_AR_DBG")) : 0;
   SRWN_CUDA(cudaFuncSetAttribute(armma::k_ar_mma, cudaFuncAttributeMaxDynamicSharedMemorySize, armma::Smem::total));
   ProfScope prof(c, st, "k_ar_mma", 1);
   armma::k_ar_mma<<<w.grid, armma::kThreads, armma::Smem::total, st>>>(p);

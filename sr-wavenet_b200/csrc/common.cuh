@@ -68,7 +68,7 @@ struct srwn_ctx {
   bool device_dirty;                  // device weights changed by srwn_adam_step: host mirror and packed images are stale
   int device;
   int sm_count;
-  // packed bf16 operand images for the tcgen05 path (built at commit)
+  // packed fp16 operand images of the fused kernel, one per stack (built at commit)
   void* d_packed;
   size_t packed_bytes;
   void* d_part;                       // work partition of the fused kernel for (part_B, part_T, team size): segs | nseg (allocated at create)
@@ -156,18 +156,18 @@ size_t ar_mma_workspace_bytes(const srwn_ctx* c, int B, int T);
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
                float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st);
 int ar_mma_check_error(const srwn_ctx* c, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st);
-// fused_bf16.cu
+// fused.cu
 bool fused_supported(const srwn_ctx* c);
 size_t fused_packed_bytes(const srwn_ctx* c);
 int fused_pack_weights(srwn_ctx* c, cudaStream_t st);
 size_t fused_workspace_bytes(const srwn_ctx* c, int op, int B, int T);
-int run_teacher_fused_bf16(srwn_ctx* c, const float* x_in, const float* enc,
-                           const float* x_scored, float* nll_out, float* nll_sum,
-                           float* logits_out, int B, int T, int fp16, void* ws, size_t ws_bytes,
-                           cudaStream_t st);
-int run_student_fused_bf16(srwn_ctx* c, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out,
-                           float* s_tot, float* mu_tot, float* x_last, int B, int T, int fp16,
-                           void* ws, size_t ws_bytes, cudaStream_t st);
+int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc,
+                      const float* x_scored, float* nll_out, float* nll_sum,
+                      float* logits_out, int B, int T, void* ws, size_t ws_bytes,
+                      cudaStream_t st);
+int run_student_fused(srwn_ctx* c, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out,
+                      float* s_tot, float* mu_tot, float* x_last, int B, int T,
+                      void* ws, size_t ws_bytes, cudaStream_t st);
 int fused_check_error(void* ws, size_t ws_bytes, const srwn_ctx* c, int B, int T, cudaStream_t st);
 size_t fused_partition_bytes(const srwn_ctx* c);
 void fused_last_partition(const srwn_ctx* c, int* teams, int* G);

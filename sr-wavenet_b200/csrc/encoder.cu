@@ -5,7 +5,7 @@
 //
 // Two paths behind srwn_teacher_encode:
 //  * fp32 (parity grade): FFMA GEMM kernels, activations and the skip sum in fp32 in the workspace.
-//  * fp16 / bf16 operands on tcgen05 tensor cores, one launch per layer (k_enc_layer):
+//  * fp16 operands on tcgen05 tensor cores, one launch per layer (k_enc_layer):
 //      - activations travel between layers as the 16-bit image of relu(h) in the UMMA K-major
 //        no-swizzle layout, one contiguous block [16 kc][129 rows][8] per tile of 128 time steps (row 128
 //        repeats row 0 of the next tile), so a tile is loaded with two bulk copies and the a[t+1] tap is the
@@ -68,18 +68,12 @@ struct LayerParams {
   int reverse;               // walk the tiles from the end: the tail of the previous layer's output is still in L2
 };
 
-template <bool FP16>
 __device__ __forceinline__ uint32_t pack2_relu(float lo, float hi) {
   uint32_t r;
-  if (FP16) asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));   // saturating: no inf in an operand image
-  else asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));
+  asm("cvt.rn.relu.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(hi), "f"(lo));   // saturating: no inf in an operand image
   return r;
 }
-template <bool FP16>
-__device__ __forceinline__ float2 unpack2(uint32_t v) {
-  if (FP16) return __half22float2(*reinterpret_cast<const __half2*>(&v));
-  return __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v));
-}
+__device__ __forceinline__ float2 unpack2(uint32_t v) { return __half22float2(*reinterpret_cast<const __half2*>(&v)); }
 
 __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t bytes, uint32_t bar) {
   asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
@@ -88,7 +82,7 @@ __device__ __forceinline__ void bulk_g2s(uint32_t dst, const void* src, uint32_t
 
 constexpr int kThreads = 10 * 32;   // warp 0 loader, warp 1 MMA issuer + TMEM owner, warps 2-5 epilogue 1, warps 6-9 epilogue 2
 
-template <bool FRONT, bool FP16>
+template <bool FRONT>
 __global__ void __launch_bounds__(kThreads, 1) k_enc_layer(const LayerParams p) {
   extern __shared__ __align__(1024) uint8_t smem[];
   const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -119,7 +113,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_enc_layer(const LayerParams p) 
   const uint32_t tmem = *tmem_slot;
   const int n_my = p.n_tiles > (int)blockIdx.x ? (p.n_tiles - 1 - (int)blockIdx.x) / (int)gridDim.x + 1 : 0;
   auto tile_of = [&](int k) { const int i = (int)blockIdx.x + k * (int)gridDim.x; return p.reverse ? p.n_tiles - 1 - i : i; };
-  constexpr uint32_t idesc = make_idesc(FP16 ? 0 : 1, 128, 128);
+  constexpr uint32_t idesc = make_idesc(0, 128, 128);      // fp16 operands
   constexpr int w_bytes = FRONT ? kFrontImg : kLayerImg;
   constexpr int res_off = FRONT ? 0 : kConvImg;               // residual image inside the shared weight area
   float* s_bias = reinterpret_cast<float*>(smem + Smem::bias);
@@ -232,7 +226,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_enc_layer(const LayerParams p) 
             lo = v[2 * j] + cbias[c];
             hi = v[2 * j + 1] + cbias[c + 1];
           }
-          w[c2 * 32 + j] = pack2_relu<FP16>(lo, hi);
+          w[c2 * 32 + j] = pack2_relu(lo, hi);
         }
       }
       if (!FRONT) {                       // accumulator drained: the conv GEMM of tile k+2 may overwrite it
@@ -267,7 +261,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_enc_layer(const LayerParams p) 
 #pragma unroll 4
         for (int i = 0; i < 16; i++) {
           const uint4 u = *reinterpret_cast<const uint4*>(yb + i * 8 * 16);
-          const float2 f0 = unpack2<FP16>(u.x), f1 = unpack2<FP16>(u.y), f2 = unpack2<FP16>(u.z), f3 = unpack2<FP16>(u.w);
+          const float2 f0 = unpack2(u.x), f1 = unpack2(u.y), f2 = unpack2(u.z), f3 = unpack2(u.w);
           acc[0] += f0.x; acc[1] += f0.y; acc[2] += f1.x; acc[3] += f1.y;
           acc[4] += f2.x; acc[5] += f2.y; acc[6] += f3.x; acc[7] += f3.y;
         }
@@ -304,7 +298,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_enc_layer(const LayerParams p) 
 #pragma unroll
             for (int e = 0; e < 4; e++) {
               const int c = c2 * 64 + j * 8 + 2 * e;
-              w[e] = pack2_relu<FP16>(v[j * 8 + 2 * e] + rbias[c], v[j * 8 + 2 * e + 1] + rbias[c + 1]);   // ops.py:49 of the next layer
+              w[e] = pack2_relu(v[j * 8 + 2 * e] + rbias[c], v[j * 8 + 2 * e + 1] + rbias[c + 1]);   // ops.py:49 of the next layer
             }
             const uint4 u = make_uint4(w[0], w[1], w[2], w[3]);
             *reinterpret_cast<uint4*>(og + ((c2 * 8 + j) * kARows + row) * 16) = u;
@@ -460,7 +454,7 @@ struct srwn_encoder {
   std::vector<uint8_t> is_set;
   float* d_f32;                    // fp32 arena: all of the above, in that order
   size_t o_front_k, o_front_b, o_conv_k, o_conv_b, o_res_k, o_res_b, o_skip_k, o_skip_b, o_lat_k, o_lat_b, o_wf, o_bf, n_f32;
-  uint8_t* d_img;                  // [2 formats][front image | L layer images]
+  uint8_t* d_img;                  // fp16 operands: front image | L layer images
   size_t img_bytes;
   bool committed;
   int sm_count;
@@ -510,7 +504,7 @@ extern "C" int srwn_encoder_create(const srwn_encoder_config_t* cfg, srwn_encode
   }
   cudaDeviceGetAttribute(&e->sm_count, cudaDevAttrMultiProcessorCount, dev);
   e->img_bytes = (size_t)enc::kFrontImg + (size_t)e->L * enc::kLayerImg;
-  if (enc_tc_supported(e) && cudaMalloc(&e->d_img, 2 * e->img_bytes) != cudaSuccess) {
+  if (enc_tc_supported(e) && cudaMalloc(&e->d_img, e->img_bytes) != cudaSuccess) {
     cudaGetLastError(); cudaFree(e->d_f32); delete e;
     return srwn_fail(SRWN_ERR_CUDA, "srwn_encoder_create: allocation failed");
   }
@@ -579,9 +573,8 @@ extern "C" int srwn_encoder_set_weight(srwn_encoder_t e, const char* name, const
   return SRWN_OK;
 }
 
-static uint16_t enc_to_bits(float f, bool fp16) {
-  if (fp16) { __half h = __float2half_rn(f); return *reinterpret_cast<uint16_t*>(&h); }
-  __nv_bfloat16 h = __float2bfloat16_rn(f);
+static uint16_t enc_to_bits(float f) {
+  __half h = __float2half_rn(f);
   return *reinterpret_cast<uint16_t*>(&h);
 }
 static inline size_t enc_kmajor(int n, int k, int rows) { return ((size_t)(k / 8) * rows + n) * 8 + (k % 8); }
@@ -617,33 +610,29 @@ extern "C" int srwn_encoder_commit(srwn_encoder_t e, void* stream) {
   SRWN_CUDA(cudaMemcpyAsync(e->d_f32, host.data(), host.size() * sizeof(float), cudaMemcpyHostToDevice, st));
   std::vector<uint8_t> img;
   if (e->d_img) {
-    img.assign(2 * e->img_bytes, 0);
-    for (int fmt = 0; fmt < 2; fmt++) {
-      const bool fp16 = fmt == 1;
-      uint8_t* base = img.data() + (size_t)fmt * e->img_bytes;
-      {  // front: res image | front_k[2][E] | front_b[E] | res bias[E]
-        uint16_t* ri = reinterpret_cast<uint16_t*>(base);
-        for (int k = 0; k < E; k++)
-          for (int n = 0; n < E; n++) ri[enc_kmajor(n, k, E)] = enc_to_bits(e->res_k[(size_t)k * E + n], fp16);
-        float* f = reinterpret_cast<float*>(base + enc::kResImg);
-        memcpy(f, e->front_k.data(), 2 * E * sizeof(float));
-        memcpy(f + 2 * E, e->front_b.data(), E * sizeof(float));
-        memcpy(f + 3 * E, e->res_b.data(), E * sizeof(float));
-      }
-      for (int l = 0; l < L; l++) {
-        uint8_t* lb = base + enc::kFrontImg + (size_t)l * enc::kLayerImg;
-        uint16_t* ci = reinterpret_cast<uint16_t*>(lb);
-        uint16_t* ri = reinterpret_cast<uint16_t*>(lb + enc::kConvImg);
-        const float* ck = e->conv_k.data() + (size_t)l * 2 * E * E;        // [tap][Cin][Cout]
-        for (int k = 0; k < 2 * E; k++)
-          for (int n = 0; n < E; n++) ci[enc_kmajor(n, k, E)] = enc_to_bits(ck[(size_t)k * E + n], fp16);
-        const float* rk = e->res_k.data() + (size_t)(l + 1) * E * E;
-        for (int k = 0; k < E; k++)
-          for (int n = 0; n < E; n++) ri[enc_kmajor(n, k, E)] = enc_to_bits(rk[(size_t)k * E + n], fp16);
-        float* f = reinterpret_cast<float*>(lb + enc::kConvImg + enc::kResImg);
-        memcpy(f, e->conv_b.data() + (size_t)l * E, E * sizeof(float));
-        memcpy(f + E, e->res_b.data() + (size_t)(l + 1) * E, E * sizeof(float));
-      }
+    img.assign(e->img_bytes, 0);
+    {  // front: res image | front_k[2][E] | front_b[E] | res bias[E]
+      uint16_t* ri = reinterpret_cast<uint16_t*>(img.data());
+      for (int k = 0; k < E; k++)
+        for (int n = 0; n < E; n++) ri[enc_kmajor(n, k, E)] = enc_to_bits(e->res_k[(size_t)k * E + n]);
+      float* f = reinterpret_cast<float*>(img.data() + enc::kResImg);
+      memcpy(f, e->front_k.data(), 2 * E * sizeof(float));
+      memcpy(f + 2 * E, e->front_b.data(), E * sizeof(float));
+      memcpy(f + 3 * E, e->res_b.data(), E * sizeof(float));
+    }
+    for (int l = 0; l < L; l++) {
+      uint8_t* lb = img.data() + enc::kFrontImg + (size_t)l * enc::kLayerImg;
+      uint16_t* ci = reinterpret_cast<uint16_t*>(lb);
+      uint16_t* ri = reinterpret_cast<uint16_t*>(lb + enc::kConvImg);
+      const float* ck = e->conv_k.data() + (size_t)l * 2 * E * E;        // [tap][Cin][Cout]
+      for (int k = 0; k < 2 * E; k++)
+        for (int n = 0; n < E; n++) ci[enc_kmajor(n, k, E)] = enc_to_bits(ck[(size_t)k * E + n]);
+      const float* rk = e->res_k.data() + (size_t)(l + 1) * E * E;
+      for (int k = 0; k < E; k++)
+        for (int n = 0; n < E; n++) ri[enc_kmajor(n, k, E)] = enc_to_bits(rk[(size_t)k * E + n]);
+      float* f = reinterpret_cast<float*>(lb + enc::kConvImg + enc::kResImg);
+      memcpy(f, e->conv_b.data() + (size_t)l * E, E * sizeof(float));
+      memcpy(f + E, e->res_b.data() + (size_t)(l + 1) * E, E * sizeof(float));
     }
     SRWN_CUDA(cudaMemcpyAsync(e->d_img, img.data(), img.size(), cudaMemcpyHostToDevice, st));
   }
@@ -678,15 +667,15 @@ extern "C" int srwn_encoder_workspace_bytes(srwn_encoder_t e, int32_t B, int32_t
   return SRWN_OK;
 }
 
-template <bool FRONT, bool FP16>
+template <bool FRONT>
 static int launch_layer(const srwn_encoder* e, const enc::LayerParams& p, cudaStream_t st) {
   static bool attr_done = false;
   if (!attr_done) {
-    SRWN_CUDA(cudaFuncSetAttribute(enc::k_enc_layer<FRONT, FP16>, cudaFuncAttributeMaxDynamicSharedMemorySize, enc::Smem::total));
+    SRWN_CUDA(cudaFuncSetAttribute(enc::k_enc_layer<FRONT>, cudaFuncAttributeMaxDynamicSharedMemorySize, enc::Smem::total));
     attr_done = true;
   }
   const int grid = p.n_tiles < e->sm_count ? p.n_tiles : e->sm_count;
-  enc::k_enc_layer<FRONT, FP16><<<grid, enc::kThreads, enc::Smem::total, st>>>(p);
+  enc::k_enc_layer<FRONT><<<grid, enc::kThreads, enc::Smem::total, st>>>(p);
   SRWN_LAUNCH_CHECK();
   return SRWN_OK;
 }
@@ -737,25 +726,24 @@ extern "C" int srwn_teacher_encode(srwn_encoder_t e, const float* x, float* enc_
     SRWN_LAUNCH_CHECK();
   } else {
     if (precision != SRWN_FP16) return srwn_fail(SRWN_ERR_UNSUPPORTED, "the tensor-core encoder is built for fp16 operands only; use SRWN_FP16 or SRWN_FP32");
-    const bool fp16 = true;
     const size_t n_tiles = rows / enc::kTile;
     uint8_t* act0 = w.take<uint8_t>(n_tiles * enc::kAStage);
     uint8_t* act1 = w.take<uint8_t>(n_tiles * enc::kAStage);
     float* pooled = w.take<float>((size_t)L * n_tiles * enc::kE);
     int* err = w.take<int>(64);
     SRWN_CUDA(cudaMemsetAsync(err, 0, 64 * sizeof(int), st));
-    const uint8_t* img = e->d_img + (fp16 ? e->img_bytes : 0);
+    const uint8_t* img = e->d_img;
     enc::LayerParams p;
     p.err = err; p.n_tiles = (int)n_tiles; p.tiles_per_utt = T / enc::kTile; p.T = T;
     p.img = img; p.in = nullptr; p.x = x; p.out = act0; p.pooled = nullptr; p.reverse = 0;
-    int rc = launch_layer<true, true>(e, p, st);
+    int rc = launch_layer<true>(e, p, st);
     if (rc) return rc;
     uint8_t* cur = act0; uint8_t* nxt = act1;
     for (int l = 0; l < L; l++) {
       p.img = img + enc::kFrontImg + (size_t)l * enc::kLayerImg;
       p.in = cur; p.x = nullptr; p.out = l + 1 < L ? nxt : nullptr; p.pooled = pooled + (size_t)l * n_tiles * enc::kE;
       p.reverse = (l & 1) ^ 1;
-      rc = launch_layer<false, true>(e, p, st);
+      rc = launch_layer<false>(e, p, st);
       if (rc) return rc;
       uint8_t* t = cur; cur = nxt; nxt = t;
     }

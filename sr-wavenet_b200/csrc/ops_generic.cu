@@ -1,6 +1,6 @@
 // Stateless, shape-generic versions of the ops.py building blocks.  These back the
 // Python mirror of ops.py (any channel count / kernel size); the model paths use the
-// specialised kernels in stack_f32.cu / fused_bf16.cu / ar_generate.cu instead.
+// specialised kernels in stack_f32.cu / fused.cu / ar_generate.cu instead.
 #include "common.cuh"
 
 // ops.py:6-20: out[b,t,co] = bias[co] + sum_k sum_ci x[b, t - d*(K-1-k), ci] * w[k,ci,co]

@@ -3,7 +3,7 @@
 // One launch per layer; the residual stream (and the teacher's skip sum) round-trips through HBM as fp32.  The layer
 // GEMMs run on the tensor cores with split TF32 operands (train::k_fwd_layer, three MMAs per product), conditioning,
 // front conv and the output heads are FFMA kernels.  This is the reference-grade path and the GPU-side cross-check for
-// the fused 16-bit tcgen05 kernel (fused_bf16.cu), which is the one the benchmark times.
+// the fused fp16 tcgen05 kernel (fused.cu), which is the one the benchmark times.
 //
 // Stored tensor convention: `hc_i` = the block input of layer i = h_i + upsampled
 // conditioning of layer i (model.py:183 adds it before ResidualDilationLayer, so it also

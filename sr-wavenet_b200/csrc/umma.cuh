@@ -1,7 +1,6 @@
 // tcgen05 / mbarrier / bulk-copy PTX wrappers shared by the tensor-core kernels (sm_100a).
 #pragma once
 #include <cuda_fp16.h>
-#include <cuda_bf16.h>
 #include <stdint.h>
 
 namespace umma {
@@ -115,15 +114,12 @@ __host__ __device__ constexpr uint32_t make_idesc(int fmt, int M, int N) {
   return (1u << 4) | ((uint32_t)fmt << 7) | ((uint32_t)fmt << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
-template <bool FP16>
+// two fp32 values as an fp16 pair; saturating: a value beyond +-65504 becomes the largest finite half, not an inf that
+// would poison every later layer
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
-  if (FP16) {   // saturating: a value beyond +-65504 becomes the largest finite half, not an inf that would poison every later layer
-    uint32_t r;
-    asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
-    return r;
-  }
-  __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
+  uint32_t r;
+  asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(r) : "f"(b), "f"(a));
+  return r;
 }
 __device__ __forceinline__ bool elect_one() {
   uint32_t pred;

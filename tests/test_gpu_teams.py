@@ -1,4 +1,4 @@
-"""-m gpu: the team wavefront of the fused kernel (csrc/fused_bf16.cu).  A piece of the (utterance, chunk) line is walked
+"""-m gpu: the team wavefront of the fused kernel (csrc/fused.cu).  A piece of the (utterance, chunk) line is walked
 by a team of G CTAs that hand the per-layer history rings from CTA to CTA through global memory and flags; the result
 must not depend on G (G = 1 is the one-CTA-per-piece schedule with no hand-off), on the partition, or on the batch order."""
 import numpy as np

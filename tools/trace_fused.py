@@ -1,4 +1,5 @@
-"""Prints the clock64 timeline of CTA 0 for a few layers of one chunk (SRWN_TRACE=<chunk index>)."""
+"""Prints the clock64 timeline of CTA 0 for a few layers of one chunk (SRWN_TRACE=<chunk index>).
+Needs the -DSRWN_TUNING build of the fused kernel: tools/exp_build.sh, then SRWN_LIB=tools/exp/libsrwn_trace.so."""
 import sys, os, ctypes
 os.environ.setdefault("SRWN_TRACE", "20")
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
