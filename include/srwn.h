@@ -155,6 +155,26 @@ int srwn_teacher_generate(srwn_handle_t h, const float* enc, const float* u1,
                           const float* u2, float* x_out, float* logits_out,
                           int32_t B, int32_t T, int32_t precision,
                           void* workspace, size_t workspace_bytes, void* stream);
+/* Resumable generation: the same recurrence continued across calls through a caller-owned DEVICE state (streaming,
+ * long outputs in bounded memory, priming with real audio).
+ * srwn_generate_state_bytes: size of the state of B utterances for `precision` (SRWN_FP32 or SRWN_FP16); it does not
+ *   depend on T.  It holds the dilation queues in the layout of the precision's kernel (fp16: ceil(B/8) * sum(d) * 512
+ *   bytes; fp32: B * sum(d) * 32 floats), x[t-1] and x[t-2] of each utterance, the position t0 of the next step and a
+ *   signature (B, precision, layers, sum(d), pool_stride).
+ * srwn_generate_state_reset: zero queues and x history, t0 = 0 (the zero padding of ops.py:9).  A state is used only on
+ *   the handle, B and precision it was last reset for; any other call is refused with SRWN_ERR_INVALID.
+ * srwn_teacher_generate_resume: steps t0 .. t0+T-1, t0 read from the state on the device (no host synchronisation);
+ *   the state then holds t0+T.  enc [B,T/P,C] are the frames of THIS call, u1 [B,T,M] and u2 [B,T] its uniforms.
+ *   x_prefix [B,n_prefix] (0 <= n_prefix <= T; NULL when 0): for the first n_prefix steps x[t] is the given sample
+ *   instead of a draw (teacher forcing through the queues: priming); logits are still computed and x_out holds the
+ *   forced values.  Workspace: srwn_workspace_bytes(SRWN_OP_TEACHER_GENERATE, B, T) with this call's T.  With the same
+ *   uniforms, generating T1 + T2 samples in two calls gives bit for bit what one call over T1 + T2 gives. */
+int srwn_generate_state_bytes(srwn_handle_t h, int32_t B, int32_t precision, size_t* bytes);
+int srwn_generate_state_reset(srwn_handle_t h, void* state, int32_t B, int32_t precision, void* stream);
+int srwn_teacher_generate_resume(srwn_handle_t h, void* state, const float* enc, const float* u1,
+                                 const float* u2, const float* x_prefix, int32_t n_prefix, float* x_out,
+                                 float* logits_out, int32_t B, int32_t T, int32_t precision,
+                                 void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- student (model.py:415-535) ------------------------------------------------- */
 /* generate(sess, inputs, encoding) (model.py:570-576): z [B,T] logistic noise ->

@@ -24,9 +24,14 @@ struct ArParams {
   float* x_out;              // [B][T]
   float* logits_out;         // [B][T][4M] or null
   int B, T, L, P, frames, M, sum_d;
+  // resumable generation (RESUME): `queues` is then the caller's state, and so are these
+  const long long* t0;       // position of step 0 of this call: slot of layer l at step t is (t0 + t) mod d_l
+  float* xhist;              // [B][2] x[t-1], x[t-2] before step 0; rewritten with those of step T on exit
+  const float* x_prefix;     // [B][n_prefix]: for t < n_prefix, x[t] is this sample instead of a draw
+  int n_prefix;
 };
 
-template <int U>
+template <int U, bool RESUME>
 __global__ void __launch_bounds__(256, 1) k_ar_generate(const ArParams p) {
   __shared__ float s_cur[U][kR], s_tap[U][kR], s_c[U][kR];
   __shared__ float s_part[8][U][kR];
@@ -43,6 +48,8 @@ __global__ void __launch_bounds__(256, 1) k_ar_generate(const ArParams p) {
   const bool own = warp < U && (b0 + warp) < p.B;
   const int ub = b0 + (warp < U ? warp : 0);
   float xm1 = 0.f, xm2 = 0.f;            // x[t-1], x[t-2] (RightShift + K=2 front conv)
+  if (RESUME && own) { xm1 = p.xhist[2 * ub]; xm2 = p.xhist[2 * ub + 1]; }
+  const long long t0 = RESUME ? *p.t0 : 0;
   float skipacc[U];
 
   for (int t = 0; t < p.T; t++) {
@@ -63,7 +70,8 @@ __global__ void __launch_bounds__(256, 1) k_ar_generate(const ArParams p) {
         float tap = 0.f;
         if (own) {
           const int d = p.dil[l];
-          float* q = p.queues + ((size_t)ub * p.sum_d + p.qoff[l] + (t % d)) * kR + lane;
+          const int slot = RESUME ? (int)((t0 + t) % d) : t % d;
+          float* q = p.queues + ((size_t)ub * p.sum_d + p.qoff[l] + slot) * kR + lane;
           tap = *q;
           *q = hreg;
         }
@@ -183,6 +191,7 @@ __global__ void __launch_bounds__(256, 1) k_ar_generate(const ArParams p) {
         for (int m = 0; m < p.M; m++) uu[m] = p.u1[((size_t)ub * p.T + t) * p.M + m];
         int k;
         xs = mol_sample_one(s_logit[warp], uu, p.u2[(size_t)ub * p.T + t], p.M, &k);   // ops.py:178-201
+        if (RESUME && t < p.n_prefix) xs = p.x_prefix[(size_t)ub * p.n_prefix + t];
         p.x_out[(size_t)ub * p.T + t] = xs;
       }
       xs = __shfl_sync(0xffffffffu, xs, 0);
@@ -190,24 +199,36 @@ __global__ void __launch_bounds__(256, 1) k_ar_generate(const ArParams p) {
     }
     __syncthreads();   // s_part / s_logit reuse in the next step
   }
+  if (RESUME && own && lane == 0) { p.xhist[2 * ub] = xm1; p.xhist[2 * ub + 1] = xm2; }
 }
+
+__global__ void k_gen_state_advance(long long* t0, int T) { *t0 += T; }
+
+int run_gen_state_advance(long long* t0, int T, cudaStream_t st) {
+  k_gen_state_advance<<<1, 1, 0, st>>>(t0, T);
+  SRWN_LAUNCH_CHECK();
+  return SRWN_OK;
+}
+
+// dilation queues of B utterances: sum_d rows of R floats each
+size_t ar_queue_bytes(const srwn_ctx* c, int B) { return (size_t)B * c->sum_dilation * kR * sizeof(float); }
 
 size_t ar_workspace_bytes(const srwn_ctx* c, int B, int T) {
   WsCarver w(nullptr, 0);
-  w.take<float>((size_t)B * c->sum_dilation * kR);
+  w.take<uint8_t>(ar_queue_bytes(c, B));
   w.take<float>((size_t)B * (T / c->cfg.pool_stride) * c->cfg.n_layers * kR);
   return w.used;
 }
 
 int run_ar_generate(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
-                    float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
+                    float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenResume* rs) {
   if (!ws || ws_bytes < ar_workspace_bytes(c, B, T))
     return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", ar_workspace_bytes(c, B, T));
   WsCarver w(ws, ws_bytes);
   const int frames = T / c->cfg.pool_stride;
-  float* queues = w.take<float>((size_t)B * c->sum_dilation * kR);
+  float* queues = reinterpret_cast<float*>(w.take<uint8_t>(ar_queue_bytes(c, B)));
   float* cond = w.take<float>((size_t)B * frames * c->cfg.n_layers * kR);
-  SRWN_CUDA(cudaMemsetAsync(queues, 0, (size_t)B * c->sum_dilation * kR * sizeof(float), st));
+  if (!rs) SRWN_CUDA(cudaMemsetAsync(queues, 0, ar_queue_bytes(c, B), st));
   const float* sw = stack_w(c, 0);
   k_cond<<<B * frames, 256, 0, st>>>(enc, sw + c->off.cond_k, sw + c->off.cond_b, cond, B * frames,
                                      c->cfg.n_layers, c->cfg.cond_channels);
@@ -217,12 +238,22 @@ int run_ar_generate(srwn_ctx* c, const float* enc, const float* u1, const float*
   p.queues = queues; p.cond = cond; p.u1 = u1; p.u2 = u2; p.x_out = x_out; p.logits_out = logits_out;
   p.B = B; p.T = T; p.L = c->cfg.n_layers; p.P = c->cfg.pool_stride; p.frames = frames;
   p.M = c->cfg.num_mixtures; p.sum_d = c->sum_dilation;
-  ProfScope prof(c, st, "k_ar_generate", 1);
-  if (B > c->sm_count) {
-    k_ar_generate<2><<<(B + 1) / 2, 256, 0, st>>>(p);
-  } else {
-    k_ar_generate<1><<<B, 256, 0, st>>>(p);
+  p.t0 = nullptr; p.xhist = nullptr; p.x_prefix = nullptr; p.n_prefix = 0;
+  if (rs) {
+    p.queues = static_cast<float*>(rs->queues); p.t0 = rs->t0; p.xhist = rs->xhist;
+    p.x_prefix = rs->x_prefix; p.n_prefix = rs->n_prefix;
   }
-  SRWN_LAUNCH_CHECK();
+  {
+    ProfScope prof(c, st, "k_ar_generate", 1);
+    const bool two = B > c->sm_count;
+    const dim3 grid = two ? (B + 1) / 2 : B;
+    if (rs) {
+      if (two) k_ar_generate<2, true><<<grid, 256, 0, st>>>(p); else k_ar_generate<1, true><<<grid, 256, 0, st>>>(p);
+    } else {
+      if (two) k_ar_generate<2, false><<<grid, 256, 0, st>>>(p); else k_ar_generate<1, false><<<grid, 256, 0, st>>>(p);
+    }
+    SRWN_LAUNCH_CHECK();
+  }
+  if (rs) return run_gen_state_advance(rs->t0, T, st);
   return SRWN_OK;
 }

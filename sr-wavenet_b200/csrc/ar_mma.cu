@@ -78,6 +78,11 @@ struct Params {
   int B, T, L, P, frames, M, sum_d;
   int dil[kMaxL];
   int qoff[kMaxL];
+  // resumable generation (k_ar_mma<true>): `queues` is then the caller's state, and so are these
+  const long long* t0;        // position of step 0 of this call: slot of layer l at step t is (t0 + t) mod d_l
+  float* xhist;               // [B][2] x[t-1], x[t-2] before step 0; rewritten with those of step T on exit
+  const float* x_prefix;      // [B][n_prefix]: for t < n_prefix, x[t] is this sample instead of a draw
+  int n_prefix;
 };
 
 __device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
@@ -196,6 +201,10 @@ __global__ void k_sampler_noise(const float* __restrict__ u1, const float* __res
   if (i < n) { const float u = u2[i]; lg2[i] = logf(u) - logf(1.f - u); }
 }
 
+// RESUME = false: one call from silence (srwn_teacher_generate).  RESUME = true: continue from the caller's state
+// (srwn_teacher_generate_resume); the extra work is a phase per layer, two loads and two stores per utterance and the
+// forced-sample select, and none of it is compiled into the one-shot kernel.
+template <bool RESUME>
 __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
   extern __shared__ __align__(128) uint8_t smem[];
   const uint32_t sbase = smem_u32(smem);
@@ -276,6 +285,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
     volatile int* sq = reinterpret_cast<volatile int*>(smem + Smem::qofs);      // [2][kMaxL]: queue slot byte offsets, by step parity
     volatile float* sx = reinterpret_cast<volatile float*>(smem + Smem::xslot);
     float xm1 = 0.f, xm2 = 0.f;                         // x[t-1], x[t-2] of utterance g
+    if (RESUME && b0 + g < p.B) { xm1 = p.xhist[2 * (b0 + g)]; xm2 = p.xhist[2 * (b0 + g) + 1]; }
     float h[4][2];                                      // layer-0 input (front conv): n-tile i, columns 8i+2q, 8i+2q+1 of row g
     uint32_t hA[4];                                     // its fp16 image, n-tile i = channels 8i+2q, 8i+2q+1 (A fragments: kt0 (0,1), kt1 (2,3))
     uint32_t hB[2];                                     // second copy of hA[2], hA[3]: a0 / a2 of the k-tile 1 quad
@@ -322,7 +332,9 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
       }
       asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
     };
-    if (j == 0 && lane < L) sq[lane] = slot_of(lane, 0);
+    // lane l < L computes the slots of layer l; resuming, its steps count from t0, i.e. from phase t0 mod d_l
+    const int ph = RESUME && j == 0 && lane < L ? (int)(*p.t0 % p.dil[lane]) : 0;
+    if (j == 0 && lane < L) sq[lane] = slot_of(lane, ph);
     chain_sync();
     prefetch(S0, 0, sq);
     prefetch(S1, 1, sq);
@@ -338,8 +350,10 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
 #pragma unroll
       for (int m = 0; m < 8; m++) g1v[m] = (samp && m < p.M) ? __ldg(p.g1 + ((size_t)ub * p.T + t) * p.M + m) : 0.f;
       if (samp) lg2v = __ldg(p.lg2 + (size_t)ub * p.T + t);
+      float xpv = 0.f;                                   // forced sample of this step (priming)
+      if (RESUME && samp && t < p.n_prefix) xpv = __ldg(p.x_prefix + (size_t)ub * p.n_prefix + t);
       // queue slots of the next step, one lane per layer (read after the barriers of this step)
-      if (j == 0 && lane < L) sq[((t + 1) & 1) * kMaxL + lane] = slot_of(lane, t + 1);
+      if (j == 0 && lane < L) sq[((t + 1) & 1) * kMaxL + lane] = slot_of(lane, ph + t + 1);
       // front: RightShift + K=2 causal conv on one channel (model.py:172-173) + bias + conditioning of layer 0
       tmem_wait_ld(cb0);
 #pragma unroll
@@ -467,6 +481,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
           const float mean = sl[p.M + k];
           const float ls = fmaxf(sl[2 * p.M + k], -7.f);                  // ops.py:192
           xs = fminf(fmaxf(fmaf(expf(ls), lg2v, mean), -1.f), 1.f);       // ops.py:197-199
+          if (RESUME && t < p.n_prefix) xs = xpv;
           p.x_out[(size_t)ub * p.T + t] = xs;
           if (p.logits_out) {
             float* dst = p.logits_out + ((size_t)ub * p.T + t) * O;
@@ -490,6 +505,7 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
       printf("chain warp %d per layer: wait tap %lld, conv mma %lld, gate+store %lld, sync %lld, residual %lld\n", j, tl_top / n, tl_conv / n, tl_gate / n, tl_sync / n, tl_res / n);
     }
 #endif
+    if (RESUME && j == 0 && q == 0 && b0 + g < p.B) { p.xhist[2 * (b0 + g)] = xm1; p.xhist[2 * (b0 + g) + 1] = xm2; }
     if (j == 0 && lane == 0 && *abort_flag) atomicExch(p.err, 1);
     asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
     chain_sync();
@@ -673,12 +689,17 @@ int ar_mma_pack_weights(srwn_ctx* c, cudaStream_t st) {
 
 struct ArMmaWs { uint8_t* queues; float *cond, *cb, *g1, *lg2; int* err; size_t bytes; int grid; };
 
+// dilation queues of B utterances: one block of sum_d slots per CTA of 8 utterances
+size_t ar_mma_queue_bytes(const srwn_ctx* c, int B) {
+  return (size_t)((B + armma::kU - 1) / armma::kU) * c->sum_dilation * armma::kSlotBytes;
+}
+
 static ArMmaWs carve_ar_mma(const srwn_ctx* c, int B, int T, void* ws, size_t cap) {
   WsCarver w(ws, cap);
   ArMmaWs r{};
   const size_t frames = T / c->cfg.pool_stride, L = c->cfg.n_layers;
   r.grid = (B + armma::kU - 1) / armma::kU;
-  r.queues = w.take<uint8_t>((size_t)r.grid * c->sum_dilation * armma::kSlotBytes);
+  r.queues = w.take<uint8_t>(ar_mma_queue_bytes(c, B));
   r.cond = w.take<float>((size_t)B * frames * L * 32);
   r.cb = w.take<float>((size_t)B * frames * (L + 1) * 32);
   r.g1 = w.take<float>((size_t)B * T * c->cfg.num_mixtures);
@@ -691,13 +712,13 @@ static ArMmaWs carve_ar_mma(const srwn_ctx* c, int B, int T, void* ws, size_t ca
 size_t ar_mma_workspace_bytes(const srwn_ctx* c, int B, int T) { return carve_ar_mma(c, B, T, nullptr, 0).bytes; }
 
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
-               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
+               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenResume* rs) {
   if (!ar_mma_supported(c) || !c->d_ar_packed)
     return srwn_fail(SRWN_ERR_UNSUPPORTED, "fp16 generation kernel supports up to %d layers and 6 mixtures", armma::kMaxL);
   ArMmaWs w = carve_ar_mma(c, B, T, ws, ws_bytes);
   if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
   const int L = c->cfg.n_layers, frames = T / c->cfg.pool_stride;
-  SRWN_CUDA(cudaMemsetAsync(w.queues, 0, (size_t)w.grid * c->sum_dilation * armma::kSlotBytes, st));   // zero padding of ops.py:9
+  if (!rs) SRWN_CUDA(cudaMemsetAsync(w.queues, 0, ar_mma_queue_bytes(c, B), st));   // zero padding of ops.py:9
   SRWN_CUDA(cudaMemsetAsync(w.err, 0, 16, st));
   const float* sw = stack_w(c, 0);
   k_cond<<<B * frames, 256, 0, st>>>(enc, sw + c->off.cond_k, sw + c->off.cond_b, w.cond, B * frames, L, c->cfg.cond_channels);
@@ -724,10 +745,18 @@ int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, 
     if (c->dilations[l] & (c->dilations[l] - 1)) pow2 = false;
   }
   p.sum_d = pow2 ? -c->sum_dilation : c->sum_dilation;
-  SRWN_CUDA(cudaFuncSetAttribute(armma::k_ar_mma, cudaFuncAttributeMaxDynamicSharedMemorySize, armma::Smem::total));
-  ProfScope prof(c, st, "k_ar_mma", 1);
-  armma::k_ar_mma<<<w.grid, armma::kThreads, armma::Smem::total, st>>>(p);
-  SRWN_LAUNCH_CHECK();
+  if (rs) {
+    p.queues = static_cast<uint8_t*>(rs->queues); p.t0 = rs->t0; p.xhist = rs->xhist;
+    p.x_prefix = rs->x_prefix; p.n_prefix = rs->n_prefix;
+  }
+  auto kernel = rs ? armma::k_ar_mma<true> : armma::k_ar_mma<false>;
+  SRWN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, armma::Smem::total));
+  {
+    ProfScope prof(c, st, "k_ar_mma", 1);
+    kernel<<<w.grid, armma::kThreads, armma::Smem::total, st>>>(p);
+    SRWN_LAUNCH_CHECK();
+  }
+  if (rs) return run_gen_state_advance(rs->t0, T, st);
   return SRWN_OK;
 }
 

@@ -113,6 +113,16 @@ struct WsCarver {
 // on-device noise (philox.cuh): element i of (seed, stream); `on` = 0 means the caller supplied the tensor
 struct NoiseSpec { unsigned long long seed, stream; int on; };
 
+// resumable generation (srwn_teacher_generate_resume): the parts of the caller's state a generation kernel reads and
+// writes, and the samples it forces.  The state's layout is kept in api.cu (gen_state_layout).
+struct GenResume {
+  long long* t0;              // position of step 0 of the call; advanced by T after the kernel
+  float* xhist;               // [B][2]: x[t0-1], x[t0-2]
+  void* queues;               // dilation queues, laid out as the precision's kernel keeps them (ar_queue_bytes / ar_mma_queue_bytes)
+  const float* x_prefix;      // [B][n_prefix], or null when n_prefix == 0
+  int n_prefix;
+};
+
 // ---- kernel entry points implemented across translation units ---------------------
 // stack_f32.cu
 int run_stack_f32(srwn_ctx* c, int stack, const float* xin, const float* enc, int B, int T,
@@ -133,9 +143,12 @@ int run_mol_sample(const float* l, const float* u1, const float* u2, float* out,
                    int32_t* idx_out, int B, int T, int M, cudaStream_t st);
 // ar_generate.cu
 size_t ar_workspace_bytes(const srwn_ctx* c, int B, int T);
+size_t ar_queue_bytes(const srwn_ctx* c, int B);
+// rs == null: one call from silence; otherwise resume from (and advance) the caller's state
 int run_ar_generate(srwn_ctx* c, const float* enc, const float* u1, const float* u2,
                     float* x_out, float* logits_out, int B, int T, void* ws, size_t ws_bytes,
-                    cudaStream_t st);
+                    cudaStream_t st, const GenResume* rs);
+int run_gen_state_advance(long long* t0, int T, cudaStream_t st);
 // train_f32.cu
 size_t train_workspace_bytes(const srwn_ctx* c, int B, int T);
 int run_student_forward_train(srwn_ctx* c, const float* z, const float* enc, float* out, float* s_tot,
@@ -153,8 +166,9 @@ int run_adam(srwn_ctx* c, const float* grads, float* m, float* v, float* scratch
 bool ar_mma_supported(const srwn_ctx* c);
 int ar_mma_pack_weights(srwn_ctx* c, cudaStream_t st);
 size_t ar_mma_workspace_bytes(const srwn_ctx* c, int B, int T);
+size_t ar_mma_queue_bytes(const srwn_ctx* c, int B);
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
-               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st);
+               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenResume* rs);
 int ar_mma_check_error(const srwn_ctx* c, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st);
 // fused.cu
 bool fused_supported(const srwn_ctx* c);

@@ -559,19 +559,40 @@ class WaveNetAutoEncoder(_CheckpointMixin):
                                     precision=precision)
         return out
 
+    def generation_state(self, batch_size, precision="fp16"):
+        """A fresh (reset) state for resumable generation of ``batch_size`` utterances: pass it to ``generate(state=...)``
+        to continue a previous call instead of starting from silence."""
+        return GenerationState(self._eng, batch_size, precision)
+
     def generate(self, encoding, conditions=None, u1=None, u2=None, num_samples=None,
-                 return_logits=False, zero_last=False, precision="fp32"):
+                 return_logits=False, zero_last=False, precision="fp32", state=None, prefix=None):
         """Autoregressive generation, the queue-based restatement of teacher.py:153-170:
         x[t] = clip(MoL_sample(logits_t)) with logits_t from x[<t] and encoding[t // pool_stride].
-        ``zero_last=True`` reproduces teacher.py:170, which zeroes the final sample.
+        ``zero_last=True`` reproduces teacher.py:170, which zeroes the final sample of this call.
         ``precision``: "fp32" (parity-grade FFMA kernel) or "fp16" (tensor-core kernel, fp16 operands
-        and queue state, fp32 accumulate / residual stream)."""
+        and queue state, fp32 accumulate / residual stream).
+
+        ``state`` (from ``generation_state``): continue where the last call on that state stopped and advance it by
+        this call's T; ``encoding``, ``u1`` and ``u2`` then cover this call's samples only.  ``prefix`` [B, n], n <= T:
+        the first n samples of this call are these (real audio, teacher-forced through the queues) instead of draws;
+        without ``state`` it primes a fresh state used for this call alone.  Splitting a generation into calls gives
+        bit for bit the audio of one call only with injected ``u1``/``u2``: noise drawn on the device comes from a new
+        Philox stream per call."""
         eng = self._eng
         enc = _with_conditions(encoding, conditions, self.condition_size)
         e, on_dev = eng.to_device(enc, "enc")
         B = e.shape[0]
         T = num_samples if num_samples is not None else e.shape[1] * self.pool_stride
         self._check(e, B, T)
+        if prefix is not None:
+            xp = eng.to_device(prefix, "prefix")[0]
+            if xp.ndim != 2 or xp.shape[0] != B or xp.shape[1] > T:
+                raise ValueError("prefix must be [B=%d, n] with n <= T=%d, got %s" % (B, T, tuple(xp.shape)))
+            if state is None:
+                state = self.generation_state(B, precision)
+        if state is not None and (state.batch_size != B or state.precision != precision):
+            raise ValueError("state was made for batch_size=%d, precision=%r; this call has %d, %r"
+                             % (state.batch_size, state.precision, B, precision))
         lo, hi = 1e-5, 1.0 - 1e-5            # ops.py:187, 196
         if u1 is None or u2 is None:
             self._noise_calls = getattr(self, "_noise_calls", 0) + 1
@@ -586,9 +607,15 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         x = torch.empty(B, T, dtype=torch.float32, device="cuda")
         logits = torch.empty(B, T, 4 * self.num_mixtures, dtype=torch.float32, device="cuda") \
             if return_logits else None
-        _lib.check(eng.lib.srwn_teacher_generate(eng.h, e.data_ptr(), u1.data_ptr(), u2.data_ptr(),
-                                                 x.data_ptr(), logits.data_ptr() if return_logits else None,
-                                                 B, T, prec, ws, wsn, _stream()))
+        lg_ptr = logits.data_ptr() if return_logits else None
+        if state is None:
+            _lib.check(eng.lib.srwn_teacher_generate(eng.h, e.data_ptr(), u1.data_ptr(), u2.data_ptr(),
+                                                     x.data_ptr(), lg_ptr, B, T, prec, ws, wsn, _stream()))
+        else:
+            n = 0 if prefix is None else int(xp.shape[1])
+            _lib.check(eng.lib.srwn_teacher_generate_resume(eng.h, state.data_ptr(), e.data_ptr(), u1.data_ptr(),
+                                                            u2.data_ptr(), xp.data_ptr() if n else None, n, x.data_ptr(),
+                                                            lg_ptr, B, T, prec, ws, wsn, _stream()))
         if prec != _lib.FP32:
             eng.check_async(_lib.OP_TEACHER_GENERATE, B, T, prec)
         if zero_last:
@@ -603,6 +630,32 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         if e.shape[1] * self.pool_stride != T:
             raise ValueError("T=%d must equal pool_stride * frames = %d (model.py:183)"
                              % (T, e.shape[1] * self.pool_stride))
+
+
+class GenerationState(object):
+    """Device buffer that carries autoregressive generation from one ``generate`` call to the next: the dilation queues,
+    the last two samples and the position of each utterance (include/srwn.h, srwn_generate_state_*).  Created reset."""
+
+    def __init__(self, eng, batch_size, precision="fp16"):
+        self._eng = eng
+        self.batch_size, self.precision = int(batch_size), precision
+        self._prec = _lib.PRECISIONS[precision]
+        n = ctypes.c_size_t()
+        _lib.check(eng.lib.srwn_generate_state_bytes(eng.h, self.batch_size, self._prec, ctypes.byref(n)))
+        self.buffer = torch.empty(n.value, dtype=torch.uint8, device="cuda")
+        self.reset()
+
+    def reset(self):
+        """Back to silence at position 0 (the zero padding of ops.py:9)."""
+        _lib.check(self._eng.lib.srwn_generate_state_reset(self._eng.h, self.buffer.data_ptr(), self.batch_size,
+                                                           self._prec, _stream()))
+
+    def position(self):
+        """Samples generated through this state since the last reset (reads the device header: synchronises)."""
+        return int(self.buffer[:8].view(torch.int64).item())
+
+    def data_ptr(self):
+        return self.buffer.data_ptr()
 
 
 def _fused_available(eng):

@@ -41,7 +41,26 @@ def build_parser():
     p.add_argument('--clips', type=int, default=None, help='number of clips (default: 10 for --test-fast, 1 for --test-slow)')
     p.add_argument('--precision', type=str, default='fp16', choices=['fp32', 'fp16'])
     p.add_argument('--check-naive', type=int, default=0, help='--test-slow: also run the per-sample loop on the first N samples')
+    p.add_argument('--prime', type=int, default=0,
+                   help='--test-slow: the first N samples of each clip are the clip itself (N a multiple of --pool-stride); '
+                        'generation continues from there')
+    p.add_argument('--chunk', type=int, default=0,
+                   help='--test-slow: generate in calls of S samples (a multiple of --pool-stride) through one state')
     return p
+
+
+def generate_chunked(teacher, encoding, u1, u2, precision, prefix, chunk, pool_stride):
+    """--test-slow in calls of `chunk` samples through one generation state: the same audio as one call."""
+    B, T = u1.shape[0], u1.shape[1]
+    state = teacher.generation_state(B, precision)
+    n = 0 if prefix is None else prefix.shape[1]
+    parts = []
+    for a in range(0, T, chunk):
+        b = min(a + chunk, T)
+        parts.append(teacher.generate(encoding[:, a // pool_stride:b // pool_stride], u1=u1[:, a:b], u2=u2[:, a:b],
+                                      precision=precision, zero_last=b == T, state=state,
+                                      prefix=prefix[:, a:min(b, n)] if a < n else None))
+    return np.concatenate(parts, axis=1)
 
 
 def main(argv=None):
@@ -53,6 +72,10 @@ def main(argv=None):
     if args.train:
         raise SystemExit("teacher training (model.py:242-248) is outside the hot path of this build")
     num_samples, batch = args.num_samples, args.batch_size
+    for flag, v in (('--prime', args.prime), ('--chunk', args.chunk)):
+        if v < 0 or v % args.pool_stride or v > num_samples:
+            raise SystemExit('%s %d must be a multiple of --pool-stride %d and at most --num-samples %d'
+                             % (flag, v, args.pool_stride, num_samples))
     audio_data = AudioReader(args.data, batch, num_samples, audio_max_length=args.audio_max_length)
     teacher = srwn.WaveNetAutoEncoder(input_size=num_samples, condition_size=0, num_mixtures=5, dilations=DILATIONS,
                                       latent_channels=args.latent_channels, skip_channels=128,
@@ -79,15 +102,20 @@ def main(argv=None):
             encoding = teacher.encode(x, None, precision=args.precision)
             u1, u2 = synth.sampler_uniforms(x.shape[0], num_samples, 5, seed=999 + count)
             ar_prec = 'fp32' if args.precision == 'fp32' else 'fp16'    # the queue kernel keeps fp16 state on the 16-bit path
+            prefix = x[:, :args.prime] if args.prime else None
             t0 = time.time()
-            regen = teacher.generate(encoding, u1=u1, u2=u2, precision=ar_prec, zero_last=True)
+            if args.chunk:
+                regen = generate_chunked(teacher, encoding, u1, u2, ar_prec, prefix, args.chunk, args.pool_stride)
+            else:
+                regen = teacher.generate(encoding, u1=u1, u2=u2, precision=ar_prec, zero_last=True, prefix=prefix)
             dt = time.time() - t0
             results['test_slow_samples_per_s'] = regen.size / dt
             print('test-slow: %d x %d samples in %.3f s (%.3g samples/s)' % (regen.shape[0], regen.shape[1], dt, regen.size / dt))
             if args.check_naive:
                 n = min(args.check_naive, num_samples)
                 x_so_far = np.zeros((x.shape[0], num_samples), dtype=np.float32)
-                for i in range(n):                              # the reference's loop, verbatim semantics
+                x_so_far[:, :args.prime] = x[:, :args.prime]    # primed: those samples are kept, not drawn
+                for i in range(min(args.prime, n), n):          # the reference's loop, verbatim semantics
                     x_so_far[:, i:] = 0
                     x_so_far[:, i] = teacher.reconstruct_with_encoding(x_so_far, encoding, u1=u1, u2=u2,
                                                                        precision=args.precision)[:, i]
