@@ -60,7 +60,8 @@ enum srwn_op {               /* argument of srwn_workspace_bytes */
   SRWN_OP_TEACHER_NLL = 1,
   SRWN_OP_TEACHER_GENERATE = 2,
   SRWN_OP_STUDENT_FORWARD = 3,
-  SRWN_OP_STUDENT_TRAIN = 4    /* workspace of srwn_student_forward_train + srwn_student_backward */
+  SRWN_OP_STUDENT_TRAIN = 4,   /* workspace of srwn_student_forward_train + srwn_student_backward */
+  SRWN_OP_TEACHER_PREFILL = 5  /* workspace of srwn_generate_state_prefill (T = its n) */
 };
 
 /* Constructor arguments of WaveNetAutoEncoder (model.py:76-77) / ParallelWaveNet
@@ -156,7 +157,8 @@ int srwn_teacher_generate(srwn_handle_t h, const float* enc, const float* u1,
                           int32_t B, int32_t T, int32_t precision,
                           void* workspace, size_t workspace_bytes, void* stream);
 /* Resumable generation: the same recurrence continued across calls through a caller-owned DEVICE state (streaming,
- * long outputs in bounded memory, priming with real audio).
+ * long outputs in bounded memory, priming with real audio: step by step through x_prefix, or in one parallel pass
+ * through srwn_generate_state_prefill).
  * srwn_generate_state_bytes: size of the state of B utterances for `precision` (SRWN_FP32 or SRWN_FP16); it does not
  *   depend on T.  It holds the dilation queues in the layout of the precision's kernel (fp16: ceil(B/8) * sum(d) * 512
  *   bytes; fp32: B * sum(d) * 32 floats), x[t-1] and x[t-2] of each utterance, the position t0 of the next step and a
@@ -175,6 +177,16 @@ int srwn_teacher_generate_resume(srwn_handle_t h, void* state, const float* enc,
                                  const float* u2, const float* x_prefix, int32_t n_prefix, float* x_out,
                                  float* logits_out, int32_t B, int32_t T, int32_t precision,
                                  void* workspace, size_t workspace_bytes, void* stream);
+/* srwn_generate_state_prefill: primes a state with n known samples in one parallel pass.  x [B,n] are the samples of
+ *   positions t0 .. t0+n-1 and enc [B,n/P,C] their frames (the convention of a resume call); t0 is read on the device.
+ *   Afterwards the state is byte for byte the state srwn_teacher_generate_resume leaves after a call of T = n with
+ *   x_prefix = x (both precisions, any t0), and holds t0+n.  No audio and no logits are produced (srwn_teacher_nll scores
+ *   a prime).  Only the last sum(d) + 2 samples reach the state, so the cost and the workspace
+ *   (srwn_workspace_bytes(SRWN_OP_TEACHER_PREFILL, B, n)) depend on B and min(n, sum(d) + 2) only.  Refused: n <= 0 or
+ *   n % pool_stride != 0, a null x, enc or state, a state not reset on this handle for this B and precision, a student
+ *   handle, fp16 where the tensor-core generation kernel does not cover the configuration, a small workspace. */
+int srwn_generate_state_prefill(srwn_handle_t h, void* state, const float* x, const float* enc, int32_t n, int32_t B,
+                                int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
 
 /* ---- student (model.py:415-535) ------------------------------------------------- */
 /* generate(sess, inputs, encoding) (model.py:570-576): z [B,T] logistic noise ->

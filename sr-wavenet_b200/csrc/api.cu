@@ -437,6 +437,8 @@ static int reject_bf16() {
 extern "C" int srwn_supports(srwn_handle_t h, int32_t op, int32_t precision) {
   if (!h) return 0;
   const bool teacher_op = op == SRWN_OP_TEACHER_LOGITS || op == SRWN_OP_TEACHER_NLL || op == SRWN_OP_TEACHER_GENERATE;
+  if (op == SRWN_OP_TEACHER_PREFILL)
+    return h->cfg.kind == SRWN_TEACHER && (precision == SRWN_FP32 || (precision == SRWN_FP16 && ar_mma_supported(h))) ? 1 : 0;
   if (op == SRWN_OP_STUDENT_TRAIN) return h->cfg.kind == SRWN_STUDENT && precision == SRWN_FP32 ? 1 : 0;
   if (teacher_op != (h->cfg.kind == SRWN_TEACHER) || op < 0 || op > SRWN_OP_STUDENT_FORWARD) return 0;
   if (precision == SRWN_FP32) return 1;
@@ -470,6 +472,11 @@ extern "C" int srwn_workspace_bytes(srwn_handle_t h, int32_t op, int32_t B, int3
   if (op == SRWN_OP_STUDENT_TRAIN) {
     if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
     *bytes = train_workspace_bytes(h, B, T);
+    return SRWN_OK;
+  }
+  if (op == SRWN_OP_TEACHER_PREFILL) {
+    if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
+    *bytes = prefill_workspace_bytes(h, B, T, precision == SRWN_FP16 ? SRWN_FP16 : SRWN_FP32);
     return SRWN_OK;
   }
   return srwn_fail(SRWN_ERR_INVALID, "unknown op %d", op);
@@ -610,6 +617,32 @@ extern "C" int srwn_generate_state_reset(srwn_handle_t h, void* state, int32_t B
   return SRWN_OK;
 }
 
+// Refuses a state that was not last reset on this handle for this B and precision (host-side signature: no synchronisation).
+static int check_state_owner(srwn_handle_t h, const void* state, int B, int precision) {
+  int32_t sig[6];
+  state_signature(h, B, precision, sig);
+  std::lock_guard<std::mutex> lk(g_states_mu);
+  auto it = g_states.find(state);
+  if (it == g_states.end() || it->second.h != h)
+    return srwn_fail(SRWN_ERR_INVALID, "state was not reset on this handle (srwn_generate_state_reset)");
+  if (memcmp(it->second.sig, sig, sizeof(sig)))
+    return srwn_fail(SRWN_ERR_INVALID, "state was made for B=%d, precision %d; this call has B=%d, precision %d",
+                     it->second.sig[0], it->second.sig[1], B, precision);
+  return SRWN_OK;
+}
+
+static GenResume state_parts(const srwn_ctx* h, void* state, int B, int precision) {
+  uint8_t* base = static_cast<uint8_t*>(state);
+  const GenStateLayout lay = gen_state_layout(h, B, precision);
+  GenResume rs;
+  rs.t0 = &reinterpret_cast<GenStateHeader*>(base)->t0;
+  rs.xhist = reinterpret_cast<float*>(base + lay.xhist);
+  rs.queues = base + lay.queues;
+  rs.x_prefix = nullptr;
+  rs.n_prefix = 0;
+  return rs;
+}
+
 extern "C" int srwn_teacher_generate_resume(srwn_handle_t h, void* state, const float* enc, const float* u1,
                                             const float* u2, const float* x_prefix, int32_t n_prefix, float* x_out,
                                             float* logits_out, int32_t B, int32_t T, int32_t precision, void* workspace,
@@ -622,28 +655,30 @@ extern "C" int srwn_teacher_generate_resume(srwn_handle_t h, void* state, const 
   if (rc) return rc;
   if (n_prefix < 0 || n_prefix > T || (n_prefix > 0 && !x_prefix))
     return srwn_fail(SRWN_ERR_INVALID, "n_prefix=%d must be in [0, T=%d], with x_prefix given when > 0", n_prefix, T);
-  {
-    int32_t sig[6];
-    state_signature(h, B, precision, sig);
-    std::lock_guard<std::mutex> lk(g_states_mu);
-    auto it = g_states.find(state);
-    if (it == g_states.end() || it->second.h != h)
-      return srwn_fail(SRWN_ERR_INVALID, "state was not reset on this handle (srwn_generate_state_reset)");
-    if (memcmp(it->second.sig, sig, sizeof(sig)))
-      return srwn_fail(SRWN_ERR_INVALID, "state was made for B=%d, precision %d; this call has B=%d, precision %d",
-                       it->second.sig[0], it->second.sig[1], B, precision);
-  }
-  uint8_t* base = static_cast<uint8_t*>(state);
-  const GenStateLayout lay = gen_state_layout(h, B, precision);
-  GenResume rs;
-  rs.t0 = &reinterpret_cast<GenStateHeader*>(base)->t0;
-  rs.xhist = reinterpret_cast<float*>(base + lay.xhist);
-  rs.queues = base + lay.queues;
+  rc = check_state_owner(h, state, B, precision);
+  if (rc) return rc;
+  GenResume rs = state_parts(h, state, B, precision);
   rs.x_prefix = n_prefix > 0 ? x_prefix : nullptr;
   rs.n_prefix = n_prefix;
   if (precision == SRWN_FP16)
     return run_ar_mma(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, &rs);
   return run_ar_generate(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, &rs);
+}
+
+extern "C" int srwn_generate_state_prefill(srwn_handle_t h, void* state, const float* x, const float* enc, int32_t n,
+                                           int32_t B, int32_t precision, void* workspace, size_t workspace_bytes,
+                                           void* stream) {
+  if (!h || !state || !x || !enc) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_prefill: null argument");
+  int rc = check_state_args(h, B, precision, "srwn_generate_state_prefill");
+  if (rc) return rc;
+  rc = check_bt(h, B, n);                     // n % P == 0 keeps t0 on a frame boundary for later resume calls
+  if (rc) return rc;
+  rc = check_state_owner(h, state, B, precision);
+  if (rc) return rc;
+  GenResume rs = state_parts(h, state, B, precision);
+  rs.x_prefix = x;
+  rs.n_prefix = n;
+  return run_prefill(h, x, enc, B, n, precision, workspace, workspace_bytes, (cudaStream_t)stream, rs);
 }
 
 // ---- student --------------------------------------------------------------------------

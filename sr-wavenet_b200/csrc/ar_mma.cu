@@ -20,6 +20,7 @@
 //     memory / L2; the pop of layer l+2 is prefetched while layer l runs.
 #include "common.cuh"
 #include "mol.cuh"
+#include "ar_mma.cuh"
 #include <cuda_fp16.h>
 #include <vector>
 #include <cstdio>
@@ -105,37 +106,12 @@ __device__ __forceinline__ bool mbar_wait(uint32_t a, uint32_t parity, volatile 
 __device__ __forceinline__ void mbar_arrive(uint32_t a) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(a) : "memory");
 }
-__device__ __forceinline__ uint32_t pack_h2(float a, float b) {
-  __half2 h = __floats2half2_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&h);
-}
 // D(16x8, fp32) += A(16x16, fp16, row) * B(16x8, fp16, col); rows 8..15 of A are zero padding (a1 = a3 = 0)
 __device__ __forceinline__ void mma8(float (&d)[2], uint32_t a0, uint32_t a2, uint32_t b0, uint32_t b1) {
   float z0 = 0.f, z1 = 0.f;
   asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
                : "+f"(d[0]), "+f"(d[1]), "+f"(z0), "+f"(z1)
                : "r"(a0), "r"(0u), "r"(a2), "r"(0u), "r"(b0), "r"(b1));
-}
-// Same instruction with all four A registers named by the caller.  Rows 8..15 of A only reach rows 8..15 of D, which
-// nobody reads, so a1 / a3 may hold anything: passing registers that already sit next to a0 / a2 (the neighbours
-// inside a 128-bit load, or a quad the caller keeps alive) saves the moves that zero padding would cost.
-__device__ __forceinline__ void mma8q(float (&d)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
-  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
-}
-__device__ __forceinline__ float tanh_fast(float x) {
-  float y;
-  asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
-  return y;
-}
-// ops.py:28,33,36: f = tanh(a); f * sigmoid(f), sigmoid on [-1,1] as 0.5 + f*P(f^2) (error 1.5e-6)
-__device__ __forceinline__ float gate(float a) {
-  const float f = tanh_fast(a);
-  const float s = f * f;
-  float t = fmaf(s, 0.0017294071149080992f, -0.020638039335608482f);
-  t = fmaf(s, t, 0.2499687224626541f);
-  return fmaf(f, 0.5f, s * t);
 }
 __device__ __forceinline__ uint4 lds128(uint32_t a) {
   uint4 v;

@@ -170,6 +170,10 @@ size_t ar_mma_queue_bytes(const srwn_ctx* c, int B);
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
                float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenResume* rs);
 int ar_mma_check_error(const srwn_ctx* c, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st);
+// ar_prefill.cu: the state srwn_teacher_generate_resume leaves after forcing rs.x_prefix [B][n], computed in parallel
+size_t prefill_workspace_bytes(const srwn_ctx* c, int B, int n, int precision);
+int run_prefill(srwn_ctx* c, const float* x, const float* enc, int B, int n, int precision, void* ws, size_t ws_bytes,
+                cudaStream_t st, const GenResume& rs);
 // fused.cu
 bool fused_supported(const srwn_ctx* c);
 size_t fused_packed_bytes(const srwn_ctx* c);

@@ -624,6 +624,30 @@ class WaveNetAutoEncoder(_CheckpointMixin):
             return eng.to_host(x, on_dev), eng.to_host(logits, on_dev)
         return eng.to_host(x, on_dev)
 
+    def prefill(self, state, audio, encoding, conditions=None):
+        """Prime ``state`` with real audio in one parallel pass: afterwards it is, byte for byte, the state that
+        ``generate(state=state, prefix=audio)`` over the same n samples leaves, and ``state.position()`` has advanced by
+        n.  ``audio`` [B, n] (n a multiple of pool_stride) continues from the state's position; ``encoding`` [B, n/P, C]
+        are its frames.  Only the last sum(dilations) + 2 samples reach the state, so a long prime costs no more than
+        that window.  Produces no audio or logits (``nll`` scores a prime)."""
+        eng = self._eng
+        if not isinstance(state, GenerationState) or state._eng is not eng:
+            raise ValueError("state must come from this model's generation_state()")
+        enc = _with_conditions(encoding, conditions, self.condition_size)
+        e = eng.to_device(enc, "enc")[0]
+        x = eng.to_device(audio, "prefill")[0]
+        B = state.batch_size
+        if x.ndim != 2 or x.shape[0] != B or x.shape[1] < 1:
+            raise ValueError("audio must be [B=%d, n] with n >= 1, got %s" % (B, tuple(x.shape)))
+        n = int(x.shape[1])
+        self._check(e, B, n)
+        prec = _lib.PRECISIONS.get(state.precision)
+        if prec is None or not eng.lib.srwn_supports(eng.h, _lib.OP_TEACHER_PREFILL, prec):
+            raise ValueError("prefill(precision=%r) is not supported for this configuration" % state.precision)
+        ws, wsn = eng.workspace(_lib.OP_TEACHER_PREFILL, B, n, prec)
+        _lib.check(eng.lib.srwn_generate_state_prefill(eng.h, state.data_ptr(), x.data_ptr(), e.data_ptr(), n, B, prec,
+                                                       ws, wsn, _stream()))
+
     def _check(self, e, B, T):
         if e.ndim != 3 or e.shape[0] != B or e.shape[2] != self.latent_channels + self.condition_size:
             raise ValueError("encoding must be [B, T/pool_stride, %d]" % (self.latent_channels + self.condition_size))

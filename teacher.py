@@ -46,6 +46,8 @@ def build_parser():
                         'generation continues from there')
     p.add_argument('--chunk', type=int, default=0,
                    help='--test-slow: generate in calls of S samples (a multiple of --pool-stride) through one state')
+    p.add_argument('--prefill', action='store_true',
+                   help='--test-slow --prime N: prime the state in one parallel pass instead of step by step (same audio)')
     return p
 
 
@@ -61,6 +63,24 @@ def generate_chunked(teacher, encoding, u1, u2, precision, prefix, chunk, pool_s
                                       precision=precision, zero_last=b == T, state=state,
                                       prefix=prefix[:, a:min(b, n)] if a < n else None))
     return np.concatenate(parts, axis=1)
+
+
+def generate_prefilled(teacher, encoding, u1, u2, precision, prefix, chunk, pool_stride):
+    """--test-slow --prime N --prefill: prime a state with the N samples in one parallel pass, then generate the rest
+    from it (in calls of `chunk` samples if given).  The same audio as priming step by step."""
+    B, T, n = u1.shape[0], u1.shape[1], prefix.shape[1]
+    state = teacher.generation_state(B, precision)
+    teacher.prefill(state, prefix, encoding[:, :n // pool_stride])
+    parts = [np.asarray(prefix, dtype=np.float32)]
+    step = chunk or T - n
+    for a in range(n, T, step):
+        b = min(a + step, T)
+        parts.append(teacher.generate(encoding[:, a // pool_stride:b // pool_stride], u1=u1[:, a:b], u2=u2[:, a:b],
+                                      precision=precision, zero_last=b == T, state=state))
+    out = np.concatenate(parts, axis=1)
+    if n == T:
+        out[:, T - 1:] = 0                                      # teacher.py:170, as the one-call path does
+    return out
 
 
 def main(argv=None):
@@ -104,7 +124,9 @@ def main(argv=None):
             ar_prec = 'fp32' if args.precision == 'fp32' else 'fp16'    # the queue kernel keeps fp16 state on the 16-bit path
             prefix = x[:, :args.prime] if args.prime else None
             t0 = time.time()
-            if args.chunk:
+            if args.prefill and args.prime:
+                regen = generate_prefilled(teacher, encoding, u1, u2, ar_prec, prefix, args.chunk, args.pool_stride)
+            elif args.chunk:
                 regen = generate_chunked(teacher, encoding, u1, u2, ar_prec, prefix, args.chunk, args.pool_stride)
             else:
                 regen = teacher.generate(encoding, u1=u1, u2=u2, precision=ar_prec, zero_last=True, prefix=prefix)
