@@ -162,7 +162,7 @@ int srwn_teacher_generate(srwn_handle_t h, const float* enc, const float* u1,
  * srwn_generate_state_bytes: size of the state of B utterances for `precision` (SRWN_FP32 or SRWN_FP16); it does not
  *   depend on T.  It holds the dilation queues in the layout of the precision's kernel (fp16: ceil(B/8) * sum(d) * 512
  *   bytes; fp32: B * sum(d) * 32 floats), x[t-1] and x[t-2] of each utterance, the position t0 of the next step and a
- *   signature (B, precision, layers, sum(d), pool_stride).
+ *   signature (B, precision, layers, sum(d), pool_stride).  Its first 8 bytes are t0, an int64.
  * srwn_generate_state_reset: zero queues and x history, t0 = 0 (the zero padding of ops.py:9).  A state is used only on
  *   the handle, B and precision it was last reset for; any other call is refused with SRWN_ERR_INVALID.
  * srwn_teacher_generate_resume: steps t0 .. t0+T-1, t0 read from the state on the device (no host synchronisation);

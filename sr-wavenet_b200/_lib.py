@@ -6,7 +6,7 @@ import ctypes
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("SRWN_LIB") or os.path.join(_HERE, "libsrwn.so")   # SRWN_LIB: tuning builds (tools/exp_build.sh)
+LIB_PATH = os.environ.get("SRWN_LIB") or os.path.join(_HERE, "libsrwn.so")   # SRWN_LIB: tuning builds (tools/exp_build.sh <source.cu> <name> [flags])
 
 ABI_VERSION = 7      # SRWN_ABI_VERSION in include/srwn.h
 OK, ERR_INVALID, ERR_CUDA, ERR_WEIGHTS, ERR_UNSUPPORTED, ERR_WORKSPACE = range(6)

@@ -1,11 +1,10 @@
 // C-ABI entry points: lifetime, weights, workspace sizing, dispatch (include/srwn.h).
 #include "common.cuh"
+#include "gen_state.cuh"
 #include <atomic>
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
-#include <map>
-#include <mutex>
 #include <new>
 
 static thread_local char g_err[512] = "";
@@ -237,11 +236,9 @@ extern "C" int srwn_create(const srwn_config_t* cfg, srwn_handle_t* out) {
   return SRWN_OK;
 }
 
-static void forget_states(const srwn_ctx* h);
-
 extern "C" int srwn_destroy(srwn_handle_t h) {
   if (!h) return SRWN_OK;
-  forget_states(h);
+  gen_state_forget(h);
   if (h->prof_ev[0]) { cudaEventDestroy(h->prof_ev[0]); cudaEventDestroy(h->prof_ev[1]); }
   cudaFree(h->d_ar_packed); cudaFree(h->d_part);
   if (h->h_err) cudaFreeHost(h->h_err);
@@ -354,7 +351,7 @@ static F32Ws carve_f32(const srwn_ctx* c, int op, int B, int T, void* ws, size_t
   return r;
 }
 
-static int check_bt(const srwn_ctx* c, int B, int T) {
+int check_bt(const srwn_ctx* c, int B, int T) {
   if (B < 1 || T < 1) return srwn_fail(SRWN_ERR_INVALID, "B and T must be positive");
   if (T % c->cfg.pool_stride != 0)
     return srwn_fail(SRWN_ERR_INVALID, "T=%d must be a multiple of pool_stride=%d (model.py:183)", T,
@@ -540,145 +537,42 @@ extern "C" int srwn_teacher_generate(srwn_handle_t h, const float* enc, const fl
   int rc = check_bt(h, B, T);
   if (rc) return rc;
   if (precision == SRWN_FP16)
-    return run_ar_mma(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, nullptr);
+    return run_ar_mma(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, nullptr,
+                      nullptr, 0);
   if (precision != SRWN_FP32)
     return srwn_fail(SRWN_ERR_UNSUPPORTED, "generation runs in fp32 (FFMA kernel) or fp16 (tensor-core kernel)");
   return run_ar_generate(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes,
-                         (cudaStream_t)stream, nullptr);
+                         (cudaStream_t)stream, nullptr, nullptr, 0);
 }
 
-// ---- resumable generation -----------------------------------------------------------------
-// State buffer: header (t0 + signature) | x history [B][2] fp32 | dilation queues of the precision's kernel.
-struct GenStateHeader {
-  long long t0;               // position of the next step
-  int32_t sig[6];             // B, precision, n_layers, sum of dilations, pool_stride, kStateMagic
-};
-static const int32_t kStateMagic = 0x5357534e;
-struct GenStateLayout { size_t xhist, queues, bytes; };
-
-static GenStateLayout gen_state_layout(const srwn_ctx* c, int B, int precision) {
-  GenStateLayout r;
-  r.xhist = 256;                                                        // header, padded to the carving granule
-  r.queues = r.xhist + (((size_t)B * 2 * sizeof(float) + 255) & ~(size_t)255);
-  r.bytes = r.queues + (precision == SRWN_FP16 ? ar_mma_queue_bytes(c, B) : ar_queue_bytes(c, B));
-  return r;
-}
-
-static void state_signature(const srwn_ctx* c, int B, int precision, int32_t* sig) {
-  const int32_t v[6] = {B, precision, c->cfg.n_layers, c->sum_dilation, c->cfg.pool_stride, kStateMagic};
-  memcpy(sig, v, sizeof(v));
-}
-
-// The signature is also kept on the host, per state buffer, so that a call can refuse a state made for another handle,
-// batch size or precision without reading the device copy (which would synchronise the stream).
-struct StateOwner { const srwn_ctx* h; int32_t sig[6]; };
-static std::mutex g_states_mu;
-static std::map<const void*, StateOwner> g_states;
-
-static void forget_states(const srwn_ctx* h) {
-  std::lock_guard<std::mutex> lk(g_states_mu);
-  for (auto it = g_states.begin(); it != g_states.end();) it = it->second.h == h ? g_states.erase(it) : std::next(it);
-}
-
-static int check_state_args(srwn_handle_t h, int B, int precision, const char* fn) {
-  if (!h) return srwn_fail(SRWN_ERR_INVALID, "%s: null handle", fn);
-  if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-  if (B < 1) return srwn_fail(SRWN_ERR_INVALID, "%s: B must be positive", fn);
-  if (precision == SRWN_FP16 && !ar_mma_supported(h))
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "fp16 generation kernel does not cover this configuration");
-  if (precision != SRWN_FP32 && precision != SRWN_FP16)
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "generation runs in fp32 (FFMA kernel) or fp16 (tensor-core kernel)");
-  return SRWN_OK;
-}
-
-extern "C" int srwn_generate_state_bytes(srwn_handle_t h, int32_t B, int32_t precision, size_t* bytes) {
-  if (!bytes) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_bytes: null argument");
-  int rc = check_state_args(h, B, precision, "srwn_generate_state_bytes");
-  if (rc) return rc;
-  *bytes = gen_state_layout(h, B, precision).bytes;
-  return SRWN_OK;
-}
-
-extern "C" int srwn_generate_state_reset(srwn_handle_t h, void* state, int32_t B, int32_t precision, void* stream) {
-  if (!state) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_reset: null state");
-  int rc = check_state_args(h, B, precision, "srwn_generate_state_reset");
-  if (rc) return rc;
-  GenStateHeader hdr{};
-  state_signature(h, B, precision, hdr.sig);
-  const cudaStream_t st = (cudaStream_t)stream;
-  uint8_t* base = static_cast<uint8_t*>(state);
-  SRWN_CUDA(cudaMemsetAsync(base, 0, gen_state_layout(h, B, precision).bytes, st));      // zero padding of ops.py:9
-  // pageable source: the copy is staged before this call returns, so `hdr` may go out of scope
-  SRWN_CUDA(cudaMemcpyAsync(base, &hdr, sizeof(hdr), cudaMemcpyHostToDevice, st));
-  std::lock_guard<std::mutex> lk(g_states_mu);
-  StateOwner& o = g_states[state];
-  o.h = h;
-  memcpy(o.sig, hdr.sig, sizeof(hdr.sig));
-  return SRWN_OK;
-}
-
-// Refuses a state that was not last reset on this handle for this B and precision (host-side signature: no synchronisation).
-static int check_state_owner(srwn_handle_t h, const void* state, int B, int precision) {
-  int32_t sig[6];
-  state_signature(h, B, precision, sig);
-  std::lock_guard<std::mutex> lk(g_states_mu);
-  auto it = g_states.find(state);
-  if (it == g_states.end() || it->second.h != h)
-    return srwn_fail(SRWN_ERR_INVALID, "state was not reset on this handle (srwn_generate_state_reset)");
-  if (memcmp(it->second.sig, sig, sizeof(sig)))
-    return srwn_fail(SRWN_ERR_INVALID, "state was made for B=%d, precision %d; this call has B=%d, precision %d",
-                     it->second.sig[0], it->second.sig[1], B, precision);
-  return SRWN_OK;
-}
-
-static GenResume state_parts(const srwn_ctx* h, void* state, int B, int precision) {
-  uint8_t* base = static_cast<uint8_t*>(state);
-  const GenStateLayout lay = gen_state_layout(h, B, precision);
-  GenResume rs;
-  rs.t0 = &reinterpret_cast<GenStateHeader*>(base)->t0;
-  rs.xhist = reinterpret_cast<float*>(base + lay.xhist);
-  rs.queues = base + lay.queues;
-  rs.x_prefix = nullptr;
-  rs.n_prefix = 0;
-  return rs;
-}
-
+// ---- resumable generation (state format: gen_state.cu) ------------------------------------
 extern "C" int srwn_teacher_generate_resume(srwn_handle_t h, void* state, const float* enc, const float* u1,
                                             const float* u2, const float* x_prefix, int32_t n_prefix, float* x_out,
                                             float* logits_out, int32_t B, int32_t T, int32_t precision, void* workspace,
                                             size_t workspace_bytes, void* stream) {
   if (!h || !state || !enc || !u1 || !u2 || !x_out)
     return srwn_fail(SRWN_ERR_INVALID, "srwn_teacher_generate_resume: null argument");
-  int rc = check_state_args(h, B, precision, "srwn_teacher_generate_resume");
-  if (rc) return rc;
-  rc = check_bt(h, B, T);
+  GenState s;
+  int rc = gen_state_open(h, state, B, T, precision, &s);
   if (rc) return rc;
   if (n_prefix < 0 || n_prefix > T || (n_prefix > 0 && !x_prefix))
     return srwn_fail(SRWN_ERR_INVALID, "n_prefix=%d must be in [0, T=%d], with x_prefix given when > 0", n_prefix, T);
-  rc = check_state_owner(h, state, B, precision);
-  if (rc) return rc;
-  GenResume rs = state_parts(h, state, B, precision);
-  rs.x_prefix = n_prefix > 0 ? x_prefix : nullptr;
-  rs.n_prefix = n_prefix;
+  if (n_prefix == 0) x_prefix = nullptr;
   if (precision == SRWN_FP16)
-    return run_ar_mma(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, &rs);
-  return run_ar_generate(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, &rs);
+    return run_ar_mma(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, &s,
+                      x_prefix, n_prefix);
+  return run_ar_generate(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, &s,
+                         x_prefix, n_prefix);
 }
 
 extern "C" int srwn_generate_state_prefill(srwn_handle_t h, void* state, const float* x, const float* enc, int32_t n,
                                            int32_t B, int32_t precision, void* workspace, size_t workspace_bytes,
                                            void* stream) {
   if (!h || !state || !x || !enc) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_prefill: null argument");
-  int rc = check_state_args(h, B, precision, "srwn_generate_state_prefill");
+  GenState s;
+  int rc = gen_state_open(h, state, B, n, precision, &s);   // n % P == 0 keeps t0 on a frame boundary for later calls
   if (rc) return rc;
-  rc = check_bt(h, B, n);                     // n % P == 0 keeps t0 on a frame boundary for later resume calls
-  if (rc) return rc;
-  rc = check_state_owner(h, state, B, precision);
-  if (rc) return rc;
-  GenResume rs = state_parts(h, state, B, precision);
-  rs.x_prefix = x;
-  rs.n_prefix = n;
-  return run_prefill(h, x, enc, B, n, precision, workspace, workspace_bytes, (cudaStream_t)stream, rs);
+  return run_prefill(h, s, x, enc, B, n, precision, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // ---- student --------------------------------------------------------------------------

@@ -5,12 +5,8 @@
 // pop + one push of R floats per layer (SURVEY.md 3.2 / 8(d) cfg4).  One persistent CTA owns
 // U utterances for all T steps; weights stay in L2 and are streamed every step.
 #include "common.cuh"
+#include "gen_state.cuh"
 #include "mol.cuh"
-
-// k_cond is defined in stack_f32.cu
-__global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ cond_k,
-                       const float* __restrict__ cond_b, float* __restrict__ cond,
-                       int frames_total, int L, int C);
 
 struct ArParams {
   const float* w;            // stack weights (fp32 arena)
@@ -71,7 +67,7 @@ __global__ void __launch_bounds__(256, 1) k_ar_generate(const ArParams p) {
         if (own) {
           const int d = p.dil[l];
           const int slot = RESUME ? (int)((t0 + t) % d) : t % d;
-          float* q = p.queues + ((size_t)ub * p.sum_d + p.qoff[l] + slot) * kR + lane;
+          float* q = p.queues + gen_f32_row(ub, p.sum_d, p.qoff[l], slot) * kR + lane;
           tap = *q;
           *q = hreg;
         }
@@ -202,47 +198,35 @@ __global__ void __launch_bounds__(256, 1) k_ar_generate(const ArParams p) {
   if (RESUME && own && lane == 0) { p.xhist[2 * ub] = xm1; p.xhist[2 * ub + 1] = xm2; }
 }
 
-__global__ void k_gen_state_advance(long long* t0, int T) { *t0 += T; }
-
-int run_gen_state_advance(long long* t0, int T, cudaStream_t st) {
-  k_gen_state_advance<<<1, 1, 0, st>>>(t0, T);
-  SRWN_LAUNCH_CHECK();
-  return SRWN_OK;
-}
-
-// dilation queues of B utterances: sum_d rows of R floats each
-size_t ar_queue_bytes(const srwn_ctx* c, int B) { return (size_t)B * c->sum_dilation * kR * sizeof(float); }
-
 size_t ar_workspace_bytes(const srwn_ctx* c, int B, int T) {
   WsCarver w(nullptr, 0);
-  w.take<uint8_t>(ar_queue_bytes(c, B));
+  w.take<uint8_t>(gen_queue_bytes(c, B, SRWN_FP32));
   w.take<float>((size_t)B * (T / c->cfg.pool_stride) * c->cfg.n_layers * kR);
   return w.used;
 }
 
 int run_ar_generate(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
-                    float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenResume* rs) {
+                    float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenState* rs,
+                    const float* x_prefix, int n_prefix) {
   if (!ws || ws_bytes < ar_workspace_bytes(c, B, T))
     return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", ar_workspace_bytes(c, B, T));
   WsCarver w(ws, ws_bytes);
   const int frames = T / c->cfg.pool_stride;
-  float* queues = reinterpret_cast<float*>(w.take<uint8_t>(ar_queue_bytes(c, B)));
+  const size_t queue_bytes = gen_queue_bytes(c, B, SRWN_FP32);
+  void* queues = w.take<uint8_t>(queue_bytes);
   float* cond = w.take<float>((size_t)B * frames * c->cfg.n_layers * kR);
-  if (!rs) SRWN_CUDA(cudaMemsetAsync(queues, 0, ar_queue_bytes(c, B), st));
+  if (!rs) SRWN_CUDA(cudaMemsetAsync(queues, 0, queue_bytes, st));
+  const GenState s = rs ? *rs : GenState{nullptr, nullptr, queues};   // one call from silence: the zeroed workspace queues
   const float* sw = stack_w(c, 0);
   k_cond<<<B * frames, 256, 0, st>>>(enc, sw + c->off.cond_k, sw + c->off.cond_b, cond, B * frames,
                                      c->cfg.n_layers, c->cfg.cond_channels);
   SRWN_LAUNCH_CHECK();
   ArParams p;
   p.w = sw; p.off = c->off; p.dil = c->d_dilations; p.qoff = c->d_queue_off;
-  p.queues = queues; p.cond = cond; p.u1 = u1; p.u2 = u2; p.x_out = x_out; p.logits_out = logits_out;
+  p.queues = static_cast<float*>(s.queues); p.cond = cond; p.u1 = u1; p.u2 = u2; p.x_out = x_out; p.logits_out = logits_out;
   p.B = B; p.T = T; p.L = c->cfg.n_layers; p.P = c->cfg.pool_stride; p.frames = frames;
   p.M = c->cfg.num_mixtures; p.sum_d = c->sum_dilation;
-  p.t0 = nullptr; p.xhist = nullptr; p.x_prefix = nullptr; p.n_prefix = 0;
-  if (rs) {
-    p.queues = static_cast<float*>(rs->queues); p.t0 = rs->t0; p.xhist = rs->xhist;
-    p.x_prefix = rs->x_prefix; p.n_prefix = rs->n_prefix;
-  }
+  p.t0 = s.t0; p.xhist = s.xhist; p.x_prefix = x_prefix; p.n_prefix = n_prefix;
   {
     ProfScope prof(c, st, "k_ar_generate", 1);
     const bool two = B > c->sm_count;
@@ -254,6 +238,5 @@ int run_ar_generate(srwn_ctx* c, const float* enc, const float* u1, const float*
     }
     SRWN_LAUNCH_CHECK();
   }
-  if (rs) return run_gen_state_advance(rs->t0, T, st);
-  return SRWN_OK;
+  return rs ? run_gen_state_advance(s.t0, T, st) : SRWN_OK;
 }

@@ -25,23 +25,11 @@
 #include <vector>
 #include <cstdio>
 
-const float* srwn_host_weights(srwn_ctx* c);
-__global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ cond_k,
-                       const float* __restrict__ cond_b, float* __restrict__ cond,
-                       int frames_total, int L, int C);
-namespace fused {
-__global__ void k_fold_bias(const float* __restrict__ cond, const float* __restrict__ front_b,
-                            const float* __restrict__ res_b, float* __restrict__ cb, int L);
-}
-
 namespace armma {
 
-constexpr int kU = 8;                         // utterances per CTA
 constexpr int kMaxL = 30;                     // chain weights of 30 layers fill shared memory
-constexpr int kChainLayerBytes = 4096 + 2048 + 128;   // Wf fragments | Wr fragments | filter bias (fp32)
 constexpr int kItemBytes = 8192;              // one ring item: skip weights of a layer / a quarter of H1 / H2
 constexpr int kStages = 3;
-constexpr int kSlotBytes = 512;               // gate output of one layer: [lane][4 x b32]
 constexpr int kThreads = 9 * 32;
 constexpr int kChainWarps = 4, kProducerWarp = 4, kSkipWarps = 4;   // warps 0..3: chain (one per SMSP), 4: producer, 5..8: skip warps
 
@@ -105,13 +93,6 @@ __device__ __forceinline__ bool mbar_wait(uint32_t a, uint32_t parity, volatile 
 }
 __device__ __forceinline__ void mbar_arrive(uint32_t a) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(a) : "memory");
-}
-// D(16x8, fp32) += A(16x16, fp16, row) * B(16x8, fp16, col); rows 8..15 of A are zero padding (a1 = a3 = 0)
-__device__ __forceinline__ void mma8(float (&d)[2], uint32_t a0, uint32_t a2, uint32_t b0, uint32_t b1) {
-  float z0 = 0.f, z1 = 0.f;
-  asm("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(z0), "+f"(z1)
-               : "r"(a0), "r"(0u), "r"(a2), "r"(0u), "r"(b0), "r"(b1));
 }
 __device__ __forceinline__ uint4 lds128(uint32_t a) {
   uint4 v;
@@ -344,8 +325,8 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
       float hj0 = j == 0 ? h[0][0] : j == 1 ? h[1][0] : j == 2 ? h[2][0] : h[3][0];      // this warp's part of the fp32 stream
       float hj1 = j == 0 ? h[0][1] : j == 1 ? h[1][1] : j == 2 ? h[2][1] : h[3][1];
       // filter-conv B fragments of this warp's n-tile: [taps k-tiles 0,1 | current k-tiles 2,3]
-      uint4 wft = lds128_ro(sbase + Smem::chain + lane * 16 + (2 * j) * 512);
-      uint4 wfc = lds128_ro(sbase + Smem::chain + lane * 16 + (2 * j + 1) * 512);
+      uint4 wft = lds128_ro(sbase + Smem::chain + lane * 16 + (2 * j) * kFragBytes);
+      uint4 wfc = lds128_ro(sbase + Smem::chain + lane * 16 + (2 * j + 1) * kFragBytes);
 
       // Register quads of the A operands (a0, a1, a2, a3); a1 / a3 are don't-care (see mma8q).  The 16 bytes a lane
       // keeps per queue slot / gate slot are ordered {k-tile 0: a0, k-tile 1: a0, k-tile 0: a2, k-tile 1: a2}, so the
@@ -364,20 +345,20 @@ __global__ void __launch_bounds__(kThreads, 1) k_ar_mma(const Params p) {
         mma8q(acc, S.tap.y, dm[2], S.tap.w, dm[3], wft.z, wft.w);
         AR_T(t_1, S.tap.x);
         AR_T(t_2, __float_as_uint(acc[0] + acc2[0]));
-        const uint4 wrj = lds128_ro(wl + 4096 + j * 512); // residual B fragments of n-tile j: land while the gate runs
+        const uint4 wrj = lds128_ro(wl + kChainWr + j * kFragBytes); // residual B fragments of n-tile j: land while the gate runs
         // push h[t] (the slot held h[t-d] until now); every chain warp holds the same image
-        if (j == 0) *reinterpret_cast<uint4*>(qbase + S.ofs) = make_uint4(hA[0], hA[2], hA[1], hA[3]);
+        if (j == 0) *reinterpret_cast<uint4*>(qbase + S.ofs) = gen_f16_pack(hA);
         if (l + 3 < L) prefetch(S, l + 3, sqt);          // this set's next use: layer l + 3
         // ---- gate (ops.py:28,33,36) of this warp's 8 channels -> one word of the A fragments of the residual / skip convs
         {
-          const float2 b = *reinterpret_cast<const float2*>(reinterpret_cast<const float*>(smem + Smem::chain + l * kChainLayerBytes + 6144) + 8 * j + 2 * q);
+          const float2 b = *reinterpret_cast<const float2*>(reinterpret_cast<const float*>(smem + Smem::chain + l * kChainLayerBytes + kChainBias) + 8 * j + 2 * q);
           const uint32_t cj = pack_h2(gate(acc[0] + acc2[0] + b.x), gate(acc[1] + acc2[1] + b.y));
           asm volatile("st.shared.u32 [%0], %1;" ::"r"(sbase + Smem::cslots + l * kSlotBytes + lane * 16 + cpos), "r"(cj) : "memory");
         }
         AR_T(t_3, 0u);
         if (l + 1 < L) {                                 // next layer's filter-conv fragments
-          wft = lds128_ro(wl + kChainLayerBytes + (2 * j) * 512);
-          wfc = lds128_ro(wl + kChainLayerBytes + (2 * j + 1) * 512);
+          wft = lds128_ro(wl + kChainLayerBytes + (2 * j) * kFragBytes);
+          wfc = lds128_ro(wl + kChainLayerBytes + (2 * j + 1) * kFragBytes);
         }
         chain_sync();                                    // the four words of every lane's slot are in place
         AR_T(t_4, 0u);
@@ -631,12 +612,12 @@ int ar_mma_pack_weights(srwn_ctx* c, cudaStream_t st) {
     uint8_t* cl = chain + (size_t)l * armma::kChainLayerBytes;
     const float* fk = w + o.filt_k + (size_t)l * 2 * kR * kR;      // [2][Cin][Cout] = K 64 x N 32
     for (int j = 0; j < 4; j++) {
-      pack_frag_pair(cl + (2 * j) * 512, fk, kR, 64, 32, 0, j);
-      pack_frag_pair(cl + (2 * j + 1) * 512, fk, kR, 64, 32, 2, j);
+      pack_frag_pair(cl + (2 * j) * armma::kFragBytes, fk, kR, 64, 32, 0, j);
+      pack_frag_pair(cl + (2 * j + 1) * armma::kFragBytes, fk, kR, 64, 32, 2, j);
     }
     const float* rk = w + o.res_k + (size_t)l * kR * kR;
-    for (int j = 0; j < 4; j++) pack_frag_pair(cl + 4096 + j * 512, rk, kR, 32, 32, 0, j);
-    memcpy(cl + 6144, w + o.filt_b + (size_t)l * kR, 32 * 4);
+    for (int j = 0; j < 4; j++) pack_frag_pair(cl + armma::kChainWr + j * armma::kFragBytes, rk, kR, 32, 32, 0, j);
+    memcpy(cl + armma::kChainBias, w + o.filt_b + (size_t)l * kR, 32 * 4);
     uint8_t* it = stream + (size_t)l * armma::kItemBytes;           // skip weights, transposed: [warp][m-tile][k-tile]
     const float* sk = w + o.skip_k + (size_t)l * kR * kS;
     for (int sw = 0; sw < 4; sw++)
@@ -665,17 +646,12 @@ int ar_mma_pack_weights(srwn_ctx* c, cudaStream_t st) {
 
 struct ArMmaWs { uint8_t* queues; float *cond, *cb, *g1, *lg2; int* err; size_t bytes; int grid; };
 
-// dilation queues of B utterances: one block of sum_d slots per CTA of 8 utterances
-size_t ar_mma_queue_bytes(const srwn_ctx* c, int B) {
-  return (size_t)((B + armma::kU - 1) / armma::kU) * c->sum_dilation * armma::kSlotBytes;
-}
-
 static ArMmaWs carve_ar_mma(const srwn_ctx* c, int B, int T, void* ws, size_t cap) {
   WsCarver w(ws, cap);
   ArMmaWs r{};
   const size_t frames = T / c->cfg.pool_stride, L = c->cfg.n_layers;
   r.grid = (B + armma::kU - 1) / armma::kU;
-  r.queues = w.take<uint8_t>(ar_mma_queue_bytes(c, B));
+  r.queues = w.take<uint8_t>(gen_queue_bytes(c, B, SRWN_FP16));
   r.cond = w.take<float>((size_t)B * frames * L * 32);
   r.cb = w.take<float>((size_t)B * frames * (L + 1) * 32);
   r.g1 = w.take<float>((size_t)B * T * c->cfg.num_mixtures);
@@ -688,13 +664,15 @@ static ArMmaWs carve_ar_mma(const srwn_ctx* c, int B, int T, void* ws, size_t ca
 size_t ar_mma_workspace_bytes(const srwn_ctx* c, int B, int T) { return carve_ar_mma(c, B, T, nullptr, 0).bytes; }
 
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
-               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenResume* rs) {
+               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenState* rs,
+               const float* x_prefix, int n_prefix) {
   if (!ar_mma_supported(c) || !c->d_ar_packed)
     return srwn_fail(SRWN_ERR_UNSUPPORTED, "fp16 generation kernel supports up to %d layers and 6 mixtures", armma::kMaxL);
   ArMmaWs w = carve_ar_mma(c, B, T, ws, ws_bytes);
   if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
   const int L = c->cfg.n_layers, frames = T / c->cfg.pool_stride;
-  if (!rs) SRWN_CUDA(cudaMemsetAsync(w.queues, 0, ar_mma_queue_bytes(c, B), st));   // zero padding of ops.py:9
+  if (!rs) SRWN_CUDA(cudaMemsetAsync(w.queues, 0, gen_queue_bytes(c, B, SRWN_FP16), st));   // zero padding of ops.py:9
+  const GenState s = rs ? *rs : GenState{nullptr, nullptr, w.queues};   // one call from silence: the zeroed workspace queues
   SRWN_CUDA(cudaMemsetAsync(w.err, 0, 16, st));
   const float* sw = stack_w(c, 0);
   k_cond<<<B * frames, 256, 0, st>>>(enc, sw + c->off.cond_k, sw + c->off.cond_b, w.cond, B * frames, L, c->cfg.cond_channels);
@@ -712,7 +690,7 @@ int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, 
   p.chain_w = img;
   p.stream = img + (size_t)L * armma::kChainLayerBytes;
   p.fixed = reinterpret_cast<const float*>(p.stream + (size_t)(L + 5) * armma::kItemBytes);
-  p.cb = w.cb; p.queues = w.queues; p.g1 = w.g1; p.lg2 = w.lg2; p.x_out = x_out; p.logits_out = logits_out; p.err = w.err;
+  p.cb = w.cb; p.queues = static_cast<uint8_t*>(s.queues); p.g1 = w.g1; p.lg2 = w.lg2; p.x_out = x_out; p.logits_out = logits_out; p.err = w.err;
   p.B = B; p.T = T; p.L = L; p.P = c->cfg.pool_stride; p.frames = frames; p.M = c->cfg.num_mixtures;
   bool pow2 = true;
   int off = 0;
@@ -721,10 +699,7 @@ int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, 
     if (c->dilations[l] & (c->dilations[l] - 1)) pow2 = false;
   }
   p.sum_d = pow2 ? -c->sum_dilation : c->sum_dilation;
-  if (rs) {
-    p.queues = static_cast<uint8_t*>(rs->queues); p.t0 = rs->t0; p.xhist = rs->xhist;
-    p.x_prefix = rs->x_prefix; p.n_prefix = rs->n_prefix;
-  }
+  p.t0 = s.t0; p.xhist = s.xhist; p.x_prefix = x_prefix; p.n_prefix = n_prefix;
   auto kernel = rs ? armma::k_ar_mma<true> : armma::k_ar_mma<false>;
   SRWN_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, armma::Smem::total));
   {
@@ -732,8 +707,7 @@ int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, 
     kernel<<<w.grid, armma::kThreads, armma::Smem::total, st>>>(p);
     SRWN_LAUNCH_CHECK();
   }
-  if (rs) return run_gen_state_advance(rs->t0, T, st);
-  return SRWN_OK;
+  return rs ? run_gen_state_advance(s.t0, T, st) : SRWN_OK;
 }
 
 int ar_mma_check_error(const srwn_ctx* c, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {

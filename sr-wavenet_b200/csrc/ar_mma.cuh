@@ -4,8 +4,17 @@
 #pragma once
 #include <cuda_fp16.h>
 #include <stdint.h>
+#include "gen_state.cuh"
 
 namespace armma {
+
+constexpr int kU = kGenGroup;                         // utterances per CTA: one group of the fp16 queues
+constexpr int kSlotBytes = kGenSlotBytes;             // queue slot / gate output of one layer: [lane][4 x b32]
+// A layer's chain image (ar_mma_pack_weights): filter-conv B fragment pairs 2j (taps) and 2j + 1 (current) of n-tile j |
+// residual-conv B fragment pairs j | filter bias (32 fp32).  A fragment pair is 32 lanes x 16 bytes.
+constexpr int kFragBytes = 512;
+constexpr int kChainWr = 8 * kFragBytes, kChainBias = kChainWr + 4 * kFragBytes;
+constexpr int kChainLayerBytes = kChainBias + 32 * 4;
 
 __device__ __forceinline__ uint32_t pack_h2(float a, float b) {
   __half2 h = __floats2half2_rn(a, b);

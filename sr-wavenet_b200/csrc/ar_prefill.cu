@@ -22,22 +22,13 @@
 //     operands, which the GPU tests check by equality.
 //   * fp32 (k_ar_generate): the FFMA sums in the step kernel's order.
 #include "common.cuh"
+#include "gen_state.cuh"
 #include "ar_mma.cuh"
 #include <algorithm>
-
-__global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ cond_k,
-                       const float* __restrict__ cond_b, float* __restrict__ cond,
-                       int frames_total, int L, int C);
-namespace fused {
-__global__ void k_fold_bias(const float* __restrict__ cond, const float* __restrict__ front_b,
-                            const float* __restrict__ res_b, float* __restrict__ cb, int L);
-}
 
 namespace prefill {
 
 constexpr int kThreads = 256;
-constexpr int kSlotBytes = 512;            // fp16 queue slot of 8 utterances (ar_mma.cu)
-constexpr int kChainLayerBytes = 4096 + 2048 + 128;
 
 // Rows of the window: buffer row r is position i = base + r of the call (i < 0 lies before t0).  The fp16 buffers keep
 // a lane's eight channels together: float q*8 + k of a row is channel 8*(k/2) + 2q + (k%2), i.e. n-tile k/2 of the
@@ -54,11 +45,6 @@ struct Layer {
   int B, Bp, Wr, base, r0, l, L, d, qoff, sum_d, P, fb, NF;
 };
 
-__device__ __forceinline__ int slot_of(const long long* t0, int i, int d) {
-  const long long t = *t0 + i;
-  return (int)(((t % d) + d) % d);
-}
-
 // ---- fp16: one warp per tile of 16 consecutive positions of one utterance ------------------------------------------
 __global__ void __launch_bounds__(kThreads) k_prefill_mma(const Layer p) {
   using namespace armma;
@@ -68,11 +54,11 @@ __global__ void __launch_bounds__(kThreads) k_prefill_mma(const Layer p) {
   float fb[8];
 #pragma unroll
   for (int j = 0; j < 4; j++) {
-    wft[j] = *reinterpret_cast<const uint4*>(p.chain + (2 * j) * 512 + lane * 16);
-    wfc[j] = *reinterpret_cast<const uint4*>(p.chain + (2 * j + 1) * 512 + lane * 16);
-    wr[j] = *reinterpret_cast<const uint4*>(p.chain + 4096 + j * 512 + lane * 16);
-    fb[2 * j] = reinterpret_cast<const float*>(p.chain + 6144)[8 * j + 2 * q];
-    fb[2 * j + 1] = reinterpret_cast<const float*>(p.chain + 6144)[8 * j + 2 * q + 1];
+    wft[j] = *reinterpret_cast<const uint4*>(p.chain + (2 * j) * kFragBytes + lane * 16);
+    wfc[j] = *reinterpret_cast<const uint4*>(p.chain + (2 * j + 1) * kFragBytes + lane * 16);
+    wr[j] = *reinterpret_cast<const uint4*>(p.chain + kChainWr + j * kFragBytes + lane * 16);
+    fb[2 * j] = reinterpret_cast<const float*>(p.chain + kChainBias)[8 * j + 2 * q];
+    fb[2 * j + 1] = reinterpret_cast<const float*>(p.chain + kChainBias)[8 * j + 2 * q + 1];
   }
   const int rows = p.Wr - p.r0, tpb = (rows + 15) / 16;
   for (int tile = warp; tile < p.Bp * tpb; tile += nwarps) {
@@ -92,10 +78,10 @@ __global__ void __launch_bounds__(kThreads) k_prefill_mma(const Layer p) {
         const float4 t0v = ts[0], t1v = ts[1];
         tap[h][0] = pack_h2(t0v.x, t0v.y); tap[h][1] = pack_h2(t0v.z, t0v.w);
         tap[h][2] = pack_h2(t1v.x, t1v.y); tap[h][3] = pack_h2(t1v.z, t1v.w);
-      } else {                                        // before t0: the state's slot holds the image {0, 2, 1, 3}
-        const uint4 s = *reinterpret_cast<const uint4*>(static_cast<const uint8_t*>(p.queues) +
-            ((size_t)(b >> 3) * p.sum_d + p.qoff + slot_of(p.t0, i, p.d)) * kSlotBytes + ((b & 7) * 4 + q) * 16);
-        tap[h][0] = s.x; tap[h][1] = s.z; tap[h][2] = s.y; tap[h][3] = s.w;
+      } else {                                        // before t0: the state's slot
+        gen_f16_unpack(*reinterpret_cast<const uint4*>(static_cast<const uint8_t*>(p.queues) +
+                                                       gen_f16_offset(b, q, p.sum_d, p.qoff, gen_slot(p.t0, i, p.d))),
+                       tap[h]);
       }
     }
     uint32_t hA[2][4];
@@ -169,7 +155,7 @@ __global__ void __launch_bounds__(kThreads) k_prefill_f32(const Layer p) {
     const int b = row / rows, r = p.r0 + row % rows, i = p.base + r;
     const float cur = p.hin[((size_t)b * p.Wr + r) * kR + lane];
     const float tap = i - p.d >= 0 ? p.hin[((size_t)b * p.Wr + r - p.d) * kR + lane]
-                                   : static_cast<const float*>(p.queues)[((size_t)b * p.sum_d + p.qoff + slot_of(p.t0, i, p.d)) * kR + lane];
+                                   : static_cast<const float*>(p.queues)[gen_f32_row(b, p.sum_d, p.qoff, gen_slot(p.t0, i, p.d)) * kR + lane];
     __syncwarp();
     s_in[wib][0][lane] = tap;
     s_in[wib][1][lane] = cur;
@@ -229,11 +215,9 @@ __global__ void k_prefill_commit_mma(const float* __restrict__ h, uint8_t* __res
   const int q = (int)(idx & 3), r = r0 + (int)((idx >> 2) % rows), b = (int)((idx >> 2) / rows);
   const float4* src = reinterpret_cast<const float4*>(h + ((size_t)b * Wr + r) * kR + q * 8);
   const float4 v0 = src[0], v1 = src[1];
-  // the step kernel's image of a lane: words of n-tiles {0, 2, 1, 3}
-  const uint4 s = make_uint4(armma::pack_h2(v0.x, v0.y), armma::pack_h2(v1.x, v1.y), armma::pack_h2(v0.z, v0.w),
-                             armma::pack_h2(v1.z, v1.w));
-  *reinterpret_cast<uint4*>(queues + ((size_t)(b >> 3) * sum_d + qoff + slot_of(t0, base + r, d)) * kSlotBytes +
-                            ((b & 7) * 4 + q) * 16) = s;
+  const uint32_t w[4] = {armma::pack_h2(v0.x, v0.y), armma::pack_h2(v0.z, v0.w), armma::pack_h2(v1.x, v1.y),
+                         armma::pack_h2(v1.z, v1.w)};
+  *reinterpret_cast<uint4*>(queues + gen_f16_offset(b, q, sum_d, qoff, gen_slot(t0, base + r, d))) = gen_f16_pack(w);
 }
 
 __global__ void k_prefill_commit_f32(const float* __restrict__ h, float* __restrict__ queues, const long long* t0,
@@ -242,7 +226,7 @@ __global__ void k_prefill_commit_f32(const float* __restrict__ h, float* __restr
   const int rows = Wr - r0;
   if (idx >= (int64_t)B * rows * kR) return;
   const int c = (int)(idx % kR), r = r0 + (int)((idx / kR) % rows), b = (int)(idx / ((int64_t)kR * rows));
-  queues[((size_t)b * sum_d + qoff + slot_of(t0, base + r, d)) * kR + c] = h[((size_t)b * Wr + r) * kR + c];
+  queues[gen_f32_row(b, sum_d, qoff, gen_slot(t0, base + r, d)) * kR + c] = h[((size_t)b * Wr + r) * kR + c];
 }
 
 // x history after the prefill: x[E-1], x[E-2]
@@ -292,8 +276,8 @@ size_t prefill_workspace_bytes(const srwn_ctx* c, int B, int n, int precision) {
   return carve_prefill(c, B, n, precision, nullptr).bytes;
 }
 
-int run_prefill(srwn_ctx* c, const float* x, const float* enc, int B, int n, int precision, void* ws, size_t ws_bytes,
-                cudaStream_t st, const GenResume& rs) {
+int run_prefill(srwn_ctx* c, const GenState& s, const float* x, const float* enc, int B, int n, int precision, void* ws,
+                size_t ws_bytes, cudaStream_t st) {
   const bool fp16 = precision == SRWN_FP16;
   if (fp16 && (!ar_mma_supported(c) || !c->d_ar_packed))
     return srwn_fail(SRWN_ERR_UNSUPPORTED, "fp16 prefill needs the tensor-core generation kernel's configuration");
@@ -319,10 +303,10 @@ int run_prefill(srwn_ctx* c, const float* x, const float* enc, int B, int n, int
   {
     const int64_t nt = (int64_t)Bp * Wr * kR;
     if (fp16)
-      prefill::k_prefill_front<true><<<blocks_for(nt, 256), 256, 0, st>>>(x, rs.xhist, sw + c->off.front_k, nullptr, w.cb, w.h[0],
+      prefill::k_prefill_front<true><<<blocks_for(nt, 256), 256, 0, st>>>(x, s.xhist, sw + c->off.front_k, nullptr, w.cb, w.h[0],
                                                                           B, Bp, n, Wr, base, P, fb, NF, L);
     else
-      prefill::k_prefill_front<false><<<blocks_for(nt, 256), 256, 0, st>>>(x, rs.xhist, sw + c->off.front_k, sw + c->off.front_b,
+      prefill::k_prefill_front<false><<<blocks_for(nt, 256), 256, 0, st>>>(x, s.xhist, sw + c->off.front_k, sw + c->off.front_b,
                                                                            w.cond, w.h[0], B, Bp, n, Wr, base, P, fb, NF, L);
     SRWN_LAUNCH_CHECK();
   }
@@ -331,8 +315,8 @@ int run_prefill(srwn_ctx* c, const float* x, const float* enc, int B, int n, int
     const float* hin = w.h[l & 1];
     if (l + 1 < L) {                                  // h_{l+1} over [n - D_{l+1}, n); the last layer's output is unused
       prefill::Layer p;
-      p.hin = hin; p.hout = w.h[(l + 1) & 1]; p.queues = rs.queues; p.t0 = rs.t0;
-      p.chain = fp16 ? img + (size_t)l * prefill::kChainLayerBytes : nullptr;
+      p.hin = hin; p.hout = w.h[(l + 1) & 1]; p.queues = s.queues; p.t0 = s.t0;
+      p.chain = fp16 ? img + (size_t)l * armma::kChainLayerBytes : nullptr;
       p.w = sw; p.off = c->off; p.cond = fp16 ? w.cb : w.cond;
       p.B = B; p.Bp = Bp; p.Wr = Wr; p.base = base; p.r0 = std::max(0, n - D[l + 1]) - base; p.l = l; p.L = L;
       p.d = c->dilations[l]; p.qoff = qoff[l]; p.sum_d = sum_d; p.P = P; p.fb = fb; p.NF = NF;
@@ -347,13 +331,13 @@ int run_prefill(srwn_ctx* c, const float* x, const float* enc, int B, int n, int
     const int r0 = std::max(0, n - c->dilations[l]) - base;
     if (fp16)
       prefill::k_prefill_commit_mma<<<blocks_for((int64_t)Bp * (Wr - r0) * 4, 256), 256, 0, st>>>(
-          hin, static_cast<uint8_t*>(rs.queues), rs.t0, Bp, Wr, base, r0, c->dilations[l], qoff[l], sum_d);
+          hin, static_cast<uint8_t*>(s.queues), s.t0, Bp, Wr, base, r0, c->dilations[l], qoff[l], sum_d);
     else
       prefill::k_prefill_commit_f32<<<blocks_for((int64_t)B * (Wr - r0) * kR, 256), 256, 0, st>>>(
-          hin, static_cast<float*>(rs.queues), rs.t0, B, Wr, base, r0, c->dilations[l], qoff[l], sum_d);
+          hin, static_cast<float*>(s.queues), s.t0, B, Wr, base, r0, c->dilations[l], qoff[l], sum_d);
     SRWN_LAUNCH_CHECK();
   }
-  prefill::k_prefill_xhist<<<blocks_for(B, 128), 128, 0, st>>>(x, rs.xhist, B, n);
+  prefill::k_prefill_xhist<<<blocks_for(B, 128), 128, 0, st>>>(x, s.xhist, B, n);
   SRWN_LAUNCH_CHECK();
-  return run_gen_state_advance(rs.t0, n, st);
+  return run_gen_state_advance(s.t0, n, st);
 }

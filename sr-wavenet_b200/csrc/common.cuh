@@ -113,18 +113,24 @@ struct WsCarver {
 // on-device noise (philox.cuh): element i of (seed, stream); `on` = 0 means the caller supplied the tensor
 struct NoiseSpec { unsigned long long seed, stream; int on; };
 
-// resumable generation (srwn_teacher_generate_resume): the parts of the caller's state a generation kernel reads and
-// writes, and the samples it forces.  The state's layout is kept in api.cu (gen_state_layout).
-struct GenResume {
+// The parts of a generation state (gen_state.cuh) a generation kernel reads and writes.
+struct GenState {
   long long* t0;              // position of step 0 of the call; advanced by T after the kernel
   float* xhist;               // [B][2]: x[t0-1], x[t0-2]
-  void* queues;               // dilation queues, laid out as the precision's kernel keeps them (ar_queue_bytes / ar_mma_queue_bytes)
-  const float* x_prefix;      // [B][n_prefix], or null when n_prefix == 0
-  int n_prefix;
+  void* queues;               // dilation queues in the precision's layout (gen_state.cuh)
 };
 
-// ---- kernel entry points implemented across translation units ---------------------
+// ---- kernels and entry points implemented across translation units ------------------
+// api.cu
+int check_bt(const srwn_ctx* c, int B, int T);
+const float* srwn_host_weights(srwn_ctx* c);
 // stack_f32.cu
+__global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ cond_k,
+                       const float* __restrict__ cond_b, float* __restrict__ cond,
+                       int frames_total, int L, int C);
+__global__ void k_front(const float* __restrict__ x, const float* __restrict__ fk,
+                        const float* __restrict__ fb, const float* __restrict__ cond,
+                        float* __restrict__ hc, int T, int P, int L, int frames);
 int run_stack_f32(srwn_ctx* c, int stack, const float* xin, const float* enc, int B, int T,
                   float* h0, float* h1, float* skip, float* cond, float** h_final,
                   cudaStream_t st);
@@ -143,12 +149,11 @@ int run_mol_sample(const float* l, const float* u1, const float* u2, float* out,
                    int32_t* idx_out, int B, int T, int M, cudaStream_t st);
 // ar_generate.cu
 size_t ar_workspace_bytes(const srwn_ctx* c, int B, int T);
-size_t ar_queue_bytes(const srwn_ctx* c, int B);
-// rs == null: one call from silence; otherwise resume from (and advance) the caller's state
+// rs == null: one call from silence; otherwise resume from (and advance) the caller's state.  For t < n_prefix, x[t]
+// is x_prefix [B][n_prefix] instead of a draw (resumed calls only).
 int run_ar_generate(srwn_ctx* c, const float* enc, const float* u1, const float* u2,
                     float* x_out, float* logits_out, int B, int T, void* ws, size_t ws_bytes,
-                    cudaStream_t st, const GenResume* rs);
-int run_gen_state_advance(long long* t0, int T, cudaStream_t st);
+                    cudaStream_t st, const GenState* rs, const float* x_prefix, int n_prefix);
 // train_f32.cu
 size_t train_workspace_bytes(const srwn_ctx* c, int B, int T);
 int run_student_forward_train(srwn_ctx* c, const float* z, const float* enc, float* out, float* s_tot,
@@ -166,15 +171,19 @@ int run_adam(srwn_ctx* c, const float* grads, float* m, float* v, float* scratch
 bool ar_mma_supported(const srwn_ctx* c);
 int ar_mma_pack_weights(srwn_ctx* c, cudaStream_t st);
 size_t ar_mma_workspace_bytes(const srwn_ctx* c, int B, int T);
-size_t ar_mma_queue_bytes(const srwn_ctx* c, int B);
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
-               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenResume* rs);
+               float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenState* rs,
+               const float* x_prefix, int n_prefix);
 int ar_mma_check_error(const srwn_ctx* c, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st);
-// ar_prefill.cu: the state srwn_teacher_generate_resume leaves after forcing rs.x_prefix [B][n], computed in parallel
+// ar_prefill.cu: the state srwn_teacher_generate_resume leaves after forcing x [B][n], computed in parallel
 size_t prefill_workspace_bytes(const srwn_ctx* c, int B, int n, int precision);
-int run_prefill(srwn_ctx* c, const float* x, const float* enc, int B, int n, int precision, void* ws, size_t ws_bytes,
-                cudaStream_t st, const GenResume& rs);
+int run_prefill(srwn_ctx* c, const GenState& s, const float* x, const float* enc, int B, int n, int precision, void* ws,
+                size_t ws_bytes, cudaStream_t st);
 // fused.cu
+namespace fused {
+__global__ void k_fold_bias(const float* __restrict__ cond, const float* __restrict__ front_b,
+                            const float* __restrict__ res_b, float* __restrict__ cb, int L);
+}
 bool fused_supported(const srwn_ctx* c);
 size_t fused_packed_bytes(const srwn_ctx* c);
 int fused_pack_weights(srwn_ctx* c, cudaStream_t st);

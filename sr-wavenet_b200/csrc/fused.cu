@@ -34,8 +34,6 @@
 #include <algorithm>
 #include <cstdlib>
 
-const float* srwn_host_weights(srwn_ctx* c);
-
 namespace fused {
 
 constexpr int kTile = 128;

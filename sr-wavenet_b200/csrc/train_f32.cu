@@ -15,13 +15,6 @@
 #include "train_tc.cuh"
 #include <type_traits>
 
-__global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ cond_k,
-                       const float* __restrict__ cond_b, float* __restrict__ cond,
-                       int frames_total, int L, int C);
-__global__ void k_front(const float* __restrict__ x, const float* __restrict__ fk,
-                        const float* __restrict__ fb, const float* __restrict__ cond,
-                        float* __restrict__ hc, int T, int P, int L, int frames);
-
 namespace train {
 
 constexpr int kTT = 64;             // time steps per tile

@@ -1,4 +1,5 @@
-"""Prints the per-phase clock stamps of the tensor-core training kernels (build with -DSRWN_TUNING: tools/exp_build_tune.sh).
+"""Prints the per-phase clock stamps of the tensor-core training kernels (build with -DSRWN_TUNING:
+`tools/exp_build.sh train_tc.cu tune -DSRWN_TUNING`).
 usage: SRWN_LIB=tools/exp/libsrwn_tune.so python tools/tc_trace.py"""
 import ctypes, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
