@@ -85,14 +85,34 @@ struct srwn_ctx {
   const char* prof_name;
 };
 
-// brackets the dominant kernel launches of a call with CUDA events on the launch stream
+// brackets the dominant kernel launches of a call with CUDA events on the launch stream; name == nullptr times nothing
 struct ProfScope {
-  srwn_ctx* c; cudaStream_t st;
-  ProfScope(srwn_ctx* c_, cudaStream_t st_, const char* name, int launches) : c(c_), st(st_) {
-    if (c->profiling) { c->prof_name = name; c->prof_launches = launches; cudaEventRecord(c->prof_ev[0], st); }
+  srwn_ctx* c; cudaStream_t st; bool on;
+  ProfScope(srwn_ctx* c_, cudaStream_t st_, const char* name, int launches) : c(c_), st(st_), on(c_->profiling && name) {
+    if (on) { c->prof_name = name; c->prof_launches = launches; cudaEventRecord(c->prof_ev[0], st); }
   }
-  ~ProfScope() { if (c->profiling) cudaEventRecord(c->prof_ev[1], st); }
+  ~ProfScope() { if (on) cudaEventRecord(c->prof_ev[1], st); }
 };
+
+// ---- programmatic dependent launch (PDL) of the layer kernels -----------------------------------------
+// A layer kernel launched with launch_dependent may start (and stage its weights) while the previous kernel on the stream
+// drains; everything the previous launch wrote is visible after grid_dependency_wait (a no-op in a plain launch).  The
+// trigger right after it lets the NEXT launch's CTAs take the SM slots this grid frees as its CTAs exit (all of this
+// grid's CTAs are resident from the start, so nothing of it can be starved).
+__device__ __forceinline__ void grid_dependency_wait() {
+  asm volatile("griddepcontrol.wait;" ::: "memory");
+  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
+}
+template <typename... KArgs, typename... Args>
+cudaError_t launch_dependent(void (*kern)(KArgs...), int grid, int block, size_t smem, cudaStream_t st, Args... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  attr[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
+}
 
 inline const float* stack_w(const srwn_ctx* c, int stack) {
   return c->d_weights + (size_t)stack * c->stack_floats;
@@ -131,6 +151,7 @@ __global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ 
 __global__ void k_front(const float* __restrict__ x, const float* __restrict__ fk,
                         const float* __restrict__ fb, const float* __restrict__ cond,
                         float* __restrict__ hc, int T, int P, int L, int frames);
+// h1 == nullptr keeps every layer input: h0 is then [L+1][B][T][R] (the training forward, not profiled)
 int run_stack_f32(srwn_ctx* c, int stack, const float* xin, const float* enc, int B, int T,
                   float* h0, float* h1, float* skip, float* cond, float** h_final,
                   cudaStream_t st);

@@ -669,11 +669,7 @@ extern "C" int srwn_encoder_workspace_bytes(srwn_encoder_t e, int32_t B, int32_t
 
 template <bool FRONT>
 static int launch_layer(const srwn_encoder* e, const enc::LayerParams& p, cudaStream_t st) {
-  static bool attr_done = false;
-  if (!attr_done) {
-    SRWN_CUDA(cudaFuncSetAttribute(enc::k_enc_layer<FRONT>, cudaFuncAttributeMaxDynamicSharedMemorySize, enc::Smem::total));
-    attr_done = true;
-  }
+  SRWN_CUDA(cudaFuncSetAttribute(enc::k_enc_layer<FRONT>, cudaFuncAttributeMaxDynamicSharedMemorySize, enc::Smem::total));
   const int grid = p.n_tiles < e->sm_count ? p.n_tiles : e->sm_count;
   enc::k_enc_layer<FRONT><<<grid, enc::kThreads, enc::Smem::total, st>>>(p);
   SRWN_LAUNCH_CHECK();

@@ -1,8 +1,8 @@
 // Student distillation step, device side (fp32 grade): forward that keeps every layer input, and the backward pass
 // of the IAF flows (model.py:415-535) given the gradient of the loss (model.py:356-379) with respect to the
-// network output.  Layer at a time; activations and their gradients round-trip HBM in fp32.  The three per-layer
-// kernels are tcgen05 kernels (train_tc.cu); this file holds the elementwise kernels around them, the teacher's
-// fp32-grade layer kernel (mma.sync, with the skip output) and the host sequence.
+// network output.  Layer at a time; activations and their gradients round-trip HBM in fp32.  The forward is the
+// fp32-grade stack of stack_f32.cu, run so that it keeps every layer input; the two backward layer kernels are tcgen05
+// kernels (train_tc.cu).  This file holds the elementwise kernels around them and the host sequence.
 //
 //   forward (per flow f):  x_0 = front(x_{f-1}) + cond_0;  x_{l+1} = (x_l + Wr c_l + br) sqrt(1/2) + cond_{l+1},
 //                          c_l = f sigmoid(f), f = tanh(W0 x_l[t-d] + W1 x_l[t] + bf)          (ops.py:23-46, F1-F3)
@@ -13,248 +13,10 @@
 #include "common.cuh"
 #include "mol.cuh"
 #include "train_tc.cuh"
-#include <type_traits>
 
 namespace train {
 
-constexpr int kTT = 64;             // time steps per tile
-constexpr int kAP = kR + 4;         // padded pitch
-constexpr int kThreads = 256;
-
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.0f / (1.0f + expf(-x)); }
-// Programmatic dependent launch: the layer kernels are launched so that a kernel's CTAs may start (and stage their weights) while
-// the previous layer's kernel drains; everything the previous launch wrote is visible after this wait (no-op in a plain launch).
-// The trigger right after it lets the NEXT launch's CTAs take the SM slots this grid frees as its CTAs exit (all of this grid's
-// CTAs are resident from the start, so nothing of it can be starved).
-__device__ __forceinline__ void grid_dependency_wait() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
-
-// ---- warp-level TF32 tensor-core helpers (mma.sync.m16n8k8, fp32 accumulate) ------------------------------
-// Used by the teacher's fp32-grade layer kernel below (operands pre-split into hi + lo TF32 parts, three MMAs per product).
-// Fragment layouts (g = lane >> 2, q = lane & 3):  A 16x8 row-major: a0 (g, q) a1 (g+8, q) a2 (g, q+4) a3 (g+8, q+4);
-// B 8x8: b0 (k = q, n = g) b1 (k = q+4, n = g);  C 16x8: c0 (g, 2q) c1 (g, 2q+1) c2 (g+8, 2q) c3 (g+8, 2q+1).
-__device__ __forceinline__ void mma_tf32(float (&d)[4], float a0, float a1, float a2, float a3, float b0, float b1) {
-  asm volatile("mma.sync.aligned.m16n8k8.row.col.f32.tf32.tf32.f32 {%0,%1,%2,%3}, {%4,%5,%6,%7}, {%8,%9}, {%0,%1,%2,%3};"
-               : "+f"(d[0]), "+f"(d[1]), "+f"(d[2]), "+f"(d[3])
-               : "r"(__float_as_uint(a0)), "r"(__float_as_uint(a1)), "r"(__float_as_uint(a2)), "r"(__float_as_uint(a3)),
-                 "r"(__float_as_uint(b0)), "r"(__float_as_uint(b1)));
-}
-constexpr int kWP = kR + 8;         // pitch of B operands read as (k = q, n = g): banks 8q + g
-// A fragment (16 rows x 8 tf32) with one ldmatrix: a 8x8 b16 matrix is 8 rows of 16 bytes = 8 rows x 4 tf32 words, and thread
-// (g, q) receives row g, word q -- the m16n8k8 A layout.  Lane l passes the row address of matrix l >> 3:
-// {rows 0-7 | rows 8-15} x {words 0-3 | words 4-7} -> a0, a1, a2, a3.  Rows are 144 bytes apart: conflict-free.
-__device__ __forceinline__ void ldsm_a(float (&a)[4], const float* lane_row_ptr) {
-  uint32_t r0, r1, r2, r3;
-  const uint32_t addr = (uint32_t)__cvta_generic_to_shared(lane_row_ptr);
-  asm volatile("ldmatrix.sync.aligned.m8n8.x4.shared.b16 {%0, %1, %2, %3}, [%4];" : "=r"(r0), "=r"(r1), "=r"(r2), "=r"(r3) : "r"(addr));
-  a[0] = __uint_as_float(r0); a[1] = __uint_as_float(r1); a[2] = __uint_as_float(r2); a[3] = __uint_as_float(r3);
-}
-
-// ---- forward layer of the training pass ---------------------------------------------------------------
-// x_{l+1} = (x_l + c Wr + br) sqrt(1/2) + cond_{l+1},  c = f sigmoid(f),  f = tanh([x_l[t-d] | x_l[t]] Wf + bf)   (ops.py:23-46)
-// Same tiling as the backward kernels (64 time steps, persistent CTAs, weights staged once).  The GEMMs run on the
-// tensor cores at fp32 grade: every operand is split into two TF32 numbers (x = hi + lo, |lo| <= 2^-11 |hi|) and a
-// product is three MMAs, lo*hi + hi*lo + hi*hi, small terms first (the dropped lo*lo term is 2^-22 relative).  The
-// stored activations are what the backward pass differentiates, so they stay within the fp32 path's 1e-4 of the oracle.
-constexpr int kSP = kS + 8;         // pitch of the skip weights: banks 8q + g
-struct FwdSmem {
-  float tap_h[kTT][kAP], tap_l[kTT][kAP], cur_h[kTT][kAP], cur_l[kTT][kAP], c_h[kTT][kAP], c_l[kTT][kAP];
-  float wf_h[2 * kR][kWP], wf_l[2 * kR][kWP], wr_h[kR][kWP], wr_l[kR][kWP], bf[kR], br[kR];
-};
-// teacher layers (skip 1x1, ops.py:44): the skip weights join the resident set and the gate output c takes over the
-// tap rows, which are dead once the filter conv has run, so that two CTAs still fit one SM
-struct FwdSmemSkip {
-  float tap_h[kTT][kAP], tap_l[kTT][kAP], cur_h[kTT][kAP], cur_l[kTT][kAP];
-  float wf_h[2 * kR][kWP], wf_l[2 * kR][kWP], wr_h[kR][kWP], wr_l[kR][kWP], bf[kR], br[kR];
-  float ws_h[kR][kSP], ws_l[kR][kSP], bs[kS];
-};
-// x = hi + lo with both parts valid TF32 numbers (low 13 mantissa bits clear).  Truncation instead of cvt.rna: hi is off by
-// up to 2^-10 |x| but x - hi is exact, and truncating lo costs 2^-10 |lo| <= 2^-20 |x|; two LOP3 + one FADD, where
-// cvt.rna.tf32.f32 expands to ~5 instructions each on sm_100a (FSETP / VIADD / SEL / LOP3: half of k_bwd_gate's ALU work).
-__device__ __forceinline__ void split_tf32(float x, float& hi, float& lo) {
-  hi = __uint_as_float(__float_as_uint(x) & 0xFFFFE000u);
-  lo = __uint_as_float(__float_as_uint(x - hi) & 0xFFFFE000u);
-}
-__device__ __forceinline__ void split_store4(float* h, float* l, float4 v) {
-  float4 vh, vl;
-  split_tf32(v.x, vh.x, vl.x); split_tf32(v.y, vh.y, vl.y); split_tf32(v.z, vh.z, vl.z); split_tf32(v.w, vh.w, vl.w);
-  *reinterpret_cast<float4*>(h) = vh;
-  *reinterpret_cast<float4*>(l) = vl;
-}
-
-template <bool SKIP>
-__global__ void __launch_bounds__(kThreads)
-k_fwd_layer(const float* __restrict__ x_l, float* __restrict__ x_next, const float* __restrict__ filt_k,
-            const float* __restrict__ filt_b, const float* __restrict__ res_k, const float* __restrict__ res_b,
-            const float* __restrict__ cond_next,     // cond + (l + 1) * R of layout [B][frames][L][R], or null after the last layer
-            int B, int T, int d, int P, int L, int frames,
-            const float* __restrict__ skip_k, const float* __restrict__ skip_b, float* __restrict__ skip, int skip_init) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  typedef typename std::conditional<SKIP, FwdSmemSkip, FwdSmem>::type Smem;
-  Smem& s = *reinterpret_cast<Smem*>(smem_raw);
-  float (*c_h)[kAP];
-  float (*c_l)[kAP];
-  if constexpr (SKIP) { c_h = s.tap_h; c_l = s.tap_l; } else { c_h = s.c_h; c_l = s.c_l; }
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, g = lane >> 2, q = lane & 3;
-  if constexpr (SKIP) {
-    for (int i = tid; i < kR * kS; i += kThreads) split_tf32(skip_k[i], s.ws_h[i / kS][i % kS], s.ws_l[i / kS][i % kS]);
-    if (tid < kS) s.bs[tid] = skip_b[tid];
-  }
-  for (int i = tid; i < 2 * kR * kR; i += kThreads) split_tf32(filt_k[i], s.wf_h[i / kR][i % kR], s.wf_l[i / kR][i % kR]);
-  for (int i = tid; i < kR * kR; i += kThreads) split_tf32(res_k[i], s.wr_h[i / kR][i % kR], s.wr_l[i / kR][i % kR]);
-  if (tid < kR) { s.bf[tid] = filt_b[tid]; s.br[tid] = res_b[tid]; }
-  const int tiles_per_b = (T + kTT - 1) / kTT;
-  const int n_tiles = B * tiles_per_b;
-  const int mt = warp & 3, nh = warp >> 2, r0 = mt * 16;
-  const int lrow = r0 + (lane & 7) + ((lane >> 3) & 1) * 8, lcol = (lane >> 4) * 4;      // this lane's row address inside an ldmatrix A tile
-  grid_dependency_wait();                            // weights are staged; the activations come from the previous launch
-  for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
-    const int b = tile / tiles_per_b, t0 = (tile % tiles_per_b) * kTT;
-    const float* xb = x_l + (size_t)b * T * kR;
-    __syncthreads();
-    for (int i = tid; i < kTT * (kR / 4); i += kThreads) {
-      const int row = i / (kR / 4), c4 = i % (kR / 4);
-      const int t = t0 + row;
-      float4 cur = make_float4(0, 0, 0, 0), tap = cur;
-      if (t < T) {
-        cur = *reinterpret_cast<const float4*>(xb + (size_t)t * kR + c4 * 4);
-        if (t - d >= 0) tap = *reinterpret_cast<const float4*>(xb + (size_t)(t - d) * kR + c4 * 4);
-      }
-      split_store4(&s.cur_h[row][c4 * 4], &s.cur_l[row][c4 * 4], cur);
-      split_store4(&s.tap_h[row][c4 * 4], &s.tap_l[row][c4 * 4], tap);
-    }
-    __syncthreads();
-    // filter conv (ops.py:6-20): W[0] pairs with x[t-d], W[1] with x[t]
-    float acc[2][4];
-#pragma unroll
-    for (int nt = 0; nt < 2; nt++) {
-      const int n0 = nh * 16 + nt * 8 + 2 * q;
-      acc[nt][0] = acc[nt][2] = s.bf[n0]; acc[nt][1] = acc[nt][3] = s.bf[n0 + 1];
-    }
-#pragma unroll
-    for (int ks = 0; ks < 8; ks++) {
-      const float (*XH)[kAP] = ks < 4 ? s.tap_h : s.cur_h;
-      const float (*XL)[kAP] = ks < 4 ? s.tap_l : s.cur_l;
-      const int kc = (ks & 3) * 8;
-      float ah[4], al[4];
-      ldsm_a(ah, &XH[lrow][kc + lcol]);
-      ldsm_a(al, &XL[lrow][kc + lcol]);
-#pragma unroll
-      for (int nt = 0; nt < 2; nt++) {
-        const int n0 = nh * 16 + nt * 8 + g;
-        const float bh0 = s.wf_h[ks * 8 + q][n0], bh1 = s.wf_h[ks * 8 + q + 4][n0];
-        const float bl0 = s.wf_l[ks * 8 + q][n0], bl1 = s.wf_l[ks * 8 + q + 4][n0];
-        mma_tf32(acc[nt], al[0], al[1], al[2], al[3], bh0, bh1);
-        mma_tf32(acc[nt], ah[0], ah[1], ah[2], ah[3], bl0, bl1);
-        mma_tf32(acc[nt], ah[0], ah[1], ah[2], ah[3], bh0, bh1);
-      }
-    }
-    if constexpr (SKIP) __syncthreads();               // every warp is done with the tap rows: c may take their place
-    // gate: tanh, sigmoid OF THE TANH, product (ops.py:28,33,36)
-#pragma unroll
-    for (int nt = 0; nt < 2; nt++) {
-      const int n0 = nh * 16 + nt * 8 + 2 * q;
-      float cv[4], ch[4], cl[4];
-#pragma unroll
-      for (int e = 0; e < 4; e++) { const float f = tanhf(acc[nt][e]); cv[e] = f * sigmoidf_(f); split_tf32(cv[e], ch[e], cl[e]); }
-      *reinterpret_cast<float2*>(&c_h[r0 + g][n0]) = make_float2(ch[0], ch[1]);
-      *reinterpret_cast<float2*>(&c_h[r0 + g + 8][n0]) = make_float2(ch[2], ch[3]);
-      *reinterpret_cast<float2*>(&c_l[r0 + g][n0]) = make_float2(cl[0], cl[1]);
-      *reinterpret_cast<float2*>(&c_l[r0 + g + 8][n0]) = make_float2(cl[2], cl[3]);
-    }
-    __syncthreads();
-    // residual 1x1 (ops.py:39), dense = (inputs + residual) * sqrt(1/2) (ops.py:40), next layer's conditioning (model.py:183)
-#pragma unroll
-    for (int nt = 0; nt < 2; nt++) {
-      const int n0 = nh * 16 + nt * 8 + 2 * q;
-      acc[nt][0] = acc[nt][2] = s.br[n0]; acc[nt][1] = acc[nt][3] = s.br[n0 + 1];
-    }
-#pragma unroll
-    for (int ks = 0; ks < 4; ks++) {
-      const int kc = ks * 8;
-      float ah[4], al[4];
-      ldsm_a(ah, &c_h[lrow][kc + lcol]);
-      ldsm_a(al, &c_l[lrow][kc + lcol]);
-      const float h0 = ah[0], h1 = ah[1], h2 = ah[2], h3 = ah[3], l0 = al[0], l1 = al[1], l2 = al[2], l3 = al[3];
-#pragma unroll
-      for (int nt = 0; nt < 2; nt++) {
-        const int n0 = nh * 16 + nt * 8 + g;
-        const float bh0 = s.wr_h[kc + q][n0], bh1 = s.wr_h[kc + q + 4][n0];
-        const float bl0 = s.wr_l[kc + q][n0], bl1 = s.wr_l[kc + q + 4][n0];
-        mma_tf32(acc[nt], l0, l1, l2, l3, bh0, bh1);
-        mma_tf32(acc[nt], h0, h1, h2, h3, bl0, bl1);
-        mma_tf32(acc[nt], h0, h1, h2, h3, bh0, bh1);
-      }
-    }
-    const int ta = t0 + r0 + g, tb = ta + 8;
-#pragma unroll
-    for (int nt = 0; nt < 2; nt++) {
-      const int n0 = nh * 16 + nt * 8 + 2 * q;
-      if (ta < T) {
-        const size_t at = ((size_t)b * T + ta) * kR + n0;
-        const float2 xv = *reinterpret_cast<const float2*>(x_l + at);
-        float2 v = make_float2((xv.x + acc[nt][0]) * SRWN_SQRT_HALF, (xv.y + acc[nt][1]) * SRWN_SQRT_HALF);
-        if (cond_next) { const float2 cn = *reinterpret_cast<const float2*>(cond_next + ((size_t)b * frames + ta / P) * L * kR + n0); v.x += cn.x; v.y += cn.y; }
-        *reinterpret_cast<float2*>(x_next + at) = v;
-      }
-      if (tb < T) {
-        const size_t at = ((size_t)b * T + tb) * kR + n0;
-        const float2 xv = *reinterpret_cast<const float2*>(x_l + at);
-        float2 v = make_float2((xv.x + acc[nt][2]) * SRWN_SQRT_HALF, (xv.y + acc[nt][3]) * SRWN_SQRT_HALF);
-        if (cond_next) { const float2 cn = *reinterpret_cast<const float2*>(cond_next + ((size_t)b * frames + tb / P) * L * kR + n0); v.x += cn.x; v.y += cn.y; }
-        *reinterpret_cast<float2*>(x_next + at) = v;
-      }
-    }
-    if constexpr (SKIP) {
-      // skip 1x1 (ops.py:44) accumulated over layers in global memory (model.py:190); warp (mt, nh): rows 16 mt.., channels 64 nh..
-      float sk[8][4];
-#pragma unroll
-      for (int nt = 0; nt < 8; nt++) {
-        const int n0 = nh * 64 + nt * 8 + 2 * q;
-        sk[nt][0] = sk[nt][2] = s.bs[n0]; sk[nt][1] = sk[nt][3] = s.bs[n0 + 1];
-      }
-#pragma unroll
-      for (int ks = 0; ks < 4; ks++) {
-        const int kc = ks * 8;
-      float ah[4], al[4];
-      ldsm_a(ah, &c_h[lrow][kc + lcol]);
-      ldsm_a(al, &c_l[lrow][kc + lcol]);
-      const float h0 = ah[0], h1 = ah[1], h2 = ah[2], h3 = ah[3], l0 = al[0], l1 = al[1], l2 = al[2], l3 = al[3];
-#pragma unroll
-        for (int nt = 0; nt < 8; nt++) {
-          const int n0 = nh * 64 + nt * 8 + g;
-          const float bh0 = s.ws_h[kc + q][n0], bh1 = s.ws_h[kc + q + 4][n0];
-          const float bl0 = s.ws_l[kc + q][n0], bl1 = s.ws_l[kc + q + 4][n0];
-          mma_tf32(sk[nt], l0, l1, l2, l3, bh0, bh1);
-          mma_tf32(sk[nt], h0, h1, h2, h3, bl0, bl1);
-          mma_tf32(sk[nt], h0, h1, h2, h3, bh0, bh1);
-        }
-      }
-#pragma unroll
-      for (int nt = 0; nt < 8; nt++) {
-        const int n0 = nh * 64 + nt * 8 + 2 * q;
-        if (ta < T) {
-          float2* dst = reinterpret_cast<float2*>(skip + ((size_t)b * T + ta) * kS + n0);
-          float2 v = make_float2(sk[nt][0], sk[nt][1]);
-          if (!skip_init) { const float2 pv = *dst; v.x += pv.x; v.y += pv.y; }
-          *dst = v;
-        }
-        if (tb < T) {
-          float2* dst = reinterpret_cast<float2*>(skip + ((size_t)b * T + tb) * kS + n0);
-          float2 v = make_float2(sk[nt][2], sk[nt][3]);
-          if (!skip_init) { const float2 pv = *dst; v.x += pv.x; v.y += pv.y; }
-          *dst = v;
-        }
-      }
-    }
-  }
-}
-
-// The per-layer kernels of the student's training pass (forward keeping activations, gate backward, conv backward) live in
-// train_tc.cu (tcgen05 kind::tf32); k_fwd_layer<true> above remains for the teacher's fp32-grade path, whose layers also
-// produce the skip output.
 
 // sums `rows` partial rows (row pitch `pitch`) of width w1 + w2 into dst1 [w1] and dst2 [w2] (+=) in a fixed order:
 // 32 columns per CTA, the rows split over the 8 warps (independent loads in flight), then a fixed-order sum of the 8 parts
@@ -548,9 +310,6 @@ static TrainWs carve_train(const srwn_ctx* c, int B, int T, void* ws, size_t cap
   const size_t n = (size_t)B * T, L = c->cfg.n_layers, F = c->cfg.num_flows, frames = T / c->cfg.pool_stride;
   r.grid = 3 * (c->sm_count > 0 ? c->sm_count : 148);     // elementwise kernels of the step (heads, front)
   r.grid_tc = c->sm_count > 0 ? c->sm_count : 148;         // tensor-core layer kernels: one persistent CTA per SM (shared memory)
-#ifdef SRWN_TC_GRID
-  r.grid_tc = SRWN_TC_GRID;                                // tuning builds: few CTAs, so that small test shapes give every CTA several tiles
-#endif
   r.acts = w.take<float>(F * (L + 1) * n * kR);
   r.cond = w.take<float>((size_t)B * frames * L * kR);
   r.scales = w.take<float>(F * n);
@@ -573,65 +332,7 @@ static TrainWs carve_train(const srwn_ctx* c, int B, int T, void* ws, size_t cap
 
 size_t train_workspace_bytes(const srwn_ctx* c, int B, int T) { return carve_train(c, B, T, nullptr, 0).bytes; }
 
-// forward of all flows in fp32, keeping every layer input (model.py:489-535)
-template <typename... KArgs, typename... Args>
-static cudaError_t launch_dependent(void (*kern)(KArgs...), int grid, int block, size_t smem, cudaStream_t st, Args... args) {
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid); cfg.blockDim = dim3(block); cfg.dynamicSmemBytes = smem; cfg.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  cfg.attrs = attr; cfg.numAttrs = 1;
-#ifdef SRWN_NO_PDL
-  cfg.numAttrs = 0;                        // tuning builds: plain stream order
-#endif
-  return cudaLaunchKernelEx(&cfg, kern, KArgs(args)...);
-}
-
-// one layer of the fp32-grade path (stack_f32.cu): x_l -> x_next, teacher layers also accumulate their skip output
-int run_layer_tf32x3(srwn_ctx* c, bool with_skip, const float* x_l, float* x_next, float* skip, const float* filt_k,
-                     const float* filt_b, const float* res_k, const float* res_b, const float* skip_k, const float* skip_b,
-                     const float* cond_next, int B, int T, int d, int P, int L, int frames, int skip_init, cudaStream_t st) {
-  const int grid = 2 * (c->sm_count > 0 ? c->sm_count : 148);
-  if (with_skip) {
-    SRWN_CUDA(cudaFuncSetAttribute(train::k_fwd_layer<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(train::FwdSmemSkip)));
-    SRWN_CUDA(launch_dependent(train::k_fwd_layer<true>, grid, train::kThreads, sizeof(train::FwdSmemSkip), st,
-        x_l, x_next, filt_k, filt_b, res_k, res_b, cond_next, B, T, d, P, L, frames, skip_k, skip_b, skip, skip_init));
-  } else {
-    SRWN_CUDA(cudaFuncSetAttribute(traintc::k_fwd_layer_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, traintc::fwd_smem_bytes()));
-    SRWN_CUDA(launch_dependent(traintc::k_fwd_layer_tc, grid / 2, traintc::kThreads, (size_t)traintc::fwd_smem_bytes(), st,
-        x_l, x_next, filt_k, filt_b, res_k, res_b, cond_next, B, T, d, P, L, frames));
-  }
-  SRWN_LAUNCH_CHECK();
-  return SRWN_OK;
-}
-
-// forward of one flow keeping every layer input: acts [L+1][B][T][R], acts[l] = block input of layer l, acts[L] = stack output
-static int run_stack_train_acts(srwn_ctx* c, int stack, const float* xin, const float* enc, int B, int T, float* acts,
-                                float* cond, int grid, cudaStream_t st) {
-  const float* w = stack_w(c, stack);
-  const StackOffsets& o = c->off;
-  const int L = c->cfg.n_layers, P = c->cfg.pool_stride, C = c->cfg.cond_channels, frames = T / P;
-  const size_t n = (size_t)B * T;
-  k_cond<<<B * frames, 256, 0, st>>>(enc, w + o.cond_k, w + o.cond_b, cond, B * frames, L, C);
-  SRWN_LAUNCH_CHECK();
-  {
-    dim3 g((unsigned)(((int64_t)T * kR + 255) / 256), B);
-    k_front<<<g, 256, 0, st>>>(xin, w + o.front_k, w + o.front_b, cond, acts, T, P, L, frames);
-    SRWN_LAUNCH_CHECK();
-  }
-  SRWN_CUDA(cudaFuncSetAttribute(traintc::k_fwd_layer_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, traintc::fwd_smem_bytes()));
-  for (int l = 0; l < L; l++) {
-    const float* cond_next = l + 1 < L ? cond + (size_t)(l + 1) * kR : nullptr;
-    SRWN_CUDA(launch_dependent(traintc::k_fwd_layer_tc, grid, traintc::kThreads, (size_t)traintc::fwd_smem_bytes(), st,
-        acts + (size_t)l * n * kR, acts + (size_t)(l + 1) * n * kR, w + o.filt_k + (size_t)l * 2 * kR * kR,
-        w + o.filt_b + (size_t)l * kR, w + o.res_k + (size_t)l * kR * kR, w + o.res_b + (size_t)l * kR, cond_next,
-        B, T, c->dilations[l], P, L, frames));
-    SRWN_LAUNCH_CHECK();
-  }
-  return SRWN_OK;
-}
-
+// forward of all flows in fp32, keeping every layer input (model.py:489-535): acts of flow f is [L+1][B][T][R]
 int run_student_forward_train(srwn_ctx* c, const float* z, const float* enc, float* out, float* s_tot,
                               float* mu_tot, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
   TrainWs w = carve_train(c, B, T, ws, ws_bytes);
@@ -640,11 +341,10 @@ int run_student_forward_train(srwn_ctx* c, const float* z, const float* enc, flo
   const int F = c->cfg.num_flows, L = c->cfg.n_layers;
   const float* xin = z;
   for (int f = 0; f < F; f++) {
-    float* acts = w.acts + (size_t)f * (L + 1) * n * kR;
-    int rc = run_stack_train_acts(c, f, xin, enc, B, T, acts, w.cond, w.grid_tc, st);
+    float* hL = nullptr;
+    int rc = run_stack_f32(c, f, xin, enc, B, T, w.acts + (size_t)f * (L + 1) * n * kR, nullptr, nullptr, w.cond, &hL, st);
     if (rc) return rc;
-    rc = run_flow_head_f32(c, f, acts + (size_t)L * n * kR, xin, w.scales + (size_t)f * n, w.means + (size_t)f * n,
-                           w.xs + (size_t)f * n, B, T, st);
+    rc = run_flow_head_f32(c, f, hL, xin, w.scales + (size_t)f * n, w.means + (size_t)f * n, w.xs + (size_t)f * n, B, T, st);
     if (rc) return rc;
     xin = w.xs + (size_t)f * n;
   }
@@ -662,12 +362,8 @@ int run_student_backward(srwn_ctx* c, const float* z, const float* enc, const fl
   const int F = c->cfg.num_flows, L = c->cfg.n_layers, P = c->cfg.pool_stride, frames = T / P, C = c->cfg.cond_channels;
   const int BF = B * frames;
   const StackOffsets& o = c->off;
-  static bool attr_done = false;
-  if (!attr_done) {
-    SRWN_CUDA(cudaFuncSetAttribute(traintc::k_bwd_gate_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, traintc::gate_smem_bytes()));
-    SRWN_CUDA(cudaFuncSetAttribute(traintc::k_bwd_conv_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, traintc::conv_smem_bytes()));
-    attr_done = true;
-  }
+  SRWN_CUDA(cudaFuncSetAttribute(traintc::k_bwd_gate_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, traintc::gate_smem_bytes()));
+  SRWN_CUDA(cudaFuncSetAttribute(traintc::k_bwd_conv_tc, cudaFuncAttributeMaxDynamicSharedMemorySize, traintc::conv_smem_bytes()));
   SRWN_CUDA(cudaMemsetAsync(grads, 0, (size_t)c->n_stacks * c->stack_floats * sizeof(float), st));
   k_bwd_compose<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(z, w.scales, w.means, d_pre, d_s_extra, F, w.d_scales, w.d_means, (int64_t)n);
   SRWN_LAUNCH_CHECK();

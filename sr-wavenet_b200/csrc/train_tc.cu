@@ -119,10 +119,6 @@ __device__ __forceinline__ float sigmoid_fast(float f) {
 __device__ __forceinline__ float4 ldg4(const float* p) { return *reinterpret_cast<const float4*>(p); }
 __device__ __forceinline__ float& f4at(float4& v, int e) { return reinterpret_cast<float*>(&v)[e]; }
 
-__device__ __forceinline__ void grid_dependency_wait() {
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-}
 // a pipeline wait that never completes is a bug in this file, not a data condition: stop the kernel instead of hanging the GPU
 __device__ __forceinline__ void wait_or_trap(uint32_t bar, uint32_t parity, volatile int* abort_words) {
   if (!mbar_wait(bar, parity, abort_words, 1, 4000000000LL)) __trap();

@@ -1,4 +1,5 @@
-// Layer kernels of the student training pass on tcgen05 (kind::tf32, 3xTF32 split): declarations for train_f32.cu.
+// Student layer kernels on tcgen05 (kind::tf32, 3xTF32 split): the forward for the fp32-grade stack (stack_f32.cu),
+// the two backward kernels for the distillation step (train_f32.cu).
 #pragma once
 #include "common.cuh"
 
