@@ -187,6 +187,20 @@ int srwn_teacher_generate_resume(srwn_handle_t h, void* state, const float* enc,
  *   handle, fp16 where the tensor-core generation kernel does not cover the configuration, a small workspace. */
 int srwn_generate_state_prefill(srwn_handle_t h, void* state, const float* x, const float* enc, int32_t n, int32_t B,
                                 int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
+/* srwn_generate_state_splice: for each i < n, utterance src_rows[i] of `src` (src_B utterances) replaces utterance
+ *   dst_rows[i] of `dst` (dst_B utterances); both states were reset on h for their B and this precision.  The row arrays
+ *   are HOST memory.  A state's position t0 is always a multiple of pool_stride (reset sets 0, resume and prefill advance
+ *   by multiples of it), so two states agree on latent-frame boundaries; the splice copies each layer's d queue entries,
+ *   rotated from src's phase t0 mod d to dst's (both t0 read on the device: no synchronisation), and the x history.
+ *   dst's t0, its other utterances and all of src stay unchanged.  Generating on dst then continues each spliced
+ *   utterance bit for bit as generating on src would (with the same frames and uniforms): continuous batching refills
+ *   the slot of a finished utterance with a freshly primed one.  No workspace; n == 0 does nothing.  Refused with
+ *   SRWN_ERR_INVALID before any work: a null state, a state not reset on this handle for its B and precision,
+ *   src == dst, n < 0, a row out of range, a destination row named twice, a student handle; SRWN_ERR_UNSUPPORTED as
+ *   srwn_generate_state_bytes for the precision. */
+int srwn_generate_state_splice(srwn_handle_t h, void* dst, int32_t dst_B, const int32_t* dst_rows,
+                               const void* src, int32_t src_B, const int32_t* src_rows, int32_t n,
+                               int32_t precision, void* stream);
 
 /* ---- student (model.py:415-535) ------------------------------------------------- */
 /* generate(sess, inputs, encoding) (model.py:570-576): z [B,T] logistic noise ->

@@ -68,6 +68,8 @@ SIGNATURES = {
     "srwn_teacher_generate_resume": (ctypes.c_int, [_vp, _vp, _fp, _fp, _fp, _fp, _i32, _fp, _fp, _i32, _i32, _i32,
                                                     _vp, _sz, _vp]),
     "srwn_generate_state_prefill": (ctypes.c_int, [_vp, _vp, _fp, _fp, _i32, _i32, _i32, _vp, _sz, _vp]),
+    "srwn_generate_state_splice": (ctypes.c_int, [_vp, _vp, _i32, ctypes.POINTER(_i32), _vp, _i32, ctypes.POINTER(_i32),
+                                                  _i32, _i32, _vp]),
     "srwn_student_forward": (ctypes.c_int, [_vp, _fp, _fp, _fp, _fp, _fp, _fp, _i32, _i32, _i32, _vp, _sz, _vp]),
     "srwn_student_sample": (ctypes.c_int, [_vp, ctypes.c_uint64, ctypes.c_uint64, _fp, _fp, _fp, _fp, _fp, _fp, _i32, _i32, _i32, _vp, _sz, _vp]),
     "srwn_random_logistic": (ctypes.c_int, [_fp, _i64, ctypes.c_uint64, ctypes.c_uint64, _vp]),

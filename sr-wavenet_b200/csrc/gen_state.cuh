@@ -8,6 +8,10 @@
 //     lane quad q own the 16 bytes at (4u + q) * 16: the fp16 pairs of channels 8j + 2q, 8j + 2q + 1 for n-tiles j in
 //     the order {0, 2, 1, 3}, which is the A-fragment quad of the filter conv's k-tile 0 (ar_mma.cuh: mma8q).
 // Layer l's input at position t lives in slot t mod d_l of its d_l slots.
+//
+// The position t0 of a state is always a multiple of pool_stride P: reset sets 0, a resume call needs T % P == 0 and a
+// prefill n % P == 0.  Two states therefore agree on latent-frame boundaries and differ only in each layer's queue phase
+// t0 mod d_l; srwn_generate_state_splice relies on this when it moves an utterance from one state into another.
 #pragma once
 #include "common.cuh"
 

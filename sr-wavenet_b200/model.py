@@ -648,6 +648,156 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         _lib.check(eng.lib.srwn_generate_state_prefill(eng.h, state.data_ptr(), x.data_ptr(), e.data_ptr(), n, B, prec,
                                                        ws, wsn, _stream()))
 
+    def generate_requests(self, requests, slots, chunk, precision="fp16"):
+        """Continuous batching: generate many utterances of different lengths through one state of ``slots`` utterances,
+        refilling the slot of each finished utterance with the next request.  A generator of ``(index, audio)``, yielded
+        as each request finishes.
+
+        A request is a dict (or just its encoding): ``encoding`` [F, latent_channels] its frames; ``conditions``
+        [condition_size] when the model has them; optionally ``prime`` [n0] real samples that start the utterance (n0 a
+        multiple of pool_stride, the frames cover the prime and the continuation) and ``u1`` [F*P - n0, M], ``u2``
+        [F*P - n0] the sampler's uniforms for its generated samples (otherwise drawn on the device).  Its audio is the
+        F*P - n0 samples after the prime, a CUDA tensor when ``encoding`` is one, else a NumPy array.
+
+        Before each ``generate`` call of ``chunk`` samples (a multiple of pool_stride) free slots are filled in arrival
+        order: primed requests through ``prefill`` of a side state (one per prime length), the others from a reset
+        state, both moved in with ``GenerationState.splice``.  Each call takes every slot's frames and uniforms at that
+        slot's own offset (idle slots get zeros); what a request generates past its end is dropped.  With injected
+        uniforms a request's audio is bit for bit that of generating it alone (B = 1, the same prime through prefill)."""
+        eng, P, M, cs = self._eng, self.pool_stride, self.num_mixtures, self.condition_size
+        slots, chunk = int(slots), int(chunk)
+        if slots < 1 or chunk < P or chunk % P:
+            raise ValueError("slots must be positive and chunk a positive multiple of pool_stride=%d" % P)
+
+        def dev(a):
+            t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
+            return t.float().cuda().contiguous()
+
+        reqs = []
+        for i, r in enumerate(requests):
+            r = r if isinstance(r, dict) else {"encoding": r}
+            e = dev(r["encoding"])
+            if e.ndim != 2 or e.shape[1] != self.latent_channels:
+                raise ValueError("request %d: encoding must be [F, %d]" % (i, self.latent_channels))
+            prime = dev(r["prime"]).reshape(-1) if r.get("prime") is not None else None
+            n0 = 0 if prime is None else int(prime.shape[0])
+            need = e.shape[0] * P - n0
+            if n0 % P or need < 0:
+                raise ValueError("request %d: the prime (%d samples) must be a multiple of %d within the %d frames"
+                                 % (i, n0, P, e.shape[0]))
+            c = None
+            if cs:
+                if r.get("conditions") is None:
+                    raise ValueError("request %d: condition_size > 0 needs `conditions`" % i)
+                c = dev(r["conditions"]).reshape(-1)
+                if c.shape[0] != cs:
+                    raise ValueError("request %d: conditions must be [%d]" % (i, cs))
+            inj = r.get("u1") is not None or r.get("u2") is not None
+            if inj:
+                if r.get("u1") is None or r.get("u2") is None:
+                    raise ValueError("request %d: inject both u1 and u2, or neither" % i)
+                u1, u2 = dev(r["u1"]), dev(r["u2"]).reshape(-1)
+                if tuple(u1.shape) != (need, M) or u2.shape[0] != need:
+                    raise ValueError("request %d: u1 must be [%d, %d] and u2 [%d]" % (i, need, M, need))
+            reqs.append({"enc": e, "prime": prime, "n0": n0, "need": need, "cond": c,
+                         "u1": u1 if inj else None, "u2": u2 if inj else None,
+                         "on_dev": isinstance(r["encoding"], torch.Tensor) and r["encoding"].is_cuda})
+        N = len(reqs)
+        if N == 0:
+            return
+
+        # every request's generation frames, uniforms and output in flat device buffers, each with one sentinel row
+        # (zeros to read, a sink to write) that idle slots and samples past a request's end point at
+        def flat(parts, tail_shape):
+            return torch.cat([p for p in parts if p is not None and p.shape[0]] +
+                             [torch.zeros((1,) + tail_shape, device="cuda")])
+        fbase, ubase, obase = np.zeros(N, np.int64), np.full(N, -1, np.int64), np.zeros(N, np.int64)
+        nf = nu = no = 0
+        for i, r in enumerate(reqs):
+            fbase[i], obase[i] = nf, no
+            nf += r["need"] // P
+            no += r["need"]
+            if r["u1"] is not None:
+                ubase[i] = nu
+                nu += r["need"]
+        enc_all = flat([r["enc"][r["n0"] // P:] for r in reqs], (self.latent_channels,))
+        cond_all = torch.stack([r["cond"] for r in reqs] + [torch.zeros(cs, device="cuda")]) if cs else None
+        u1_all = flat([r["u1"] for r in reqs], (M,))
+        u2_all = flat([r["u2"] for r in reqs], ())
+        out_all = torch.empty(no + 1, dtype=torch.float32, device="cuda")
+        need_np = np.array([r["need"] for r in reqs], np.int64)
+
+        main = self.generation_state(slots, precision)
+        silence = self.generation_state(1, precision)           # reset, never generated on: the source of fresh slots
+        slot_req = np.full(slots, -1, np.int64)                  # request in each slot, -1 idle
+        slot_pos = np.zeros(slots, np.int64)                     # samples it has generated
+        ar_f = torch.arange(chunk // P, device="cuda")
+        ar_s = torch.arange(chunk, device="cuda")
+        lo, hi = 1e-5, 1.0 - 1e-5                                # ops.py:187, 196
+        nxt = 0
+        while True:
+            # fill the free slots from the queue
+            fresh, primed = [], {}
+            while nxt < N and (slot_req < 0).any():
+                if reqs[nxt]["need"] == 0:
+                    yield nxt, self._request_audio(out_all[:0], reqs[nxt]["on_dev"])
+                    nxt += 1
+                    continue
+                s = int(np.flatnonzero(slot_req < 0)[0])
+                slot_req[s], slot_pos[s] = nxt, 0
+                if reqs[nxt]["n0"]:
+                    primed.setdefault(reqs[nxt]["n0"], []).append(s)
+                else:
+                    fresh.append(s)
+                nxt += 1
+            if fresh:
+                main.splice(fresh, silence, [0] * len(fresh))
+            for n0, rows in primed.items():
+                rs = [reqs[slot_req[s]] for s in rows]
+                side = self.generation_state(len(rows), precision)
+                self.prefill(side, torch.stack([r["prime"] for r in rs]),
+                             torch.stack([r["enc"][:n0 // P] for r in rs]),
+                             conditions=torch.stack([r["cond"] for r in rs]) if cs else None)
+                main.splice(rows, side)
+            active = slot_req >= 0
+            if not active.any():
+                return
+            # gather every slot's frames and uniforms at its own offset (sentinel rows for idle slots and past the end)
+            rq = np.where(active, slot_req, 0)
+            left = torch.from_numpy(np.where(active, need_np[rq] - slot_pos, 0)).cuda()
+            pos = torch.from_numpy(slot_pos).cuda()
+            fb = torch.from_numpy(fbase[rq] + slot_pos // P).cuda()
+            ub = torch.from_numpy(np.where(active, ubase[rq], -1) + slot_pos).cuda()
+            ob = torch.from_numpy(obase[rq] + slot_pos).cuda()
+            inj = torch.from_numpy(active & (ubase[rq] >= 0)).cuda()
+            fvalid = ar_f[None, :] * P < left[:, None]
+            svalid = ar_s[None, :] < left[:, None]
+            fidx = torch.where(fvalid, fb[:, None] + ar_f[None, :], enc_all.shape[0] - 1)
+            uidx = torch.where(svalid & inj[:, None], ub[:, None] + ar_s[None, :], u2_all.shape[0] - 1)
+            oidx = torch.where(svalid, ob[:, None] + ar_s[None, :], out_all.shape[0] - 1)
+            enc_c = enc_all[fidx]
+            u1_c, u2_c = u1_all[uidx], u2_all[uidx]
+            drawn = np.flatnonzero(active & (ubase[rq] < 0))
+            if drawn.size:                                         # uniforms of requests without injected ones
+                self._noise_calls = getattr(self, "_noise_calls", 0) + 1
+                d1 = eng.random_uniform((slots, chunk, M), self.seed, 2 * self._noise_calls, lo, hi)
+                d2 = eng.random_uniform((slots, chunk), self.seed, 2 * self._noise_calls + 1, lo, hi)
+                dr = torch.from_numpy(drawn).cuda()
+                u1_c[dr], u2_c[dr] = d1[dr], d2[dr]
+            cond_c = cond_all[torch.from_numpy(np.where(active, slot_req, N)).cuda()] if cs else None
+            x = self.generate(enc_c, conditions=cond_c, u1=u1_c, u2=u2_c, precision=precision, state=main)
+            out_all[oidx.reshape(-1)] = x.reshape(-1)
+            # hand out the requests that have finished and free their slots
+            slot_pos[active] += chunk
+            for s in np.flatnonzero(active & (slot_pos >= need_np[rq])):
+                i = int(slot_req[s])
+                slot_req[s] = -1
+                yield i, self._request_audio(out_all[obase[i]:obase[i] + need_np[i]], reqs[i]["on_dev"])
+
+    @staticmethod
+    def _request_audio(x, on_dev):
+        return x.clone() if on_dev else x.cpu().numpy()
+
     def _check(self, e, B, T):
         if e.ndim != 3 or e.shape[0] != B or e.shape[2] != self.latent_channels + self.condition_size:
             raise ValueError("encoding must be [B, T/pool_stride, %d]" % (self.latent_channels + self.condition_size))
@@ -677,6 +827,31 @@ class GenerationState(object):
     def position(self):
         """Samples generated through this state since the last reset (reads the device header: synchronises)."""
         return int(self.buffer[:8].view(torch.int64).item())
+
+    def splice(self, rows, src, src_rows=None):
+        """Utterance ``src_rows[i]`` of ``src`` (default: utterance i) replaces utterance ``rows[i]`` of this state
+        (include/srwn.h, srwn_generate_state_splice).  ``src`` is another state of the same model and precision, at any
+        position: each layer's queue is rotated to this state's phase, so generating here continues the utterance bit for
+        bit as generating on ``src`` would.  This state's position, its other utterances and ``src`` are unchanged."""
+        if not isinstance(src, GenerationState) or src._eng is not self._eng:
+            raise ValueError("src must be a state of this state's model")
+        if src is self or src.buffer.data_ptr() == self.buffer.data_ptr():
+            raise ValueError("src and this state are the same state")
+        if src.precision != self.precision:
+            raise ValueError("src has precision %r, this state %r" % (src.precision, self.precision))
+        rows = [int(r) for r in rows]
+        src_rows = list(range(len(rows))) if src_rows is None else [int(r) for r in src_rows]
+        if len(src_rows) != len(rows):
+            raise ValueError("%d destination rows but %d source rows" % (len(rows), len(src_rows)))
+        if any(r < 0 or r >= self.batch_size for r in rows) or any(r < 0 or r >= src.batch_size for r in src_rows):
+            raise ValueError("rows must be in [0, %d) and src_rows in [0, %d)" % (self.batch_size, src.batch_size))
+        if len(set(rows)) != len(rows):
+            raise ValueError("a destination row is named twice")
+        n = len(rows)
+        dst_a, src_a = (ctypes.c_int32 * max(n, 1))(*rows), (ctypes.c_int32 * max(n, 1))(*src_rows)
+        _lib.check(self._eng.lib.srwn_generate_state_splice(self._eng.h, self.data_ptr(), self.batch_size, dst_a,
+                                                           src.data_ptr(), src.batch_size, src_a, n, self._prec,
+                                                           _stream()))
 
     def data_ptr(self):
         return self.buffer.data_ptr()
