@@ -17,15 +17,11 @@ import numpy as np
 import torch
 
 from . import _lib
+from .model import _cuda_f32
 
 
 def _stream():
     return torch.cuda.current_stream().cuda_stream
-
-
-def _dev(a):
-    t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
-    return t.float().contiguous().cuda() if not (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous()) else t
 
 
 class _BlockStack(object):
@@ -93,7 +89,7 @@ class _BlockStack(object):
     def forward(self, inputs):
         """inputs [B, T] -> pooled [B, T - input_size + 1, outputs] (fp32 CUDA tensor)."""
         lib = _lib.load()
-        x = _dev(inputs)
+        x = _cuda_f32(inputs)
         if x.ndim != 2:
             raise ValueError("inputs must be [batch, time]")
         B, T = x.shape

@@ -15,7 +15,7 @@ import time
 import numpy as np
 import torch
 
-from . import _lib, synth
+from . import _lib, synth, tf_checkpoint
 
 
 def _as_i32_array(values):
@@ -23,50 +23,95 @@ def _as_i32_array(values):
     return arr
 
 
-class _Engine(object):
-    """Owns one libsrwn handle plus the caller-side workspace and pinned staging buffers."""
+def _f32(a):
+    """NumPy array or tensor -> contiguous fp32 tensor; host data stays on the host."""
+    t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
+    return t.float().contiguous()
 
-    def __init__(self, kind, dilations, filter_width, dilation_channels, skip_channels, cond_channels,
-                 pool_stride, num_mixtures=0, num_flows=0):
+
+def _cuda_f32(a):
+    """NumPy array or tensor -> contiguous fp32 CUDA tensor (a tensor that already is one is returned as it is)."""
+    return _f32(a).cuda()
+
+
+class _Workspace(object):
+    """Caller-side device workspace of a library call: grows to the largest size asked of it and is never shrunk."""
+
+    def __init__(self):
+        self._buf = None
+
+    def get(self, query, *args):
+        """(pointer, bytes) of at least the size ``query(*args, &n)`` reports."""
+        n = ctypes.c_size_t()
+        _lib.check(query(*args, ctypes.byref(n)))
+        if self._buf is None or self._buf.numel() < n.value:
+            self._buf = None             # release the old buffer before the larger one is allocated
+            self._buf = torch.empty(max(n.value, 256), dtype=torch.uint8, device="cuda")
+        return self._buf.data_ptr(), self._buf.numel()
+
+
+class _Handle(object):
+    """One libsrwn handle: its lifetime, weight upload and commit, workspace and profiling switch.  The decoder and the
+    encoder handle (include/srwn.h) differ only in the names of the entry points they pass in: create, destroy,
+    set_weight, commit and set_profiling."""
+
+    def __init__(self, what, cfg, entry_points):
         lib = _lib.load()
         if not torch.cuda.is_available():
-            raise RuntimeError("the SR-WaveNet hot path needs a CUDA device (no CPU fallback)")
-        self._dil = _as_i32_array(dilations)
-        cfg = _lib.Config(kind, len(dilations), self._dil, filter_width, dilation_channels, skip_channels,
-                          cond_channels, pool_stride, num_mixtures, num_flows)
+            raise RuntimeError("the SR-WaveNet %s needs a CUDA device (no CPU fallback)" % what)
+        create, self._destroy, self._set_weight, self._commit, self._set_profiling = (getattr(lib, n) for n in entry_points)
         h = ctypes.c_void_p()
-        _lib.check(lib.srwn_create(ctypes.byref(cfg), ctypes.byref(h)))
-        self.lib, self.h, self.kind = lib, h, kind
-        self.cond_channels = cond_channels
-        self.pool_stride = pool_stride
-        self._ws = None
-        self._pinned = {}
+        _lib.check(create(ctypes.byref(cfg), ctypes.byref(h)))
+        self.lib, self.h = lib, h
+        self._ws = _Workspace()
 
     def __del__(self):
         try:
             if getattr(self, "h", None):
-                self.lib.srwn_destroy(self.h)
+                self._destroy(self.h)
                 self.h = None
         except Exception:
             pass
 
-    def set_weights(self, weights, prefix_filter=None):
+    def set_weights(self, weights):
         for name, arr in weights.items():
-            if prefix_filter and not name.startswith(prefix_filter):
-                continue
             a = np.ascontiguousarray(arr, dtype=np.float32)
             shape = (ctypes.c_int64 * a.ndim)(*a.shape)
-            _lib.check(self.lib.srwn_set_weight(self.h, name.encode(), a.ctypes.data_as(ctypes.c_void_p),
-                                                shape, a.ndim))
-        _lib.check(self.lib.srwn_commit_weights(self.h, torch.cuda.current_stream().cuda_stream))
+            _lib.check(self._set_weight(self.h, name.encode(), a.ctypes.data_as(ctypes.c_void_p), shape, a.ndim))
+        _lib.check(self._commit(self.h, _stream()))
+
+    def set_profiling(self, enable):
+        _lib.check(self._set_profiling(self.h, int(bool(enable))))
+
+
+class _Engine(_Handle):
+    """Owns one libsrwn handle plus the caller-side workspace and pinned staging buffers."""
+
+    def __init__(self, kind, dilations, filter_width, dilation_channels, skip_channels, cond_channels,
+                 pool_stride, num_mixtures=0, num_flows=0):
+        self._dil = _as_i32_array(dilations)
+        cfg = _lib.Config(kind, len(dilations), self._dil, filter_width, dilation_channels, skip_channels,
+                          cond_channels, pool_stride, num_mixtures, num_flows)
+        _Handle.__init__(self, "hot path", cfg, ("srwn_create", "srwn_destroy", "srwn_set_weight",
+                                                 "srwn_commit_weights", "srwn_set_profiling"))
+        self.kind = kind
+        self.cond_channels = cond_channels
+        self.pool_stride = pool_stride
+        self._pinned = {}
+
+    def check_encoding(self, e, B, T):
+        """The library reads ``cond_channels`` floats for each of the T / pool_stride frames of each of the B rows and
+        knows nothing else of the encoding's shape, so it is checked here, before any launch."""
+        if e.ndim != 3 or e.shape[0] != B or e.shape[2] != self.cond_channels:
+            raise ValueError("encoding must be [B, T/pool_stride, %d]" % self.cond_channels)
+        if e.shape[1] * self.pool_stride != T:
+            raise ValueError("T=%d must equal pool_stride * frames = %d (model.py:183)"
+                             % (T, e.shape[1] * self.pool_stride))
 
     def get_weight(self, name, shape):
         out = np.empty(shape, dtype=np.float32)
         _lib.check(self.lib.srwn_get_weight(self.h, name.encode(), out.ctypes.data_as(ctypes.c_void_p), out.size))
         return out
-
-    def set_profiling(self, enable):
-        _lib.check(self.lib.srwn_set_profiling(self.h, int(bool(enable))))
 
     def last_kernel_ms(self):
         """(elapsed ms, launches, kernel name) of the dominant kernel(s) of the last call."""
@@ -97,19 +142,13 @@ class _Engine(object):
                                                    torch.cuda.current_stream().cuda_stream))
 
     def workspace(self, op, B, T, precision):
-        n = ctypes.c_size_t()
-        _lib.check(self.lib.srwn_workspace_bytes(self.h, op, B, T, precision, ctypes.byref(n)))
-        if self._ws is None or self._ws.numel() < n.value:
-            self._ws = None
-            self._ws = torch.empty(max(n.value, 256), dtype=torch.uint8, device="cuda")
-        return self._ws.data_ptr(), self._ws.numel()
+        return self._ws.get(self.lib.srwn_workspace_bytes, self.h, op, B, T, precision)
 
     def to_device(self, a, key):
         """NumPy / CPU tensor -> CUDA fp32 tensor through a persistent pinned staging buffer."""
-        if isinstance(a, torch.Tensor) and a.is_cuda:
-            return a.float().contiguous(), True
-        t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
-        t = t.float().contiguous()
+        t = _f32(a)
+        if t.is_cuda:
+            return t, True
         if not t.is_pinned():
             buf, ev = self._pinned.get(key, (None, None))
             if buf is None or buf.shape != t.shape:
@@ -135,63 +174,39 @@ class _Engine(object):
         torch.cuda.current_stream().synchronize()
         return buf.numpy().copy()
 
+    def finish(self, t, on_dev, op, B, T, precision):
+        """Result hand-over of a call ``op`` over [B, T] at ``precision``.  Host boundary (NumPy in -> NumPy out): the copy
+        synchronises anyway, so a fused launch that aborted on the device raises here instead of returning partial data.
+        Device-resident results are not synchronised; an abort then refuses the NEXT call on the handle (pinned abort
+        words, include/srwn.h)."""
+        out = self.to_host(t, on_dev)
+        if not on_dev and precision != _lib.FP32:
+            self.check_async(op, B, T, precision)
+        return out
 
-class _EncoderEngine(object):
+
+class _EncoderEngine(_Handle):
     """Owns one libsrwn encoder handle (include/srwn.h, srwn_encoder_*) and its workspace."""
 
     def __init__(self, n_layers, filter_width, encoder_channels, skip_channels, latent_channels, pool_stride):
-        lib = _lib.load()
-        if not torch.cuda.is_available():
-            raise RuntimeError("the SR-WaveNet encoder needs a CUDA device (no CPU fallback)")
         cfg = _lib.EncoderConfig(n_layers, filter_width, encoder_channels, skip_channels, latent_channels,
                                  pool_stride)
-        h = ctypes.c_void_p()
-        _lib.check(lib.srwn_encoder_create(ctypes.byref(cfg), ctypes.byref(h)))
-        self.lib, self.h = lib, h
+        _Handle.__init__(self, "encoder", cfg, ("srwn_encoder_create", "srwn_encoder_destroy", "srwn_encoder_set_weight",
+                                                "srwn_encoder_commit", "srwn_encoder_set_profiling"))
         self.latent_channels, self.pool_stride = latent_channels, pool_stride
-        self._ws = None
-        self.committed = False
-
-    def __del__(self):
-        try:
-            if getattr(self, "h", None):
-                self.lib.srwn_encoder_destroy(self.h)
-                self.h = None
-        except Exception:
-            pass
-
-    def set_weights(self, weights):
-        for name, arr in weights.items():
-            a = np.ascontiguousarray(arr, dtype=np.float32)
-            shape = (ctypes.c_int64 * a.ndim)(*a.shape)
-            _lib.check(self.lib.srwn_encoder_set_weight(self.h, name.encode(), a.ctypes.data_as(ctypes.c_void_p),
-                                                        shape, a.ndim))
-        _lib.check(self.lib.srwn_encoder_commit(self.h, torch.cuda.current_stream().cuda_stream))
-        self.committed = True
 
     def supports(self, prec):
         return bool(self.lib.srwn_encoder_supports(self.h, prec))
-
-    def set_profiling(self, enable):
-        _lib.check(self.lib.srwn_encoder_set_profiling(self.h, int(bool(enable))))
 
     def last_ms(self):
         ms = ctypes.c_float()
         _lib.check(self.lib.srwn_encoder_last_ms(self.h, ctypes.byref(ms)))
         return ms.value
 
-    def workspace(self, B, T, prec):
-        n = ctypes.c_size_t()
-        _lib.check(self.lib.srwn_encoder_workspace_bytes(self.h, B, T, prec, ctypes.byref(n)))
-        if self._ws is None or self._ws.numel() < n.value:
-            self._ws = None
-            self._ws = torch.empty(max(n.value, 256), dtype=torch.uint8, device="cuda")
-        return self._ws.data_ptr(), self._ws.numel()
-
     def encode(self, x, prec, check=True):
         """x: CUDA fp32 [B,T] -> CUDA fp32 [B, T // P, latent]."""
         B, T = x.shape
-        ws, wsn = self.workspace(B, T, prec)
+        ws, wsn = self._ws.get(self.lib.srwn_encoder_workspace_bytes, self.h, B, T, prec)
         out = torch.empty(B, T // self.pool_stride, self.latent_channels, dtype=torch.float32, device="cuda")
         _lib.check(self.lib.srwn_teacher_encode(self.h, x.data_ptr(), out.data_ptr(), B, T, prec, ws, wsn, _stream()))
         if check and prec != _lib.FP32:
@@ -216,8 +231,10 @@ def _with_conditions(encoding, conditions, condition_size):
     return encoding
 
 
-class _CheckpointMixin(object):
-    """Stand-in for tf.train.Saver (model.py:217-239).  ``save`` writes ``<logdir>/model.ckpt-<step>.npz`` (name-keyed,
+class _Model(object):
+    """What the teacher and the student share: Glorot-initialised weights with zero biases, the host copy of the weights
+    that ``get_weights`` returns, the precisions the engine offers, and the stand-in for tf.train.Saver
+    (model.py:217-239).  ``save`` writes ``<logdir>/model.ckpt-<step>.npz`` (name-keyed,
     TF variable names) plus the ``checkpoint`` state file, throttled to once per 60 s unless ``force``; with
     ``checkpoint_format = "tf"`` it writes a TensorFlow tensor bundle (``.index`` + ``.data-00000-of-00001``) instead.
     ``load`` restores whichever of the two the state file points to, so a checkpoint directory written by the
@@ -226,13 +243,26 @@ class _CheckpointMixin(object):
 
     checkpoint_format = "npz"
 
+    def _init_weights(self, w):
+        for k in w:                      # TF initialises biases to zero (ops.py:18, tf.layers default)
+            if k.endswith('Bias') or k.endswith('/bias'):
+                w[k][...] = 0
+        self._weights = {}
+        self.set_weights(w)
+
+    def _mirror_weights(self, weights):
+        self._weights.update({k: np.array(v, dtype=np.float32) for k, v in weights.items()})
+
+    def available_precisions(self):
+        op = _lib.OP_TEACHER_LOGITS if self._eng.kind == _lib.TEACHER else _lib.OP_STUDENT_FORWARD
+        return ["fp32", "fp16"] if self._eng.lib.srwn_supports(self._eng.h, op, _lib.FP16) else ["fp32"]
+
     def _save(self, logdir, global_step, force):
         if force or time.time() - self.last_checkpoint_time > 60:
             if not os.path.isdir(logdir):
                 os.makedirs(logdir)
             path = os.path.join(logdir, 'model.ckpt-%d' % global_step)
             if self.checkpoint_format == "tf":
-                from . import tf_checkpoint
                 tf_checkpoint.write_checkpoint(path, self.get_weights())
             else:
                 np.savez(path + '.npz', **self.get_weights())
@@ -247,16 +277,12 @@ class _CheckpointMixin(object):
 
     def _load(self, logdir):
         if logdir is not None and os.path.exists(logdir):
-            state = os.path.join(logdir, 'checkpoint')
-            if os.path.exists(state):
-                with open(state) as f:
-                    name = f.readline().split('"')[1]
-                path = name if os.path.isabs(name) else os.path.join(logdir, name)
+            path = tf_checkpoint.latest_checkpoint(logdir)
+            if path is not None:
                 if os.path.exists(path + '.npz'):
                     with np.load(path + '.npz') as z:
                         self.set_weights({k: z[k] for k in z.files})
                 elif os.path.exists(path + '.index'):
-                    from . import tf_checkpoint
                     known = self.get_weights()
                     found = {k: v for k, v in tf_checkpoint.read_checkpoint(path).items()
                              if k in known and tuple(v.shape) == tuple(known[k].shape)}
@@ -272,7 +298,7 @@ class _CheckpointMixin(object):
         return None
 
 
-class WaveNetAutoEncoder(_CheckpointMixin):
+class WaveNetAutoEncoder(_Model):
     """model.py:75-285: decoder (the hot path) and encoder; constructor signature kept verbatim."""
 
     def __init__(self, input_size, condition_size, num_mixtures, dilations, filter_width=2,
@@ -292,6 +318,7 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         self.learning_rate = learning_rate
         self.precision = "fp32"
         self.seed = int.from_bytes(os.urandom(7), "little")      # the reference's RNG is unseeded (SURVEY F10); set for reproducible draws
+        self._noise_calls = 0
         self.last_checkpoint_time = time.time()
         self.createNetwork()
 
@@ -310,11 +337,7 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         we = synth.make_encoder_weights(len(self.dilations), self.filter_width, self.encoder_channels,
                                         self.skip_channels, self.latent_channels, seed=None, gain=1.0)
         w.update(we)
-        for k in w:                      # TF initialises biases to zero (ops.py:18, tf.layers default)
-            if k.endswith('Bias') or k.endswith('/bias'):
-                w[k][...] = 0
-        self._weights = {}
-        self.set_weights(w)
+        self._init_weights(w)
 
     def createEncoder(self, h, reuse=False, precision=None):
         """model.py:137-155 -> encoding [B, T/pool_stride, latent].  h [B,T,1] or [B,T]."""
@@ -342,13 +365,10 @@ class WaveNetAutoEncoder(_CheckpointMixin):
             self._eng.set_weights(dec)
         if enc:
             self._enc_eng.set_weights(enc)
-        self._weights.update({k: np.array(v, dtype=np.float32) for k, v in weights.items()})
+        self._mirror_weights(weights)
 
     def get_weights(self):
         return dict(self._weights)
-
-    def available_precisions(self):
-        return ["fp32", "fp16"] if _fused_available(self._eng) else ["fp32"]
 
     def load(self, logdir):
         return self._load(logdir)
@@ -361,12 +381,9 @@ class WaveNetAutoEncoder(_CheckpointMixin):
                         dilation_channels=32, input_size=0):
         """A teacher built from a checkpoint directory alone (what ParallelWaveNet(teacher=<dir>) needs,
         model.py:323-334): mixtures, skip and encoder widths come from the stored variable shapes."""
-        state = os.path.join(logdir, 'checkpoint')
-        if not os.path.exists(state):
+        path = tf_checkpoint.latest_checkpoint(logdir)
+        if path is None:
             raise IOError("no teacher checkpoint under %s (expected the files WaveNetAutoEncoder.save writes)" % logdir)
-        with open(state) as f:
-            name = f.readline().split('"')[1]
-        path = name if os.path.isabs(name) else os.path.join(logdir, name)
         L = len(dilations)
         k_head2 = '%sconv1d_%d/kernel' % (synth.TEACHER_PREFIX, 3 * L + 1)
         k_enc0 = '%snc_conv_NC/conv1d/kernel' % synth.ENCODER_PREFIX
@@ -374,7 +391,6 @@ class WaveNetAutoEncoder(_CheckpointMixin):
             with np.load(path + '.npz') as z:
                 head2, enc0 = z[k_head2].shape, z[k_enc0].shape
         else:                                              # a tf.train.Saver checkpoint (tensor bundle)
-            from . import tf_checkpoint
             shapes = {n: sh for n, sh, _ in tf_checkpoint.list_variables(path)}
             head2, enc0 = shapes[k_head2], shapes[k_enc0]
         t = cls(input_size=input_size, condition_size=condition_size, num_mixtures=head2[2] // 4, dilations=dilations,
@@ -415,15 +431,6 @@ class WaveNetAutoEncoder(_CheckpointMixin):
     def _prec(self, precision):
         return _lib.PRECISIONS[precision or self.precision]
 
-    def _finish(self, t, on_dev, op, B, T, prec):
-        """Result hand-over.  Host boundary (NumPy in -> NumPy out): the copy synchronises anyway, so a fused launch that
-        aborted on the device raises here instead of returning partial data.  Device-resident results are not
-        synchronised; an abort then refuses the NEXT call on the handle (pinned abort words, include/srwn.h)."""
-        out = self._eng.to_host(t, on_dev)
-        if not on_dev and prec != _lib.FP32:
-            self._eng.check_async(op, B, T, prec)
-        return out
-
     def get_logits(self, inputs, encoding, conditions=None, precision=None):
         """model.py:279-285 -> logits [B,T,4M]."""
         eng = self._eng
@@ -431,13 +438,13 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         x, on_dev = eng.to_device(inputs, "x")
         e, _ = eng.to_device(enc, "enc")
         B, T = x.shape
-        self._check(e, B, T)
+        eng.check_encoding(e, B, T)
         prec = self._prec(precision)
         ws, wsn = eng.workspace(_lib.OP_TEACHER_LOGITS, B, T, prec)
         logits = torch.empty(B, T, 4 * self.num_mixtures, dtype=torch.float32, device="cuda")
         _lib.check(eng.lib.srwn_teacher_logits(eng.h, x.data_ptr(), e.data_ptr(), logits.data_ptr(), B, T,
                                                prec, ws, wsn, _stream()))
-        return self._finish(logits, on_dev, _lib.OP_TEACHER_LOGITS, B, T, prec)
+        return eng.finish(logits, on_dev, _lib.OP_TEACHER_LOGITS, B, T, prec)
 
     def nll(self, inputs, encoding, conditions=None, scored=None, sum_all=True, precision=None):
         """``loss_encoding`` of model.py:114-115: teacher-forced mixture-of-logistics negative
@@ -450,18 +457,18 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         e, _ = eng.to_device(enc, "enc")
         xs = x if scored is None else eng.to_device(scored, "xs")[0]
         B, T = x.shape
-        self._check(e, B, T)
+        eng.check_encoding(e, B, T)
         prec = self._prec(precision)
         ws, wsn = eng.workspace(_lib.OP_TEACHER_NLL, B, T, prec)
         if sum_all:
             out = torch.empty(1, dtype=torch.float32, device="cuda")
             _lib.check(eng.lib.srwn_teacher_nll(eng.h, x.data_ptr(), e.data_ptr(), xs.data_ptr(), None,
                                                 out.data_ptr(), None, B, T, prec, ws, wsn, _stream()))
-            return out if on_dev else float(self._finish(out, False, _lib.OP_TEACHER_NLL, B, T, prec)[0])
+            return out if on_dev else float(eng.finish(out, False, _lib.OP_TEACHER_NLL, B, T, prec)[0])
         out = torch.empty(B, T, 1, dtype=torch.float32, device="cuda")
         _lib.check(eng.lib.srwn_teacher_nll(eng.h, x.data_ptr(), e.data_ptr(), xs.data_ptr(), out.data_ptr(),
                                             None, None, B, T, prec, ws, wsn, _stream()))
-        return self._finish(out, on_dev, _lib.OP_TEACHER_NLL, B, T, prec)
+        return eng.finish(out, on_dev, _lib.OP_TEACHER_NLL, B, T, prec)
 
     def nll_stream(self, batches, precision=None, depth=2):
         """Scores a sequence of host batches: ``batches`` yields ``(inputs [B,T], encoding [B,T/P,C])`` (NumPy arrays or CPU
@@ -479,12 +486,8 @@ class WaveNetAutoEncoder(_CheckpointMixin):
                       out=torch.empty(1, dtype=torch.float32, device="cuda"), host=torch.empty(1, dtype=torch.float32, pin_memory=True))
                  for _ in range(depth)]
 
-        def host32(a):
-            t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
-            return t.float().contiguous()
-
         def upload(slot, batch):
-            x, e = host32(batch[0]), host32(_with_conditions(batch[1], None, self.condition_size))
+            x, e = _f32(batch[0]), _f32(_with_conditions(batch[1], None, self.condition_size))
             if slot["x"] is None or slot["x"].shape != x.shape or slot["e"].shape != e.shape:
                 slot["x"] = torch.empty(x.shape, dtype=torch.float32, device="cuda")
                 slot["e"] = torch.empty(e.shape, dtype=torch.float32, device="cuda")
@@ -503,7 +506,7 @@ class WaveNetAutoEncoder(_CheckpointMixin):
 
         def launch(slot):
             B, T = slot["x"].shape
-            self._check(slot["e"], B, T)
+            eng.check_encoding(slot["e"], B, T)
             ws, wsn = eng.workspace(_lib.OP_TEACHER_NLL, B, T, prec)
             compute.wait_event(slot["up"])
             _lib.check(eng.lib.srwn_teacher_nll(eng.h, slot["x"].data_ptr(), slot["e"].data_ptr(), slot["x"].data_ptr(), None,
@@ -583,7 +586,7 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         e, on_dev = eng.to_device(enc, "enc")
         B = e.shape[0]
         T = num_samples if num_samples is not None else e.shape[1] * self.pool_stride
-        self._check(e, B, T)
+        eng.check_encoding(e, B, T)
         if prefix is not None:
             xp = eng.to_device(prefix, "prefix")[0]
             if xp.ndim != 2 or xp.shape[0] != B or xp.shape[1] > T:
@@ -593,13 +596,9 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         if state is not None and (state.batch_size != B or state.precision != precision):
             raise ValueError("state was made for batch_size=%d, precision=%r; this call has %d, %r"
                              % (state.batch_size, state.precision, B, precision))
-        lo, hi = 1e-5, 1.0 - 1e-5            # ops.py:187, 196
-        if u1 is None or u2 is None:
-            self._noise_calls = getattr(self, "_noise_calls", 0) + 1
-        u1 = eng.random_uniform((B, T, self.num_mixtures), self.seed, 2 * self._noise_calls, lo, hi) if u1 is None \
-            else eng.to_device(u1, "u1")[0]
-        u2 = eng.random_uniform((B, T), self.seed, 2 * self._noise_calls + 1, lo, hi) if u2 is None \
-            else eng.to_device(u2, "u2")[0]
+        d1, d2 = self._draw_uniforms(B, T) if u1 is None or u2 is None else (None, None)
+        u1 = d1 if u1 is None else eng.to_device(u1, "u1")[0]
+        u2 = d2 if u2 is None else eng.to_device(u2, "u2")[0]
         prec = _lib.PRECISIONS[precision]
         if not eng.lib.srwn_supports(eng.h, _lib.OP_TEACHER_GENERATE, prec):
             raise RuntimeError("generate(precision=%r) is not supported for this configuration" % precision)
@@ -616,6 +615,8 @@ class WaveNetAutoEncoder(_CheckpointMixin):
             _lib.check(eng.lib.srwn_teacher_generate_resume(eng.h, state.data_ptr(), e.data_ptr(), u1.data_ptr(),
                                                             u2.data_ptr(), xp.data_ptr() if n else None, n, x.data_ptr(),
                                                             lg_ptr, B, T, prec, ws, wsn, _stream()))
+        # not eng.finish: the generation kernel's abort flag lives in the workspace and is not sticky, so no later call
+        # would see it; device-resident results are checked here too
         if prec != _lib.FP32:
             eng.check_async(_lib.OP_TEACHER_GENERATE, B, T, prec)
         if zero_last:
@@ -640,7 +641,7 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         if x.ndim != 2 or x.shape[0] != B or x.shape[1] < 1:
             raise ValueError("audio must be [B=%d, n] with n >= 1, got %s" % (B, tuple(x.shape)))
         n = int(x.shape[1])
-        self._check(e, B, n)
+        eng.check_encoding(e, B, n)
         prec = _lib.PRECISIONS.get(state.precision)
         if prec is None or not eng.lib.srwn_supports(eng.h, _lib.OP_TEACHER_PREFILL, prec):
             raise ValueError("prefill(precision=%r) is not supported for this configuration" % state.precision)
@@ -664,22 +665,18 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         state, both moved in with ``GenerationState.splice``.  Each call takes every slot's frames and uniforms at that
         slot's own offset (idle slots get zeros); what a request generates past its end is dropped.  With injected
         uniforms a request's audio is bit for bit that of generating it alone (B = 1, the same prime through prefill)."""
-        eng, P, M, cs = self._eng, self.pool_stride, self.num_mixtures, self.condition_size
+        P, M, cs = self.pool_stride, self.num_mixtures, self.condition_size
         slots, chunk = int(slots), int(chunk)
         if slots < 1 or chunk < P or chunk % P:
             raise ValueError("slots must be positive and chunk a positive multiple of pool_stride=%d" % P)
 
-        def dev(a):
-            t = a if isinstance(a, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(a, dtype=np.float32))
-            return t.float().cuda().contiguous()
-
         reqs = []
         for i, r in enumerate(requests):
             r = r if isinstance(r, dict) else {"encoding": r}
-            e = dev(r["encoding"])
+            e = _cuda_f32(r["encoding"])
             if e.ndim != 2 or e.shape[1] != self.latent_channels:
                 raise ValueError("request %d: encoding must be [F, %d]" % (i, self.latent_channels))
-            prime = dev(r["prime"]).reshape(-1) if r.get("prime") is not None else None
+            prime = _cuda_f32(r["prime"]).reshape(-1) if r.get("prime") is not None else None
             n0 = 0 if prime is None else int(prime.shape[0])
             need = e.shape[0] * P - n0
             if n0 % P or need < 0:
@@ -689,14 +686,14 @@ class WaveNetAutoEncoder(_CheckpointMixin):
             if cs:
                 if r.get("conditions") is None:
                     raise ValueError("request %d: condition_size > 0 needs `conditions`" % i)
-                c = dev(r["conditions"]).reshape(-1)
+                c = _cuda_f32(r["conditions"]).reshape(-1)
                 if c.shape[0] != cs:
                     raise ValueError("request %d: conditions must be [%d]" % (i, cs))
             inj = r.get("u1") is not None or r.get("u2") is not None
             if inj:
                 if r.get("u1") is None or r.get("u2") is None:
                     raise ValueError("request %d: inject both u1 and u2, or neither" % i)
-                u1, u2 = dev(r["u1"]), dev(r["u2"]).reshape(-1)
+                u1, u2 = _cuda_f32(r["u1"]), _cuda_f32(r["u2"]).reshape(-1)
                 if tuple(u1.shape) != (need, M) or u2.shape[0] != need:
                     raise ValueError("request %d: u1 must be [%d, %d] and u2 [%d]" % (i, need, M, need))
             reqs.append({"enc": e, "prime": prime, "n0": n0, "need": need, "cond": c,
@@ -733,7 +730,6 @@ class WaveNetAutoEncoder(_CheckpointMixin):
         slot_pos = np.zeros(slots, np.int64)                     # samples it has generated
         ar_f = torch.arange(chunk // P, device="cuda")
         ar_s = torch.arange(chunk, device="cuda")
-        lo, hi = 1e-5, 1.0 - 1e-5                                # ops.py:187, 196
         nxt = 0
         while True:
             # fill the free slots from the queue
@@ -779,9 +775,7 @@ class WaveNetAutoEncoder(_CheckpointMixin):
             u1_c, u2_c = u1_all[uidx], u2_all[uidx]
             drawn = np.flatnonzero(active & (ubase[rq] < 0))
             if drawn.size:                                         # uniforms of requests without injected ones
-                self._noise_calls = getattr(self, "_noise_calls", 0) + 1
-                d1 = eng.random_uniform((slots, chunk, M), self.seed, 2 * self._noise_calls, lo, hi)
-                d2 = eng.random_uniform((slots, chunk), self.seed, 2 * self._noise_calls + 1, lo, hi)
+                d1, d2 = self._draw_uniforms(slots, chunk)
                 dr = torch.from_numpy(drawn).cuda()
                 u1_c[dr], u2_c[dr] = d1[dr], d2[dr]
             cond_c = cond_all[torch.from_numpy(np.where(active, slot_req, N)).cuda()] if cs else None
@@ -794,16 +788,17 @@ class WaveNetAutoEncoder(_CheckpointMixin):
                 slot_req[s] = -1
                 yield i, self._request_audio(out_all[obase[i]:obase[i] + need_np[i]], reqs[i]["on_dev"])
 
+    def _draw_uniforms(self, rows, T):
+        """The sampler's two U(1e-5, 1 - 1e-5) draws (ops.py:187, 196), [rows, T, M] and [rows, T], on the device from
+        Philox streams 2k and 2k + 1 of ``seed``, k counting the calls that draw: a seeded model repeats its noise."""
+        self._noise_calls += 1
+        lo, hi = 1e-5, 1.0 - 1e-5
+        return (self._eng.random_uniform((rows, T, self.num_mixtures), self.seed, 2 * self._noise_calls, lo, hi),
+                self._eng.random_uniform((rows, T), self.seed, 2 * self._noise_calls + 1, lo, hi))
+
     @staticmethod
     def _request_audio(x, on_dev):
         return x.clone() if on_dev else x.cpu().numpy()
-
-    def _check(self, e, B, T):
-        if e.ndim != 3 or e.shape[0] != B or e.shape[2] != self.latent_channels + self.condition_size:
-            raise ValueError("encoding must be [B, T/pool_stride, %d]" % (self.latent_channels + self.condition_size))
-        if e.shape[1] * self.pool_stride != T:
-            raise ValueError("T=%d must equal pool_stride * frames = %d (model.py:183)"
-                             % (T, e.shape[1] * self.pool_stride))
 
 
 class GenerationState(object):
@@ -857,12 +852,7 @@ class GenerationState(object):
         return self.buffer.data_ptr()
 
 
-def _fused_available(eng):
-    op = _lib.OP_TEACHER_LOGITS if eng.kind == _lib.TEACHER else _lib.OP_STUDENT_FORWARD
-    return bool(eng.lib.srwn_supports(eng.h, op, _lib.FP16))
-
-
-class ParallelWaveNet(_CheckpointMixin):
+class ParallelWaveNet(_Model):
     """model.py:290-656.  ``teacher`` is a checkpoint directory in the reference; here it may also
     be a ``WaveNetAutoEncoder`` instance or None.  Methods keep the explicit ``sess`` first argument
     (ignored)."""
@@ -902,14 +892,11 @@ class ParallelWaveNet(_CheckpointMixin):
         self._eng = _Engine(_lib.STUDENT, self.dilations, self.filter_width, self.dilation_channels,
                             self.skip_channels, self.latent_channels + self.condition_size,
                             self.pool_stride, num_flows=self.num_flows)
+        self._stft_ws = _Workspace()      # the power loss's STFT calls take no handle: their workspace is kept here
         w = synth.make_student_weights(self.dilations, self.num_flows, self.filter_width,
                                        self.dilation_channels, self.skip_channels,
                                        self.latent_channels + self.condition_size, seed=None)
-        for k in w:
-            if k.endswith('Bias') or k.endswith('/bias'):
-                w[k][...] = 0
-        self._weights = {}
-        self.set_weights(w)
+        self._init_weights(w)
 
     def _flow_model(self, scope):
         """A one-flow network holding the variables of ``scope`` ('Flow<i>'): model.py:457-486 builds each flow as its own
@@ -945,15 +932,12 @@ class ParallelWaveNet(_CheckpointMixin):
     def set_weights(self, weights):
         """name -> ndarray with TF variable names (``ParallelWaveNet/Flow{f}/Flow{f}/...``)."""
         self._eng.set_weights(weights)
-        self._weights.update({k: np.array(v, dtype=np.float32) for k, v in weights.items()})
+        self._mirror_weights(weights)
 
     def get_weights(self):
         if getattr(self, "_packed_stale", False):        # trained on the device since the last read-back
             self.sync_weights()
         return dict(self._weights)
-
-    def available_precisions(self):
-        return ["fp32", "fp16"] if _fused_available(self._eng) else ["fp32"]
 
     def load(self, sess, logdir):
         if isinstance(self.teacher, str):
@@ -973,8 +957,7 @@ class ParallelWaveNet(_CheckpointMixin):
         else:
             z, on_dev = eng.to_device(inputs, "z")
             B, T = z.shape
-        if e.ndim != 3 or e.shape[0] != B or e.shape[1] * self.pool_stride != T:
-            raise ValueError("encoding must be [B, T/pool_stride, C] with T == pool_stride * frames")
+        eng.check_encoding(e, B, T)
         prec = _lib.PRECISIONS[precision or self.precision]
         if prec != _lib.FP32 and getattr(self, "_packed_stale", False):
             self.sync_weights()
@@ -989,29 +972,20 @@ class ParallelWaveNet(_CheckpointMixin):
             bufs.pop("z", None)
             _lib.check(eng.lib.srwn_student_forward(eng.h, z.data_ptr(), e.data_ptr(), g("out"), g("s_tot"),
                                                     g("mu_tot"), g("x_last"), B, T, prec, ws, wsn, _stream()))
-        self._last_call = (B, T, prec)
-        return bufs, on_dev
-
-    def _to_host(self, t, on_dev):
-        """see WaveNetAutoEncoder._finish"""
-        out = self._eng.to_host(t, on_dev)
-        B, T, prec = self._last_call
-        if not on_dev and prec != _lib.FP32:
-            self._eng.check_async(_lib.OP_STUDENT_FORWARD, B, T, prec)
-        return out
+        return bufs, (on_dev, _lib.OP_STUDENT_FORWARD, B, T, prec)
 
     def generate(self, sess, inputs, encoding, conditions=None, precision=None):
         """model.py:570-576 -> out [B,T,1] = clip(z*s_tot + mu_tot, -1, 1).  ``inputs=None`` draws the logistic noise of
         student.py:172 on the device (inside the fused flow kernel on the fp16 path): nothing but the encoding is uploaded."""
-        bufs, on_dev = self._forward(inputs, encoding, conditions, precision)
-        return self._to_host(bufs["out"][:, :, None], on_dev)
+        bufs, call = self._forward(inputs, encoding, conditions, precision)
+        return self._eng.finish(bufs["out"][:, :, None], *call)
 
     def forward_all(self, inputs, encoding, conditions=None, precision=None):
         """out, s_tot, mu_tot (model.py:517-535) and the chained flow output, each [B,T]; with ``inputs=None`` also the
         noise ``z`` that was drawn."""
         want = ("out", "s_tot", "mu_tot", "x_last") + (("z",) if inputs is None else ())
-        bufs, on_dev = self._forward(inputs, encoding, conditions, precision, want=want)
-        return {k: self._to_host(v, on_dev) for k, v in bufs.items()}
+        bufs, call = self._forward(inputs, encoding, conditions, precision, want=want)
+        return {k: self._eng.finish(v, *call) for k, v in bufs.items()}
 
     def _entropies(self, inputs, encoding, conditions):
         bufs, _ = self._forward(inputs, encoding, conditions, want=("s_tot",))
@@ -1050,8 +1024,9 @@ class ParallelWaveNet(_CheckpointMixin):
         x, _ = eng.to_device(truth, "truth")
         e, _ = eng.to_device(enc, "enc")
         B, T = z.shape
-        if e.ndim != 3 or e.shape[0] != B or e.shape[1] * self.pool_stride != T or x.shape != z.shape:
-            raise ValueError("inputs/truth must be [B,T], encoding [B, T/pool_stride, C]")
+        eng.check_encoding(e, B, T)
+        if x.shape != z.shape:
+            raise ValueError("truth must be [B,T] like inputs")
         tl = self._teacher_logits(x, e, teacher_logits, teacher_precision).contiguous()
         M = tl.shape[2] // 4
         ws, wsn = eng.workspace(_lib.OP_STUDENT_TRAIN, B, T, _lib.FP32)
@@ -1090,15 +1065,11 @@ class ParallelWaveNet(_CheckpointMixin):
         Returns (power_loss: float64 CUDA tensor [1], d_out [B,T] fp32)."""
         eng = self._eng
         B, T = out.shape
-        n = ctypes.c_size_t()
-        _lib.check(eng.lib.srwn_stft_workspace_bytes(B, T, frame_length, frame_step, ctypes.byref(n)))
-        if getattr(self, "_stft_ws", None) is None or self._stft_ws.numel() < n.value:
-            self._stft_ws = torch.empty(max(n.value, 256), dtype=torch.uint8, device="cuda")
+        ws, wsn = self._stft_ws.get(eng.lib.srwn_stft_workspace_bytes, B, T, frame_length, frame_step)
         p = torch.empty(1, dtype=torch.float64, device="cuda")
         g = torch.empty_like(out)
         _lib.check(eng.lib.srwn_stft_power_loss(truth.data_ptr(), out.data_ptr(), float(self.gamma), p.data_ptr(),
-                                                g.data_ptr(), B, T, frame_length, frame_step, self._stft_ws.data_ptr(),
-                                                self._stft_ws.numel(), _stream()))
+                                                g.data_ptr(), B, T, frame_length, frame_step, ws, wsn, _stream()))
         return p, g
 
     def grad_of(self, flat_grads, name):

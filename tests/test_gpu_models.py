@@ -194,6 +194,28 @@ def test_teacher_errors(srwn):
         t.train(x)
 
 
+@pytest.mark.parametrize("kind", ["teacher", "student"])
+def test_encoding_channel_count_is_refused_before_any_launch(srwn, kind):
+    """The library reads latent_channels + condition_size floats per frame and is only given a pointer: an encoding with
+    one channel too few would be read past its end, one too many would be misread.  Both are refused before a launch."""
+    C, P, B, T = 32, 128, 2, 512
+    x, z = synth.synthetic_audio(B, T), synth.logistic_noise(B, T)
+    if kind == "teacher":
+        m, _ = _teacher(srwn, [1, 2, 4], C=C, P=P)
+        calls = [lambda e: m.get_logits(x, e), lambda e: m.nll(x, e), lambda e: m.generate(e)]
+    else:
+        m, _ = _student(srwn, [1, 2, 4], 2, C=C, P=P)
+        calls = [lambda e: m.generate(None, z, e), lambda e: m.generate(None, None, e),
+                 lambda e: m.forward_all(z, e), lambda e: m.loss_and_grads(z, x, e)]
+    launches = srwn._lib.launch_count()
+    for channels in (C - 1, C + 1):
+        enc = synth.synthetic_encoding(B, T // P, channels)
+        for call in calls:
+            with pytest.raises(ValueError):
+                call(enc)
+    assert srwn._lib.launch_count() == launches
+
+
 def test_generate_golden_small(srwn, golden_small):
     g = golden_small
     dil = [int(d) for d in g["dilations"]]
