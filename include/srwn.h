@@ -61,7 +61,8 @@ enum srwn_op {               /* argument of srwn_workspace_bytes */
   SRWN_OP_TEACHER_GENERATE = 2,
   SRWN_OP_STUDENT_FORWARD = 3,
   SRWN_OP_STUDENT_TRAIN = 4,   /* workspace of srwn_student_forward_train + srwn_student_backward */
-  SRWN_OP_TEACHER_PREFILL = 5  /* workspace of srwn_generate_state_prefill (T = its n) */
+  SRWN_OP_TEACHER_PREFILL = 5, /* workspace of srwn_generate_state_prefill (T = its n) */
+  SRWN_OP_STUDENT_STREAM = 6   /* workspace of srwn_student_forward_resume (T = its S) */
 };
 
 /* Constructor arguments of WaveNetAutoEncoder (model.py:76-77) / ParallelWaveNet
@@ -218,6 +219,33 @@ int srwn_student_forward(srwn_handle_t h, const float* z, const float* enc, floa
 int srwn_student_sample(srwn_handle_t h, uint64_t seed, uint64_t stream_id, const float* enc, float* out,
                         float* s_tot, float* mu_tot, float* x_last, float* z_out, int32_t B, int32_t T,
                         int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
+/* Synthesis in chunks: the same flows continued across calls through a caller-owned DEVICE state (audio while the
+ * encoding is still arriving, clips longer than one call's workspace).
+ * srwn_student_state_bytes: size of the state of B utterances for `precision` (SRWN_FP32 or SRWN_FP16; it does not depend
+ *   on the clip length).  It holds, per flow, the last H samples of that flow's input (z for flow 0, flow f-1's output
+ *   after), the last H/P frames of `enc`, the position t0 and a signature (B, precision, flows, layers, sum(d), P, C); its
+ *   first 8 bytes are t0, an int64.  H = (filter_width - 1) * sum(d) + filter_width rounded up to a multiple of
+ *   pool_stride P: the rows one output sample of a flow depends on.
+ * srwn_student_state_reset: zero histories, t0 = 0.  A state is used only on the handle, B and precision it was last
+ *   reset for.
+ * srwn_student_forward_resume: the S samples t0 .. t0+S-1 (S > 0 and t0 multiples of P).  z [B,S] their noise, or NULL
+ *   to draw it on the device (element b*S + s of Philox stream (seed, stream_id), as srwn_student_sample; z_out [B,S],
+ *   optional, receives the draws); enc [B,S/P,C] their frames; out, and optionally s_tot, mu_tot, x_last, as
+ *   srwn_student_forward, each [B,S].  The host passes t0 (it sets how many carried rows the call recomputes:
+ *   min(t0, H)); the state holds t0 as well, and a call whose t0 disagrees raises the handle's abort words on the device
+ *   (no synchronisation): the outputs of that call are invalid, the state is left as it was, later calls are refused
+ *   with SRWN_ERR_CUDA until srwn_check_async_error(SRWN_OP_STUDENT_STREAM, ...) reports it.  Afterwards the state holds
+ *   t0+S.  Workspace: srwn_workspace_bytes(SRWN_OP_STUDENT_STREAM, B, S).  With injected noise, any split of a clip into
+ *   such calls gives bit for bit the out, s_tot, mu_tot and x_last of one srwn_student_forward over the clip, in both
+ *   precisions.  Refused with SRWN_ERR_INVALID before any work: a null state, enc or out, a teacher handle, S <= 0 or
+ *   S % P != 0, t0 < 0 or t0 % P != 0, a state not reset on this handle for this B and precision; SRWN_BF16 with
+ *   SRWN_ERR_UNSUPPORTED. */
+int srwn_student_state_bytes(srwn_handle_t h, int32_t B, int32_t precision, size_t* bytes);
+int srwn_student_state_reset(srwn_handle_t h, void* state, int32_t B, int32_t precision, void* stream);
+int srwn_student_forward_resume(srwn_handle_t h, void* state, int64_t t0, const float* z, uint64_t seed, uint64_t stream_id,
+                                const float* enc, float* out, float* s_tot, float* mu_tot, float* x_last, float* z_out,
+                                int32_t B, int32_t S, int32_t precision, void* workspace, size_t workspace_bytes,
+                                void* stream);
 int srwn_random_logistic(float* out, int64_t n, uint64_t seed, uint64_t stream_id, void* stream);
 int srwn_random_uniform(float* out, int64_t n, uint64_t seed, uint64_t stream_id, float lo, float hi, void* stream);
 

@@ -12,7 +12,8 @@ ABI_VERSION = 7      # SRWN_ABI_VERSION in include/srwn.h
 OK, ERR_INVALID, ERR_CUDA, ERR_WEIGHTS, ERR_UNSUPPORTED, ERR_WORKSPACE = range(6)
 TEACHER, STUDENT = 0, 1
 FP32, BF16, FP16 = 0, 1, 2
-OP_TEACHER_LOGITS, OP_TEACHER_NLL, OP_TEACHER_GENERATE, OP_STUDENT_FORWARD, OP_STUDENT_TRAIN, OP_TEACHER_PREFILL = range(6)
+OP_TEACHER_LOGITS, OP_TEACHER_NLL, OP_TEACHER_GENERATE, OP_STUDENT_FORWARD, OP_STUDENT_TRAIN, OP_TEACHER_PREFILL, \
+    OP_STUDENT_STREAM = range(7)
 DISTILL_SUMS_LEN = 1024   # SRWN_DISTILL_SUMS_LEN
 PRECISIONS = {"fp32": FP32, "fp16": FP16}      # BF16 is refused by the library (include/srwn.h)
 
@@ -72,6 +73,10 @@ SIGNATURES = {
                                                   _i32, _i32, _vp]),
     "srwn_student_forward": (ctypes.c_int, [_vp, _fp, _fp, _fp, _fp, _fp, _fp, _i32, _i32, _i32, _vp, _sz, _vp]),
     "srwn_student_sample": (ctypes.c_int, [_vp, ctypes.c_uint64, ctypes.c_uint64, _fp, _fp, _fp, _fp, _fp, _fp, _i32, _i32, _i32, _vp, _sz, _vp]),
+    "srwn_student_state_bytes": (ctypes.c_int, [_vp, _i32, _i32, ctypes.POINTER(_sz)]),
+    "srwn_student_state_reset": (ctypes.c_int, [_vp, _vp, _i32, _i32, _vp]),
+    "srwn_student_forward_resume": (ctypes.c_int, [_vp, _vp, _i64, _fp, ctypes.c_uint64, ctypes.c_uint64, _fp, _fp, _fp, _fp,
+                                                   _fp, _fp, _i32, _i32, _i32, _vp, _sz, _vp]),
     "srwn_random_logistic": (ctypes.c_int, [_fp, _i64, ctypes.c_uint64, ctypes.c_uint64, _vp]),
     "srwn_random_uniform": (ctypes.c_int, [_fp, _i64, ctypes.c_uint64, ctypes.c_uint64, ctypes.c_float, ctypes.c_float, _vp]),
     "srwn_weights_flat": (ctypes.c_int, [_vp, _fp, _i64, _i32, _vp]),

@@ -185,7 +185,7 @@ extern "C" int srwn_create(const srwn_config_t* cfg, srwn_handle_t* out) {
   c->committed = false; c->device_dirty = false;
   c->d_weights = nullptr; c->d_dilations = nullptr; c->d_queue_off = nullptr;
   c->d_packed = nullptr; c->packed_bytes = 0; c->d_ar_packed = nullptr;
-  c->d_part = nullptr; c->part_B = c->part_T = c->part_teams = c->part_G = 0; c->part_team_req = -1;
+  c->d_part = nullptr; c->part_B = c->part_T = c->part_out0 = c->part_teams = c->part_G = 0; c->part_team_req = -1;
   c->team_size = 0; c->h_err = nullptr; c->wait_limit_clocks = 1000000000LL;
   c->profiling = 0; c->prof_launches = 0; c->prof_name = "";
   c->prof_ev[0] = c->prof_ev[1] = nullptr;
@@ -224,9 +224,10 @@ extern "C" int srwn_create(const srwn_config_t* cfg, srwn_handle_t* out) {
     c->packed_bytes = fused_packed_bytes(c);
     if (c->packed_bytes) e = cudaMalloc(&c->d_packed, c->packed_bytes);
     if (e == cudaSuccess && c->packed_bytes) e = cudaMalloc(&c->d_part, fused_partition_bytes(c));
-    if (e == cudaSuccess && c->packed_bytes) e = cudaHostAlloc((void**)&c->h_err, 64, cudaHostAllocMapped);
-    if (e == cudaSuccess && c->h_err) memset(c->h_err, 0, 64);
   }
+  // abort words: every handle has them (a student stream call raises them in either precision)
+  if (e == cudaSuccess) e = cudaHostAlloc((void**)&c->h_err, 64, cudaHostAllocMapped);
+  if (e == cudaSuccess) memset(c->h_err, 0, 64);
   if (e != cudaSuccess) {
     int rc = srwn_fail(SRWN_ERR_CUDA, "srwn_create: %s", cudaGetErrorString(e));
     srwn_destroy(c);
@@ -406,7 +407,7 @@ extern "C" int srwn_last_kernel_ms(srwn_handle_t h, float* ms, int32_t* launches
 extern "C" int srwn_check_async_error(srwn_handle_t h, int32_t op, int32_t B, int32_t T, int32_t precision,
                                       void* workspace, size_t workspace_bytes, void* stream) {
   if (!h) return srwn_fail(SRWN_ERR_INVALID, "srwn_check_async_error: null handle");
-  if (precision == SRWN_FP32) {
+  if (precision == SRWN_FP32 && op != SRWN_OP_STUDENT_STREAM) {
     SRWN_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
     return SRWN_OK;
   }
@@ -419,6 +420,7 @@ extern "C" int srwn_check_async_error(srwn_handle_t h, int32_t op, int32_t B, in
 extern "C" int srwn_peek_async_error(srwn_handle_t h) {
   if (!h) return srwn_fail(SRWN_ERR_INVALID, "srwn_peek_async_error: null handle");
   const volatile int* e = h->h_err;
+  if (e && e[0] && e[1] == kAbortStreamPosition) return stream_position_fail(e, "student stream call aborted");
   if (e && e[0])
     return srwn_fail(SRWN_ERR_CUDA, "fused kernel aborted: pipeline wait timed out (code 0x%x, chunk %d, cta %d)", e[1], e[2], e[3]);
   return SRWN_OK;
@@ -427,7 +429,7 @@ extern "C" int srwn_peek_async_error(srwn_handle_t h) {
 // bf16 MMA operands cannot meet the 2e-2 max-abs bound on logits for the 30-layer stack (exact arithmetic on bf16-rounded
 // operands already gives 2.45e-2, tools/bf16_emulation.py; the kernel measured 2.5e-2), so the 16-bit path is fp16
 // (same tensor rate, 8x finer mantissa, measured 3.6e-3) and SRWN_BF16 is refused rather than shipped with a looser bound.
-static int reject_bf16() {
+int reject_bf16() {
   return srwn_fail(SRWN_ERR_UNSUPPORTED, "SRWN_BF16 is not offered: bf16 operands miss the 2e-2 logit bound on this stack; use SRWN_FP16");
 }
 
@@ -437,6 +439,8 @@ extern "C" int srwn_supports(srwn_handle_t h, int32_t op, int32_t precision) {
   if (op == SRWN_OP_TEACHER_PREFILL)
     return h->cfg.kind == SRWN_TEACHER && (precision == SRWN_FP32 || (precision == SRWN_FP16 && ar_mma_supported(h))) ? 1 : 0;
   if (op == SRWN_OP_STUDENT_TRAIN) return h->cfg.kind == SRWN_STUDENT && precision == SRWN_FP32 ? 1 : 0;
+  if (op == SRWN_OP_STUDENT_STREAM)
+    return h->cfg.kind == SRWN_STUDENT && (precision == SRWN_FP32 || (precision == SRWN_FP16 && fused_supported(h))) ? 1 : 0;
   if (teacher_op != (h->cfg.kind == SRWN_TEACHER) || op < 0 || op > SRWN_OP_STUDENT_FORWARD) return 0;
   if (precision == SRWN_FP32) return 1;
   if (op == SRWN_OP_TEACHER_GENERATE) return precision == SRWN_FP16 && ar_mma_supported(h) ? 1 : 0;
@@ -469,6 +473,11 @@ extern "C" int srwn_workspace_bytes(srwn_handle_t h, int32_t op, int32_t B, int3
   if (op == SRWN_OP_STUDENT_TRAIN) {
     if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
     *bytes = train_workspace_bytes(h, B, T);
+    return SRWN_OK;
+  }
+  if (op == SRWN_OP_STUDENT_STREAM) {
+    if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
+    *bytes = student_stream_workspace_bytes(h, B, T, precision == SRWN_FP16 ? SRWN_FP16 : SRWN_FP32);
     return SRWN_OK;
   }
   if (op == SRWN_OP_TEACHER_PREFILL) {
@@ -598,18 +607,32 @@ static int student_forward_impl(srwn_handle_t h, const float* z, NoiseSpec noise
     if (rc) return rc;
     z = zbuf; noise.on = 0; z_out = nullptr;
   }
-  const float* xin = z;
-  for (int f = 0; f < F; f++) {                       // model.py:509-513, strictly sequential
+  float* x[17] = {const_cast<float*>(z)};            // flow f reads x[f] and writes x[f + 1] (num_flows <= 16, srwn_create)
+  for (int f = 0; f < F; f++) x[f + 1] = (f == F - 1 && x_last) ? x_last : ((f & 1) ? w.xb : w.xa);
+  const float *scales = nullptr, *means = nullptr;
+  rc = run_student_flows_f32(h, x, enc, B, T, 0, workspace, workspace_bytes, &scales, &means, st);
+  if (rc) return rc;
+  return run_flow_compose(z, noise, z_out, scales, means, F, out, s_tot, mu_tot, (int64_t)n, st);
+}
+
+int run_student_flows_f32(srwn_ctx* h, float* const* x, const float* enc, int B, int T, int t_out, void* ws, size_t ws_bytes,
+                          const float** scales, const float** means, cudaStream_t st) {
+  F32Ws w = carve_f32(h, SRWN_OP_STUDENT_FORWARD, B, T, ws, ws_bytes, false);
+  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  const size_t n = (size_t)B * T;
+  for (int f = 0; f < h->cfg.num_flows; f++) {       // model.py:509-513, strictly sequential
     float* hf = nullptr;
-    rc = run_stack_f32(h, f, xin, enc, B, T, w.h0, w.h1, nullptr, w.cond, &hf, st);
+    int rc = run_stack_f32(h, f, x[f], enc, B, T, w.h0, w.h1, nullptr, w.cond, &hf, st);
     if (rc) return rc;
-    float* xout = (f == F - 1 && x_last) ? x_last : ((f & 1) ? w.xb : w.xa);
-    rc = run_flow_head_f32(h, f, hf, xin, w.scales + (size_t)f * n, w.means + (size_t)f * n, xout,
-                           B, T, st);
+    rc = run_flow_head_f32(h, f, hf, x[f], w.scales + (size_t)f * n, w.means + (size_t)f * n, x[f + 1], B, T, st, t_out);
     if (rc) return rc;
-    xin = xout;
   }
-  return run_flow_compose(z, noise, z_out, w.scales, w.means, F, out, s_tot, mu_tot, (int64_t)n, st);
+  *scales = w.scales; *means = w.means;
+  return SRWN_OK;
+}
+
+size_t student_f32_workspace_bytes(const srwn_ctx* h, int B, int T) {
+  return carve_f32(h, SRWN_OP_STUDENT_FORWARD, B, T, nullptr, 0, false).bytes;
 }
 
 extern "C" int srwn_student_forward(srwn_handle_t h, const float* z, const float* enc, float* out,
@@ -627,6 +650,25 @@ extern "C" int srwn_student_sample(srwn_handle_t h, uint64_t seed, uint64_t stre
   if (!h || !enc || !out) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_sample: null argument");
   return student_forward_impl(h, nullptr, NoiseSpec{seed, stream_id, 1}, z_out, enc, out, s_tot, mu_tot, x_last, B, T,
                               precision, workspace, workspace_bytes, (cudaStream_t)stream);
+}
+
+// ---- student synthesis in chunks through a carried flow state (state format and kernels: student_stream.cu) ----------
+extern "C" int srwn_student_forward_resume(srwn_handle_t h, void* state, int64_t t0, const float* z, uint64_t seed,
+                                           uint64_t stream_id, const float* enc, float* out, float* s_tot, float* mu_tot,
+                                           float* x_last, float* z_out, int32_t B, int32_t S, int32_t precision,
+                                           void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h || !state || !enc || !out) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_forward_resume: null argument");
+  if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
+  if (precision == SRWN_BF16) return reject_bf16();
+  if (precision != SRWN_FP32 && precision != SRWN_FP16) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
+  int rc = check_bt(h, B, S);
+  if (rc) return rc;
+  if (t0 < 0 || t0 % h->cfg.pool_stride)
+    return srwn_fail(SRWN_ERR_INVALID, "t0=%lld must be a non-negative multiple of pool_stride=%d", (long long)t0,
+                     h->cfg.pool_stride);
+  const NoiseSpec noise{seed, stream_id, z ? 0 : 1};
+  return run_student_stream(h, state, t0, z, noise, enc, out, s_tot, mu_tot, x_last, z ? nullptr : z_out, B, S, precision,
+                            workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // ---- student distillation step (model.py:356-401) ----------------------------------------------

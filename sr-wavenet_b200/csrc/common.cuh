@@ -71,12 +71,13 @@ struct srwn_ctx {
   // packed fp16 operand images of the fused kernel, one per stack (built at commit)
   void* d_packed;
   size_t packed_bytes;
-  void* d_part;                       // work partition of the fused kernel for (part_B, part_T, team size): segs | nseg (allocated at create)
-  int part_B, part_T, part_team_req, part_teams, part_G;
+  void* d_part;                       // work partition of the fused kernel for (part_B, part_T, part_out0, team size): segs | nseg (allocated at create)
+  int part_B, part_T, part_out0, part_team_req, part_teams, part_G;
   std::vector<uint8_t> part_host;     // host staging of d_part
   int team_size;                      // srwn_set_team_size: CTAs per team of the fused kernel, 0 = chosen per (B, T)
   long long wait_limit_clocks;        // srwn_set_wait_limit: how long a fused-kernel pipeline wait may spin before aborting
-  int* h_err;                         // pinned, mapped: abort words of the fused kernel [flag, code, chunk, cta]
+  int* h_err;                         // pinned, mapped: abort words of the fused kernel [flag, code, chunk, cta] (or of a student
+                                      // stream call whose t0 disagreed with its state: [flag, kAbortStreamPosition, state t0, call t0])
   void* d_ar_packed;                  // fragment-ordered fp16 weights of the tensor-core generation kernel (built at commit)
   // optional timing of the dominant kernel(s) of the last call (srwn_set_profiling)
   int profiling;
@@ -157,8 +158,21 @@ int run_stack_f32(srwn_ctx* c, int stack, const float* xin, const float* enc, in
                   cudaStream_t st);
 int run_teacher_head_f32(srwn_ctx* c, const float* skip, float* logits, int B, int T,
                          cudaStream_t st);
+// xout is written for rows t >= t_out of each utterance only (scale and mean for every row)
 int run_flow_head_f32(srwn_ctx* c, int stack, const float* h, const float* xin, float* scale,
-                      float* mean, float* xout, int B, int T, cudaStream_t st);
+                      float* mean, float* xout, int B, int T, cudaStream_t st, int t_out = 0);
+// s_tot = prod s_f; mu_tot = sum_f mu_f * prod_{j>f} s_j in the reference's loop order (model.py:517-533), for row i of the
+// [F][n] scales and means (k_flow_compose and the student stream's composition share it: the same bits)
+__device__ __forceinline__ void flow_compose_at(const float* __restrict__ scales, const float* __restrict__ means, int F,
+                                                int64_t n, int64_t i, float& st, float& mt) {
+  st = 1.f; mt = 0.f;
+  for (int f = 0; f < F; f++) {
+    st *= scales[(size_t)f * n + i];
+    float mu = means[(size_t)f * n + i];
+    for (int j = f + 1; j < F; j++) mu *= scales[(size_t)j * n + i];
+    mt += mu;
+  }
+}
 int run_flow_compose(const float* z, NoiseSpec noise, float* z_out, const float* scales, const float* means, int F,
                      float* out, float* s_tot, float* mu_tot, int64_t n, cudaStream_t st);
 // random.cu
@@ -200,6 +214,19 @@ int ar_mma_check_error(const srwn_ctx* c, int B, int T, void* ws, size_t ws_byte
 size_t prefill_workspace_bytes(const srwn_ctx* c, int B, int n, int precision);
 int run_prefill(srwn_ctx* c, const GenState& s, const float* x, const float* enc, int B, int n, int precision, void* ws,
                 size_t ws_bytes, cudaStream_t st);
+// api.cu: the F flows of the fp32 path over [B][T] rows: flow f reads x[f] and writes x[f+1] for rows t >= t_out;
+// *scales and *means ([F][B][T], in the workspace) receive every flow's affine parameters
+int run_student_flows_f32(srwn_ctx* h, float* const* x, const float* enc, int B, int T, int t_out, void* ws, size_t ws_bytes,
+                          const float** scales, const float** means, cudaStream_t st);
+size_t student_f32_workspace_bytes(const srwn_ctx* h, int B, int T);
+int reject_bf16();
+// student_stream.cu: chunked synthesis through a carried flow state (srwn_student_forward_resume)
+constexpr int kAbortStreamPosition = 0x5000000;     // abort code: the call's t0 disagreed with its state's
+int stream_position_fail(const volatile int* e, const char* lead);
+size_t student_stream_workspace_bytes(const srwn_ctx* h, int B, int S, int precision);
+int run_student_stream(srwn_ctx* h, void* state, long long t0, const float* z, NoiseSpec noise, const float* enc, float* out,
+                       float* s_tot, float* mu_tot, float* x_last, float* z_out, int B, int S, int precision, void* ws,
+                       size_t ws_bytes, cudaStream_t st);
 // fused.cu
 namespace fused {
 __global__ void k_fold_bias(const float* __restrict__ cond, const float* __restrict__ front_b,
@@ -216,6 +243,11 @@ int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc,
 int run_student_fused(srwn_ctx* c, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out,
                       float* s_tot, float* mu_tot, float* x_last, int B, int T,
                       void* ws, size_t ws_bytes, cudaStream_t st);
+// the flows of run_student_fused as the stream call runs them: flow f reads x[f] and writes x[f+1] for rows t >= t_out
+// (the work partition starts every utterance at row 0 and its outputs at t_out); noise must be off when t_out > 0
+int run_student_flows_fused(srwn_ctx* c, float* const* x, NoiseSpec noise, const float* enc, int B, int T, int t_out,
+                            void* ws, size_t ws_bytes, const float** scales, const float** means, cudaStream_t st);
 int fused_check_error(void* ws, size_t ws_bytes, const srwn_ctx* c, int B, int T, cudaStream_t st);
+int sticky_error(const srwn_ctx* c);     // SRWN_ERR_CUDA while the handle's abort words are raised (no synchronisation)
 size_t fused_partition_bytes(const srwn_ctx* c);
 void fused_last_partition(const srwn_ctx* c, int* teams, int* G);

@@ -1020,10 +1020,15 @@ struct Partition { std::vector<Seg> segs; std::vector<int> nseg; int teams, G; d
 
 // warm_cost[k] = cost (in full chunks) of the k warm-up chunks nearest the first output row: a warm-up chunk skips the skip
 // GEMM and the head and runs only the layers inside the dependency cone (k_fused: rsuf[l+1] > dist); a fixed part per chunk
-// (front conv, conditioning loads, chunk barrier) plus a part proportional to the layers it runs
-static bool try_partition(int B, int T, int kChunk, const std::vector<double>& warm_cost, int teams, double budget, Partition* out) {
+// (front conv, conditioning loads, chunk barrier) plus a part proportional to the layers it runs.
+// Outputs start at row out0 of each utterance (0 for a one-call launch; the history length of a student stream call, whose
+// rows before out0 are carried inputs): the output rows are cut into chunks counted from out0, an utterance's first piece
+// starts at row 0 and warms up over rows [0, out0), later pieces warm up as usual, clamped at row 0.
+static bool try_partition(int B, int T, int out0, int kChunk, const std::vector<double>& warm_cost, int teams, double budget,
+                          Partition* out) {
   const int warm_chunks = (int)warm_cost.size() - 1;
-  const int NC = (T + kChunk - 1) / kChunk;
+  const int NC = (T - out0 + kChunk - 1) / kChunk;
+  const int lead = std::min(warm_chunks, (out0 + kChunk - 1) / kChunk);   // warm-up of the first piece (cost model only)
   std::vector<Seg> segs((size_t)teams * kMaxSeg);
   std::vector<int> nseg(teams, 0);
   int tm = 0;
@@ -1032,7 +1037,8 @@ static bool try_partition(int B, int T, int kChunk, const std::vector<double>& w
     int c0 = 0;
     while (c0 < NC) {
       if (tm >= teams) return false;
-      const int warm = c0 == 0 ? 0 : std::min(warm_chunks, c0);
+      const int t_out = out0 + c0 * kChunk;
+      const int warm = c0 == 0 ? lead : std::min(warm_chunks, (t_out + kChunk - 1) / kChunk);
       double room = budget - used - warm_cost[warm];
       int take = (int)room;
       if (take < 1 || nseg[tm] >= kMaxSeg) {
@@ -1040,8 +1046,8 @@ static bool try_partition(int B, int T, int kChunk, const std::vector<double>& w
       }
       take = std::min(take, NC - c0);
       Seg s;
-      s.b = b; s.t_start = (c0 - warm) * kChunk; s.t_out = c0 * kChunk;
-      s.t_end = std::min(T, (c0 + take) * kChunk);
+      s.b = b; s.t_start = c0 == 0 ? 0 : std::max(0, t_out - warm * kChunk); s.t_out = t_out;
+      s.t_end = std::min(T, out0 + (c0 + take) * kChunk);
       segs[(size_t)tm * kMaxSeg + nseg[tm]++] = s;
       used += take + warm_cost[warm];
       c0 += take;
@@ -1051,16 +1057,16 @@ static bool try_partition(int B, int T, int kChunk, const std::vector<double>& w
   return true;
 }
 
-static Partition partition_for(int B, int T, int kChunk, const std::vector<double>& warm_cost, int teams) {
+static Partition partition_for(int B, int T, int out0, int kChunk, const std::vector<double>& warm_cost, int teams) {
   const int warm_chunks = (int)warm_cost.size() - 1;
-  const long long total = (long long)B * ((T + kChunk - 1) / kChunk);
+  const long long total = (long long)B * ((T - out0 + kChunk - 1) / kChunk);
   double lo = (double)total / teams, hi = lo + warm_chunks + 2;
   Partition best;
-  while (!try_partition(B, T, kChunk, warm_cost, teams, hi, &best)) hi *= 1.5;
+  while (!try_partition(B, T, out0, kChunk, warm_cost, teams, hi, &best)) hi *= 1.5;
   for (int it = 0; it < 24; it++) {
     const double mid = 0.5 * (lo + hi);
     Partition cand;
-    if (try_partition(B, T, kChunk, warm_cost, teams, mid, &cand)) { hi = mid; best = cand; } else lo = mid;
+    if (try_partition(B, T, out0, kChunk, warm_cost, teams, mid, &cand)) { hi = mid; best = cand; } else lo = mid;
   }
   best.cost = hi;
   return best;
@@ -1072,8 +1078,9 @@ static Partition partition_for(int B, int T, int kChunk, const std::vector<doubl
 // least G lags.  Larger G shares the mid-utterance warm-up between more CTAs; `force_G` > 0 overrides the choice.
 constexpr double kLagLayers = 1.5;
 constexpr int kMaxTeam = 18;
-static Partition make_partition(int B, int T, int kChunk, double handoff_cost, const std::vector<int>& dilations, int grid, int force_G) {
-  const int NC = (T + kChunk - 1) / kChunk;
+static Partition make_partition(int B, int T, int out0, int kChunk, double handoff_cost, const std::vector<int>& dilations, int grid,
+                                int force_G) {
+  const int NC = (T - out0 + kChunk - 1) / kChunk;
   const int L = (int)dilations.size();
   std::vector<int> rsuf(L + 1, 0);
   for (int l = L - 1; l >= 0; l--) rsuf[l] = rsuf[l + 1] + dilations[l];
@@ -1092,7 +1099,7 @@ static Partition make_partition(int B, int T, int kChunk, double handoff_cost, c
     int teams = grid / G;
     if ((long long)teams > total) teams = (int)total;
     if (teams < 1) continue;
-    Partition cand = partition_for(B, T, kChunk, warm_cost, teams);
+    Partition cand = partition_for(B, T, out0, kChunk, warm_cost, teams);
     const double lag = kLagLayers / L;
     const double period = std::max(1.0, G * lag);
     // measured (profiles/r02d_handoff_variants.log, r02e_team_sizes.log): a teacher chunk costs about 10 % more with the
@@ -1162,15 +1169,16 @@ static int launch_fused(srwn_ctx* c, const Params& p, int grid, cudaStream_t st)
 
 // a fused launch that aborted (a bounded wait expired) leaves its error words in pinned host memory; every later call on
 // the handle is refused until srwn_check_async_error has reported it
-static int sticky_error(const srwn_ctx* c) {
+int sticky_error(const srwn_ctx* c) {
   const volatile int* e = c->h_err;
+  if (e && e[0] && e[1] == kAbortStreamPosition) return stream_position_fail(e, "an earlier call aborted");
   if (e && e[0])
     return srwn_fail(SRWN_ERR_CUDA, "an earlier fused launch aborted: pipeline wait timed out (code 0x%x, chunk %d, cta %d); "
                      "results of that call are invalid", e[1], e[2], e[3]);
   return SRWN_OK;
 }
 
-static int prepare(srwn_ctx* c, int stack, const float* enc, int B, int T, const FusedWs& w, Params* p,
+static int prepare(srwn_ctx* c, int stack, const float* enc, int B, int T, int out0, const FusedWs& w, Params* p,
                    int* grid, bool first, cudaStream_t st) {
   const int L = c->cfg.n_layers, P = c->cfg.pool_stride, frames = T / P;
   const float* sw = stack_w(c, stack);
@@ -1190,16 +1198,16 @@ static int prepare(srwn_ctx* c, int stack, const float* enc, int B, int T, const
   }
   (void)sw;
   const size_t seg_bytes = (size_t)c->sm_count * kMaxSeg * sizeof(Seg), n_bytes = (size_t)c->sm_count * sizeof(int);
-  if (first && (c->part_B != B || c->part_T != T || c->part_team_req != c->team_size)) {
-    // the work partition depends on (B, T) and the team size only: built once, kept on the device next to the handle.
+  if (first && (c->part_B != B || c->part_T != T || c->part_out0 != out0 || c->part_team_req != c->team_size)) {
+    // the work partition depends on (B, T, out0) and the team size only: built once, kept on the device next to the handle.
     // The staging vector belongs to the handle (a copy from pageable memory returns once the bytes are staged).
     const bool teacher = c->cfg.kind == SRWN_TEACHER;
-    Partition part = make_partition(B, T, chunk_of(teacher), teacher ? 1.10 : 1.04, c->dilations, c->sm_count, c->team_size);
+    Partition part = make_partition(B, T, out0, chunk_of(teacher), teacher ? 1.10 : 1.04, c->dilations, c->sm_count, c->team_size);
     c->part_host.assign(seg_bytes + n_bytes, 0);
     memcpy(c->part_host.data(), part.segs.data(), std::min(seg_bytes, part.segs.size() * sizeof(Seg)));
     memcpy(c->part_host.data() + seg_bytes, part.nseg.data(), std::min(n_bytes, part.nseg.size() * sizeof(int)));
     SRWN_CUDA(cudaMemcpyAsync(c->d_part, c->part_host.data(), c->part_host.size(), cudaMemcpyHostToDevice, st));
-    c->part_B = B; c->part_T = T; c->part_team_req = c->team_size;
+    c->part_B = B; c->part_T = T; c->part_out0 = out0; c->part_team_req = c->team_size;
     c->part_teams = part.teams; c->part_G = part.G;
   }
   *grid = c->part_teams * c->part_G;
@@ -1232,7 +1240,7 @@ int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc, const fl
   if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
   Params p;
   int grid = 0;
-  int rc = prepare(c, 0, enc, B, T, w, &p, &grid, true, st);
+  int rc = prepare(c, 0, enc, B, T, 0, w, &p, &grid, true, st);
   if (rc) return rc;
   p.x_in = x_in; p.x_scored = x_scored; p.logits_out = logits_out; p.nll_out = nll_out;
   p.nll_partial = (x_scored && nll_sum) ? w.partial : nullptr;
@@ -1248,28 +1256,40 @@ int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc, const fl
   return SRWN_OK;
 }
 
-int run_student_fused(srwn_ctx* c, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out, float* s_tot,
-                      float* mu_tot, float* x_last, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
+int run_student_flows_fused(srwn_ctx* c, float* const* x, NoiseSpec noise, const float* enc, int B, int T, int t_out,
+                            void* ws, size_t ws_bytes, const float** scales, const float** means, cudaStream_t st) {
   if (!fused_supported(c)) return srwn_fail(SRWN_ERR_UNSUPPORTED, "fused 16-bit path needs dilations <= %d, layers <= %d, pool_stride %% 128 == 0", kHalo, kMaxLayers);
   FusedWs w = carve_fused(c, B, T, ws, ws_bytes);
   if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
   const size_t n = (size_t)B * T;
   const int F = c->cfg.num_flows;
-  const float* xin = z;
   int grid = 0;
   for (int f = 0; f < F; f++) {                     // model.py:509-513: flows are strictly sequential
     Params p;
-    int rc = prepare(c, f, enc, B, T, w, &p, &grid, f == 0, st);
+    int rc = prepare(c, f, enc, B, T, t_out, w, &p, &grid, f == 0, st);
     if (rc) return rc;
-    float* xout = (f == F - 1 && x_last) ? x_last : ((f & 1) ? w.xb : w.xa);
-    p.x_in = xin; p.scale_out = w.scales + (size_t)f * n; p.mean_out = w.means + (size_t)f * n; p.x_out = xout;
+    p.x_in = x[f]; p.scale_out = w.scales + (size_t)f * n; p.mean_out = w.means + (size_t)f * n; p.x_out = x[f + 1];
     if (f == 0) p.noise = noise;                    // later flows read the previous flow's output
     ProfScope prof(c, st, "k_fused<student,fp16>", 1);
     rc = launch_fused<false>(c, p, grid, st);
     if (rc) return rc;
-    xin = xout;
   }
-  return run_flow_compose(z, noise, z_out, w.scales, w.means, F, out, s_tot, mu_tot, (int64_t)n, st);
+  *scales = w.scales; *means = w.means;
+  return SRWN_OK;
+}
+
+int run_student_fused(srwn_ctx* c, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out, float* s_tot,
+                      float* mu_tot, float* x_last, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
+  if (!fused_supported(c)) return srwn_fail(SRWN_ERR_UNSUPPORTED, "fused 16-bit path needs dilations <= %d, layers <= %d, pool_stride %% 128 == 0", kHalo, kMaxLayers);
+  FusedWs w = carve_fused(c, B, T, ws, ws_bytes);
+  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  const int F = c->cfg.num_flows;
+  float* x[17] = {const_cast<float*>(z)};          // flow f reads x[f] and writes x[f + 1] (num_flows <= 16, srwn_create)
+  for (int f = 0; f < F; f++) x[f + 1] = (f == F - 1 && x_last) ? x_last : ((f & 1) ? w.xb : w.xa);
+  const float *scales = nullptr, *means = nullptr;
+  int rc = run_student_flows_fused(c, x, noise, enc, B, T, 0, ws, ws_bytes, &scales, &means, st);
+  if (rc) return rc;
+  return run_flow_compose(z, noise, z_out, scales, means, F, out, s_tot, mu_tot, (int64_t)B * T, st);
 }
 
 // reads (and clears) the abort words of the fused launches issued so far; synchronises the stream
@@ -1277,6 +1297,11 @@ int fused_check_error(void* ws, size_t ws_bytes, const srwn_ctx* c, int B, int T
   (void)ws; (void)ws_bytes; (void)B; (void)T;
   SRWN_CUDA(cudaStreamSynchronize(st));
   volatile int* e = c->h_err;
+  if (e && e[0] && e[1] == kAbortStreamPosition) {
+    const int rc = stream_position_fail(e, "student stream call aborted");
+    e[0] = 0; e[1] = 0; e[2] = 0; e[3] = 0;
+    return rc;
+  }
   if (e && e[0]) {
     const int code = e[1], chunk = e[2], cta = e[3];
     e[0] = 0; e[1] = 0; e[2] = 0; e[3] = 0;

@@ -28,8 +28,9 @@ void state_signature(const srwn_ctx* c, int B, int precision, int32_t* sig) {
 }
 
 // The signature is also kept on the host, per state buffer, so that a call can refuse a state made for another handle,
-// batch size or precision without reading the device copy (which would synchronise the stream).
-struct StateOwner { const srwn_ctx* h; int32_t sig[6]; };
+// batch size or precision without reading the device copy (which would synchronise the stream).  Generation states and
+// the student's synthesis states (student_stream.cu) share the registry; their signatures differ in length and magic.
+struct StateOwner { const srwn_ctx* h; std::vector<int32_t> sig; };
 std::mutex g_states_mu;
 std::map<const void*, StateOwner> g_states;
 
@@ -44,23 +45,11 @@ int check_state_args(const srwn_ctx* h, int B, int precision, const char* fn) {
   return SRWN_OK;
 }
 
-// Refuses a state that was not last reset on this handle for this B and precision (host-side signature: no synchronisation).
-int check_state_owner(const srwn_ctx* h, const void* state, int B, int precision) {
-  int32_t sig[6];
-  state_signature(h, B, precision, sig);
-  std::lock_guard<std::mutex> lk(g_states_mu);
-  auto it = g_states.find(state);
-  if (it == g_states.end() || it->second.h != h)
-    return srwn_fail(SRWN_ERR_INVALID, "state was not reset on this handle (srwn_generate_state_reset)");
-  if (memcmp(it->second.sig, sig, sizeof(sig)))
-    return srwn_fail(SRWN_ERR_INVALID, "state was made for B=%d, precision %d; this call has B=%d, precision %d",
-                     it->second.sig[0], it->second.sig[1], B, precision);
-  return SRWN_OK;
-}
-
 // The owner check, then the state's parts (the layout of B utterances in `precision`).
 int open_owned(const srwn_ctx* h, void* state, int B, int precision, GenState* s) {
-  const int rc = check_state_owner(h, state, B, precision);
+  int32_t sig[6];
+  state_signature(h, B, precision, sig);
+  const int rc = state_owner_check(h, state, sig, 6, "srwn_generate_state_reset");
   if (rc) return rc;
   uint8_t* base = static_cast<uint8_t*>(state);
   const GenStateLayout lay = gen_state_layout(h, B, precision);
@@ -70,6 +59,26 @@ int open_owned(const srwn_ctx* h, void* state, int B, int precision, GenState* s
   return SRWN_OK;
 }
 }  // namespace
+
+void state_owner_record(const srwn_ctx* h, const void* state, const int32_t* sig, int n) {
+  std::lock_guard<std::mutex> lk(g_states_mu);
+  StateOwner& o = g_states[state];
+  o.h = h;
+  o.sig.assign(sig, sig + n);
+}
+
+// Refuses a state that was not last reset on this handle with this signature (B and precision first).
+int state_owner_check(const srwn_ctx* h, const void* state, const int32_t* sig, int n, const char* reset_fn) {
+  std::lock_guard<std::mutex> lk(g_states_mu);
+  auto it = g_states.find(state);
+  if (it == g_states.end() || it->second.h != h)
+    return srwn_fail(SRWN_ERR_INVALID, "state was not reset on this handle (%s)", reset_fn);
+  const std::vector<int32_t>& have = it->second.sig;
+  if (have.size() != (size_t)n || memcmp(have.data(), sig, n * sizeof(int32_t)))
+    return srwn_fail(SRWN_ERR_INVALID, "state was made for B=%d, precision %d; this call has B=%d, precision %d",
+                     have.empty() ? 0 : have[0], have.size() < 2 ? 0 : have[1], sig[0], sig[1]);
+  return SRWN_OK;
+}
 
 // dilation queues of B utterances: fp32, sum_d rows of R floats each; fp16, one block of sum_d slots per group
 size_t gen_queue_bytes(const srwn_ctx* c, int B, int precision) {
@@ -109,10 +118,7 @@ extern "C" int srwn_generate_state_reset(srwn_handle_t h, void* state, int32_t B
   SRWN_CUDA(cudaMemsetAsync(base, 0, gen_state_layout(h, B, precision).bytes, st));      // zero padding of ops.py:9
   // pageable source: the copy is staged before this call returns, so `hdr` may go out of scope
   SRWN_CUDA(cudaMemcpyAsync(base, &hdr, sizeof(hdr), cudaMemcpyHostToDevice, st));
-  std::lock_guard<std::mutex> lk(g_states_mu);
-  StateOwner& o = g_states[state];
-  o.h = h;
-  memcpy(o.sig, hdr.sig, sizeof(hdr.sig));
+  state_owner_record(h, state, hdr.sig, 6);
   return SRWN_OK;
 }
 

@@ -23,7 +23,10 @@ size_t gen_queue_bytes(const srwn_ctx* c, int B, int precision);
 // Checks the arguments of a call on `state` (the C entry points' order: handle, B, precision, then check_bt(B, T)), then
 // that the state was last reset on h for B and precision, without touching the device; fills *s with the state's parts.
 int gen_state_open(const srwn_ctx* h, void* state, int B, int T, int precision, GenState* s);
-void gen_state_forget(const srwn_ctx* h);    // srwn_destroy: h's states are no longer valid
+void gen_state_forget(const srwn_ctx* h);    // srwn_destroy: h's states (generation and synthesis) are no longer valid
+// host registry of state owners: the handle and signature a state buffer was last reset with
+void state_owner_record(const srwn_ctx* h, const void* state, const int32_t* sig, int n);
+int state_owner_check(const srwn_ctx* h, const void* state, const int32_t* sig, int n, const char* reset_fn);
 int run_gen_state_advance(long long* t0, int T, cudaStream_t st);
 
 // fp32 queues: row of layer l (queue offset qoff), slot `slot`, utterance b

@@ -394,7 +394,7 @@ int run_teacher_head_f32(srwn_ctx* c, const float* skip, float* logits, int B, i
 __global__ void k_flow_head(const float* __restrict__ h, const float* __restrict__ xin,
                             const float* __restrict__ hk, const float* __restrict__ hb,
                             float* __restrict__ scale, float* __restrict__ mean,
-                            float* __restrict__ xout, int64_t n) {
+                            float* __restrict__ xout, int64_t n, int T, int t_out) {
   const int64_t gid = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   const int64_t row = gid >> 3;          // 8 lanes per time step
   const int q = (int)(gid & 7);
@@ -417,22 +417,21 @@ __global__ void k_flow_head(const float* __restrict__ h, const float* __restrict
     const float sc = expf(p0 + hb[0]);       // no clamp on the log-scale (model.py:479)
     const float mu = p1 + hb[1];
     scale[row] = sc; mean[row] = mu;
-    xout[row] = fmaf(xin[row], sc, mu);      // model.py:482
+    if (t_out == 0 || row % T >= t_out) xout[row] = fmaf(xin[row], sc, mu);      // model.py:482
   }
 }
 
 int run_flow_head_f32(srwn_ctx* c, int stack, const float* h, const float* xin, float* scale,
-                      float* mean, float* xout, int B, int T, cudaStream_t st) {
+                      float* mean, float* xout, int B, int T, cudaStream_t st, int t_out) {
   const float* w = stack_w(c, stack);
   const int64_t n = (int64_t)B * T;
   k_flow_head<<<(unsigned)((n * 8 + 255) / 256), 256, 0, st>>>(h, xin, w + c->off.head1_k,
-                                                               w + c->off.head1_b, scale, mean, xout, n);
+                                                               w + c->off.head1_b, scale, mean, xout, n, T, t_out);
   SRWN_LAUNCH_CHECK();
   return SRWN_OK;
 }
 
-// s_tot = prod s_f; mu_tot = sum_f mu_f * prod_{j>f} s_j in the reference's loop order
-// (model.py:517-533); out = clip(z*s_tot + mu_tot, -1, 1) (model.py:535)
+// s_tot, mu_tot (flow_compose_at); out = clip(z*s_tot + mu_tot, -1, 1) (model.py:535)
 __global__ void k_flow_compose(const float* __restrict__ z, NoiseSpec noise, float* __restrict__ z_out,
                                const float* __restrict__ scales,
                                const float* __restrict__ means, int F, float* __restrict__ out,
@@ -442,13 +441,8 @@ __global__ void k_flow_compose(const float* __restrict__ z, NoiseSpec noise, flo
   // the student's input noise (student.py:104): supplied, or the same Philox draw the flow kernel evaluated
   const float zi = noise.on ? philox::logistic_at(noise.seed, noise.stream, (uint64_t)i) : z[i];
   if (z_out) z_out[i] = zi;
-  float st = 1.f, mt = 0.f;
-  for (int f = 0; f < F; f++) {
-    st *= scales[(size_t)f * n + i];
-    float mu = means[(size_t)f * n + i];
-    for (int j = f + 1; j < F; j++) mu *= scales[(size_t)j * n + i];
-    mt += mu;
-  }
+  float st, mt;
+  flow_compose_at(scales, means, F, n, i, st, mt);
   if (s_tot) s_tot[i] = st;
   if (mu_tot) mu_tot[i] = mt;
   out[i] = fminf(fmaxf(fmaf(zi, st, mt), -1.f), 1.f);

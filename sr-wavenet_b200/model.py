@@ -180,7 +180,7 @@ class _Engine(_Handle):
         Device-resident results are not synchronised; an abort then refuses the NEXT call on the handle (pinned abort
         words, include/srwn.h)."""
         out = self.to_host(t, on_dev)
-        if not on_dev and precision != _lib.FP32:
+        if not on_dev and (precision != _lib.FP32 or op == _lib.OP_STUDENT_STREAM):    # a stream call checks its t0 in both
             self.check_async(op, B, T, precision)
         return out
 
@@ -852,6 +852,34 @@ class GenerationState(object):
         return self.buffer.data_ptr()
 
 
+class SynthesisState(object):
+    """Device buffer that carries the student's flows from one ``generate`` call to the next: per flow the last H inputs,
+    the last H / pool_stride frames and the position (include/srwn.h, srwn_student_state_*).  Created reset.  The host
+    keeps its own copy of the position, which each call passes to the library (it sets the call's shape)."""
+
+    def __init__(self, eng, batch_size, precision="fp16"):
+        self._eng = eng
+        self.batch_size, self.precision = int(batch_size), precision
+        self._prec = _lib.PRECISIONS[precision]
+        n = ctypes.c_size_t()
+        _lib.check(eng.lib.srwn_student_state_bytes(eng.h, self.batch_size, self._prec, ctypes.byref(n)))
+        self.buffer = torch.empty(n.value, dtype=torch.uint8, device="cuda")
+        self.reset()
+
+    def reset(self):
+        """Back to the start of an utterance: position 0, silence before it."""
+        _lib.check(self._eng.lib.srwn_student_state_reset(self._eng.h, self.buffer.data_ptr(), self.batch_size,
+                                                          self._prec, _stream()))
+        self._t0 = 0
+
+    def position(self):
+        """Samples synthesized through this state since the last reset (reads the device header: synchronises)."""
+        return int(self.buffer[:8].view(torch.int64).item())
+
+    def data_ptr(self):
+        return self.buffer.data_ptr()
+
+
 class ParallelWaveNet(_Model):
     """model.py:290-656.  ``teacher`` is a checkpoint directory in the reference; here it may also
     be a ``WaveNetAutoEncoder`` instance or None.  Methods keep the explicit ``sess`` first argument
@@ -947,8 +975,17 @@ class ParallelWaveNet(_Model):
     def save(self, sess, logdir, global_step, force=False):
         return self._save(logdir, global_step, force)
 
-    def _forward(self, inputs, encoding, conditions, precision=None, want=("out",)):
+    def synthesis_state(self, batch_size, precision="fp16"):
+        """A fresh (reset) state for synthesizing ``batch_size`` utterances in chunks: pass it to ``generate(state=...)``
+        or ``forward_all(state=...)`` to continue the previous call on it."""
+        return SynthesisState(self._eng, batch_size, precision)
+
+    def _forward(self, inputs, encoding, conditions, precision=None, want=("out",), state=None):
         eng = self._eng
+        if state is not None:
+            if not isinstance(state, SynthesisState) or state._eng is not eng:
+                raise ValueError("state must come from this model's synthesis_state()")
+            precision = precision or state.precision
         enc = _with_conditions(encoding, conditions, self.condition_size)
         e, on_dev = eng.to_device(enc, "enc")
         if inputs is None:          # student.py:104 / :172 draws the logistic noise on the host; here it is drawn on the device
@@ -959,12 +996,25 @@ class ParallelWaveNet(_Model):
             B, T = z.shape
         eng.check_encoding(e, B, T)
         prec = _lib.PRECISIONS[precision or self.precision]
+        if state is not None and (state.batch_size != B or state.precision != precision):
+            raise ValueError("state was made for batch_size=%d, precision=%r; this call has %d, %r"
+                             % (state.batch_size, state.precision, B, precision))
         if prec != _lib.FP32 and getattr(self, "_packed_stale", False):
             self.sync_weights()
-        ws, wsn = eng.workspace(_lib.OP_STUDENT_FORWARD, B, T, prec)
+        op = _lib.OP_STUDENT_FORWARD if state is None else _lib.OP_STUDENT_STREAM
+        ws, wsn = eng.workspace(op, B, T, prec)
         bufs = {k: torch.empty(B, T, dtype=torch.float32, device="cuda") for k in set(want) | {"out"}}
         g = lambda k: bufs[k].data_ptr() if k in bufs else None
-        if z is None:
+        if state is not None:               # this call's T samples continue the state (device noise: a new Philox stream)
+            if z is None:
+                self._noise_calls += 1
+            _lib.check(eng.lib.srwn_student_forward_resume(eng.h, state.data_ptr(), state._t0,
+                                                           None if z is None else z.data_ptr(), self.seed,
+                                                           self._noise_calls, e.data_ptr(), g("out"), g("s_tot"),
+                                                           g("mu_tot"), g("x_last"), g("z"), B, T, prec, ws, wsn,
+                                                           _stream()))
+            state._t0 += T
+        elif z is None:
             self._noise_calls += 1
             _lib.check(eng.lib.srwn_student_sample(eng.h, self.seed, self._noise_calls, e.data_ptr(), g("out"), g("s_tot"),
                                                    g("mu_tot"), g("x_last"), g("z"), B, T, prec, ws, wsn, _stream()))
@@ -972,19 +1022,25 @@ class ParallelWaveNet(_Model):
             bufs.pop("z", None)
             _lib.check(eng.lib.srwn_student_forward(eng.h, z.data_ptr(), e.data_ptr(), g("out"), g("s_tot"),
                                                     g("mu_tot"), g("x_last"), B, T, prec, ws, wsn, _stream()))
-        return bufs, (on_dev, _lib.OP_STUDENT_FORWARD, B, T, prec)
+        return bufs, (on_dev, op, B, T, prec)
 
-    def generate(self, sess, inputs, encoding, conditions=None, precision=None):
+    def generate(self, sess, inputs, encoding, conditions=None, precision=None, state=None):
         """model.py:570-576 -> out [B,T,1] = clip(z*s_tot + mu_tot, -1, 1).  ``inputs=None`` draws the logistic noise of
-        student.py:172 on the device (inside the fused flow kernel on the fp16 path): nothing but the encoding is uploaded."""
-        bufs, call = self._forward(inputs, encoding, conditions, precision)
+        student.py:172 on the device (inside the fused flow kernel on the fp16 path): nothing but the encoding is uploaded.
+
+        ``state`` (from ``synthesis_state``): these T samples (a multiple of pool_stride) continue the clip where the last
+        call on that state stopped, and the state advances by T; ``inputs`` and ``encoding`` then cover this call's
+        samples only and the precision defaults to the state's.  With injected noise, any split of a clip into such calls
+        gives bit for bit the audio of one call; noise drawn on the device comes from a new Philox stream per call
+        (``forward_all`` returns it as ``z``)."""
+        bufs, call = self._forward(inputs, encoding, conditions, precision, state=state)
         return self._eng.finish(bufs["out"][:, :, None], *call)
 
-    def forward_all(self, inputs, encoding, conditions=None, precision=None):
+    def forward_all(self, inputs, encoding, conditions=None, precision=None, state=None):
         """out, s_tot, mu_tot (model.py:517-535) and the chained flow output, each [B,T]; with ``inputs=None`` also the
-        noise ``z`` that was drawn."""
+        noise ``z`` that was drawn.  ``state``: as in ``generate``."""
         want = ("out", "s_tot", "mu_tot", "x_last") + (("z",) if inputs is None else ())
-        bufs, call = self._forward(inputs, encoding, conditions, precision, want=want)
+        bufs, call = self._forward(inputs, encoding, conditions, precision, want=want, state=state)
         return {k: self._eng.finish(v, *call) for k, v in bufs.items()}
 
     def _entropies(self, inputs, encoding, conditions):

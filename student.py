@@ -45,7 +45,19 @@ def build_parser():
     p.add_argument('--clips', type=int, default=20, help='--test: number of clips')
     p.add_argument('--precision', type=str, default='fp16', choices=['fp32', 'fp16'])
     p.add_argument('--seed', type=int, default=None, help='seed of the host-side logistic noise (student.py:104 leaves it unseeded)')
+    p.add_argument('--chunk', type=int, default=0,
+                   help='--test: synthesize each clip in calls of S samples (a multiple of --pool-stride) through one '
+                        'synthesis state; the same audio as one call')
     return p
+
+
+def generate_chunked(student, noise, encoding, precision, chunk, pool_stride):
+    """--test --chunk: the clip in calls of `chunk` samples through one synthesis state: the same audio as one call."""
+    B, T = noise.shape
+    state = student.synthesis_state(B, precision)
+    parts = [student.generate(None, noise[:, a:a + chunk], encoding[:, a // pool_stride:(a + chunk) // pool_stride], None,
+                              state=state) for a in range(0, T, chunk)]
+    return np.concatenate(parts, axis=1)
 
 
 def main(argv=None):
@@ -54,6 +66,8 @@ def main(argv=None):
     from sr_wavenet_b200.audio_data import AudioReader, write_wav
 
     num_samples, batch = args.num_samples, args.batch_size
+    if args.chunk < 0 or args.chunk % args.pool_stride:
+        raise SystemExit('--chunk %d must be a multiple of --pool-stride %d' % (args.chunk, args.pool_stride))
     audio_data = AudioReader(args.data, batch, num_samples, audio_max_length=args.audio_max_length)
     teacher = args.teacher
     if teacher is None or not os.path.exists(os.path.join(teacher, 'checkpoint')):
@@ -98,7 +112,10 @@ def main(argv=None):
             regen = student.reconstruct(None, x, None, precision=args.precision)
             noise = rng.logistic(0, 1, x.shape).astype(np.float32)
             entropy = student.getEntropy(None, noise, encoding, None)
-            output = student.generate(None, noise, encoding, None, precision=args.precision)
+            if args.chunk:
+                output = generate_chunked(student, noise, encoding, args.precision, args.chunk, args.pool_stride)
+            else:
+                output = student.generate(None, noise, encoding, None, precision=args.precision)
             print('Entropy', entropy)
             write_wav(os.path.join(args.out_dir, 'test_wav_%d.wav' % step), args.sample_rate, x[0])
             write_wav(os.path.join(args.out_dir, 'regen_wav_%d.wav' % step), args.sample_rate, regen[0])
