@@ -121,7 +121,9 @@ int srwn_peek_async_error(srwn_handle_t h);
  * has been called, so a caller that keeps its results on the device cannot consume them unnoticed for long. */
 /* Fused tensor-core kernel: CTAs per team (teams walk contiguous pieces of the (utterance, chunk) line as a wavefront
  * over chunks and layers, handing the per-layer history rings from CTA to CTA).  0 (default) = chosen per (B, T).
- * Results do not depend on it.  srwn_last_partition reports the choice of the last fused call. */
+ * Results do not depend on it.  A team holds at most 8 utterances, so a size that leaves fewer than B / 8 teams
+ * (SM count / size) is lowered to the largest that does not.  srwn_last_partition reports the choice of the last fused
+ * call. */
 int srwn_set_team_size(srwn_handle_t h, int32_t ctas_per_team);
 /* How many SM clocks a pipeline wait inside the fused kernel may spin before the launch aborts (default 1e9, about half a
  * second; every wait is bounded so that a lost signal surfaces as SRWN_ERR_CUDA instead of a hung GPU). */
@@ -133,6 +135,9 @@ int srwn_workspace_bytes(srwn_handle_t h, int32_t op, int32_t B, int32_t T,
                          int32_t precision, size_t* bytes);
 
 /* ---- teacher (model.py:158-200) ------------------------------------------------- */
+/* Batch limit of the 16-bit path: an SRWN_FP16 call of srwn_teacher_logits or srwn_teacher_nll takes at most 8 utterances
+ * per SM (B <= 1184 on 148 SMs); a larger B is refused with SRWN_ERR_UNSUPPORTED before any launch (split the batch over
+ * calls, or use SRWN_FP32).  srwn_teacher_generate has no such limit. */
 /* get_logits(inputs, encoding) (model.py:279-285): x [B,T] teacher-forcing audio,
  * enc [B,T/P,C] -> logits [B,T,4M]. */
 int srwn_teacher_logits(srwn_handle_t h, const float* x, const float* enc, float* logits,
@@ -204,6 +209,9 @@ int srwn_generate_state_splice(srwn_handle_t h, void* dst, int32_t dst_B, const 
                                int32_t precision, void* stream);
 
 /* ---- student (model.py:415-535) ------------------------------------------------- */
+/* Batch limit of the 16-bit path: an SRWN_FP16 call of srwn_student_forward, srwn_student_sample or
+ * srwn_student_forward_resume takes at most 8 utterances per SM (B <= 1184 on 148 SMs); a larger B is refused with
+ * SRWN_ERR_UNSUPPORTED before any launch (split the batch over calls, or use SRWN_FP32). */
 /* generate(sess, inputs, encoding) (model.py:570-576): z [B,T] logistic noise ->
  * out [B,T] = clip(z*s_tot + mu_tot, -1, 1) (model.py:535); s_tot, mu_tot [B,T]
  * (model.py:517-533) and x_last [B,T] (chained flow output) are optional outputs. */

@@ -233,6 +233,7 @@ __global__ void k_fold_bias(const float* __restrict__ cond, const float* __restr
                             const float* __restrict__ res_b, float* __restrict__ cb, int L);
 }
 bool fused_supported(const srwn_ctx* c);
+int fused_check_batch(const srwn_ctx* c, int B);   // SRWN_ERR_UNSUPPORTED past sm_count * 8 utterances (srwn.h)
 size_t fused_packed_bytes(const srwn_ctx* c);
 int fused_pack_weights(srwn_ctx* c, cudaStream_t st);
 size_t fused_workspace_bytes(const srwn_ctx* c, int op, int B, int T);

@@ -30,6 +30,7 @@
 #include "mol.cuh"
 #include "umma.cuh"
 #include "philox.cuh"
+#include "partition.h"
 #include <cuda_fp16.h>
 #include <algorithm>
 #include <cstdlib>
@@ -45,7 +46,6 @@ __host__ __device__ constexpr int tiles_of(bool teacher) { return teacher ? 3 : 
 __host__ __device__ constexpr int chunk_of(bool teacher) { return kTile * tiles_of(teacher); }     // time steps per chunk
 constexpr int kHalo = 512;                      // largest dilation the layout supports
 constexpr int kMaxLayers = 40;
-constexpr int kMaxSeg = 8;
 
 // packed operand image (bytes, per layer): WF [8 kc][32 n][8] | WRS [4 kc][160 or 32 n][8]
 constexpr int kWfBytes = 64 * 32 * 2;           // 4096
@@ -53,8 +53,6 @@ constexpr int kWrsTeacher = 32 * 160 * 2;       // 10240
 constexpr int kWrsStudent = 32 * 32 * 2;        // 2048
 constexpr int kH1Bytes = 128 * 128 * 2;         // 32768
 constexpr int kH2Bytes = 128 * 32 * 2;          // 8192
-
-struct Seg { int b, t_start, t_out, t_end; };
 
 struct Params {
   const uint8_t* packed;      // per-stack packed image
@@ -950,6 +948,14 @@ bool fused_supported(const srwn_ctx* c) {
   return true;
 }
 
+// one fused launch gives every utterance a segment of its own: at most sm_count teams of kMaxSeg segments (partition.h)
+int fused_check_batch(const srwn_ctx* c, int B) {
+  if (B > fused_max_batch(c->sm_count))
+    return srwn_fail(SRWN_ERR_UNSUPPORTED, "the fused 16-bit kernel takes at most %lld utterances per call (%d per SM on %d SMs), "
+                     "got B = %d", fused_max_batch(c->sm_count), kMaxSeg, c->sm_count, B);
+  return SRWN_OK;
+}
+
 size_t fused_packed_bytes(const srwn_ctx* c) {
   return fused_supported(c) ? (size_t)c->n_stacks * stack_image_bytes(c) : 0;
 }
@@ -1013,102 +1019,6 @@ int fused_pack_weights(srwn_ctx* c, cudaStream_t st) {
   SRWN_CUDA(cudaMemcpyAsync(c->d_packed, host.data(), host.size(), cudaMemcpyHostToDevice, st));
   SRWN_CUDA(cudaStreamSynchronize(st));
   return SRWN_OK;
-}
-
-// ---- work partition: equal-cost contiguous pieces of the (utterance, chunk) line, one per team of G CTAs ---------
-struct Partition { std::vector<Seg> segs; std::vector<int> nseg; int teams, G; double cost; };
-
-// warm_cost[k] = cost (in full chunks) of the k warm-up chunks nearest the first output row: a warm-up chunk skips the skip
-// GEMM and the head and runs only the layers inside the dependency cone (k_fused: rsuf[l+1] > dist); a fixed part per chunk
-// (front conv, conditioning loads, chunk barrier) plus a part proportional to the layers it runs.
-// Outputs start at row out0 of each utterance (0 for a one-call launch; the history length of a student stream call, whose
-// rows before out0 are carried inputs): the output rows are cut into chunks counted from out0, an utterance's first piece
-// starts at row 0 and warms up over rows [0, out0), later pieces warm up as usual, clamped at row 0.
-static bool try_partition(int B, int T, int out0, int kChunk, const std::vector<double>& warm_cost, int teams, double budget,
-                          Partition* out) {
-  const int warm_chunks = (int)warm_cost.size() - 1;
-  const int NC = (T - out0 + kChunk - 1) / kChunk;
-  const int lead = std::min(warm_chunks, (out0 + kChunk - 1) / kChunk);   // warm-up of the first piece (cost model only)
-  std::vector<Seg> segs((size_t)teams * kMaxSeg);
-  std::vector<int> nseg(teams, 0);
-  int tm = 0;
-  double used = 0;
-  for (int b = 0; b < B; b++) {
-    int c0 = 0;
-    while (c0 < NC) {
-      if (tm >= teams) return false;
-      const int t_out = out0 + c0 * kChunk;
-      const int warm = c0 == 0 ? lead : std::min(warm_chunks, (t_out + kChunk - 1) / kChunk);
-      double room = budget - used - warm_cost[warm];
-      int take = (int)room;
-      if (take < 1 || nseg[tm] >= kMaxSeg) {
-        if (used == 0 && nseg[tm] < kMaxSeg) take = 1; else { tm++; used = 0; continue; }
-      }
-      take = std::min(take, NC - c0);
-      Seg s;
-      s.b = b; s.t_start = c0 == 0 ? 0 : std::max(0, t_out - warm * kChunk); s.t_out = t_out;
-      s.t_end = std::min(T, out0 + (c0 + take) * kChunk);
-      segs[(size_t)tm * kMaxSeg + nseg[tm]++] = s;
-      used += take + warm_cost[warm];
-      c0 += take;
-    }
-  }
-  if (out) { out->segs.swap(segs); out->nseg.swap(nseg); out->teams = teams; }
-  return true;
-}
-
-static Partition partition_for(int B, int T, int out0, int kChunk, const std::vector<double>& warm_cost, int teams) {
-  const int warm_chunks = (int)warm_cost.size() - 1;
-  const long long total = (long long)B * ((T - out0 + kChunk - 1) / kChunk);
-  double lo = (double)total / teams, hi = lo + warm_chunks + 2;
-  Partition best;
-  while (!try_partition(B, T, out0, kChunk, warm_cost, teams, hi, &best)) hi *= 1.5;
-  for (int it = 0; it < 24; it++) {
-    const double mid = 0.5 * (lo + hi);
-    Partition cand;
-    if (try_partition(B, T, out0, kChunk, warm_cost, teams, mid, &cand)) { hi = mid; best = cand; } else lo = mid;
-  }
-  best.cost = hi;
-  return best;
-}
-
-// Team size: a team of G CTAs walks its piece as a wavefront, member j+1 about `kLagLayers` layers behind member j, so
-// (a) a piece costs (chunks + warm-up) / G per member, (b) the wavefront fills and drains over (G-1) lags, (c) member 0
-// can only start its next chunk when member G-1 is through the same layer of the previous one: a chunk period is at
-// least G lags.  Larger G shares the mid-utterance warm-up between more CTAs; `force_G` > 0 overrides the choice.
-constexpr double kLagLayers = 1.5;
-constexpr int kMaxTeam = 18;
-static Partition make_partition(int B, int T, int out0, int kChunk, double handoff_cost, const std::vector<int>& dilations, int grid,
-                                int force_G) {
-  const int NC = (T - out0 + kChunk - 1) / kChunk;
-  const int L = (int)dilations.size();
-  std::vector<int> rsuf(L + 1, 0);
-  for (int l = L - 1; l >= 0; l--) rsuf[l] = rsuf[l + 1] + dilations[l];
-  const int warm_chunks = (rsuf[0] + kChunk - 1) / kChunk;
-  std::vector<double> warm_cost(warm_chunks + 1, 0.0);
-  for (int k = 0; k < warm_chunks; k++) {                      // chunk k ends k * kChunk rows before the first output row
-    int lc = 0;
-    while (lc < L && rsuf[lc + 1] > k * kChunk) lc++;
-    warm_cost[k + 1] = warm_cost[k] + 0.1 + 0.9 * std::max(lc, 1) / (double)L;    // measured: flat optimum around (0.1, 0.9) .. (0, 1)
-  }
-  const long long total = (long long)B * NC;
-  Partition best;
-  double best_time = 1e300;
-  for (int G = 1; G <= std::min(kMaxTeam, grid); G++) {
-    if (force_G > 0 && G != std::min(force_G, std::min(kMaxTeam, grid))) continue;
-    int teams = grid / G;
-    if ((long long)teams > total) teams = (int)total;
-    if (teams < 1) continue;
-    Partition cand = partition_for(B, T, out0, kChunk, warm_cost, teams);
-    const double lag = kLagLayers / L;
-    const double period = std::max(1.0, G * lag);
-    // measured (profiles/r02d_handoff_variants.log, r02e_team_sizes.log): a teacher chunk costs about 10 % more with the
-    // hand-off (flag waits of the loader, row counting) than without; a student chunk about 4 % since its weight stage is
-    // released by a plain arrive (32x64000: 1.825 ms with one CTA per piece, 1.725 ms with teams of 4)
-    const double time = (cand.cost / G + (G > 1 ? 0.5 : 0.0)) * period * (G > 1 ? handoff_cost : 1.0) + (G - 1) * lag;
-    if (time < best_time) { best_time = time; best = cand; best.G = G; }
-  }
-  return best;
 }
 
 struct FusedWs {
@@ -1203,6 +1113,7 @@ static int prepare(srwn_ctx* c, int stack, const float* enc, int B, int T, int o
     // The staging vector belongs to the handle (a copy from pageable memory returns once the bytes are staged).
     const bool teacher = c->cfg.kind == SRWN_TEACHER;
     Partition part = make_partition(B, T, out0, chunk_of(teacher), teacher ? 1.10 : 1.04, c->dilations, c->sm_count, c->team_size);
+    if (part.teams == 0) return srwn_fail(SRWN_ERR_UNSUPPORTED, "no work partition holds B = %d utterances", B);   // fused_check_batch
     c->part_host.assign(seg_bytes + n_bytes, 0);
     memcpy(c->part_host.data(), part.segs.data(), std::min(seg_bytes, part.segs.size() * sizeof(Seg)));
     memcpy(c->part_host.data() + seg_bytes, part.nseg.data(), std::min(n_bytes, part.nseg.size() * sizeof(int)));
@@ -1236,6 +1147,7 @@ int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc, const fl
                       float* nll_out, float* nll_sum, float* logits_out, int B, int T,
                       void* ws, size_t ws_bytes, cudaStream_t st) {
   if (!fused_supported(c)) return srwn_fail(SRWN_ERR_UNSUPPORTED, "fused 16-bit path needs dilations <= %d, layers <= %d, pool_stride %% 128 == 0", kHalo, kMaxLayers);
+  if (int rc = fused_check_batch(c, B)) return rc;
   FusedWs w = carve_fused(c, B, T, ws, ws_bytes);
   if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
   Params p;
@@ -1259,6 +1171,7 @@ int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc, const fl
 int run_student_flows_fused(srwn_ctx* c, float* const* x, NoiseSpec noise, const float* enc, int B, int T, int t_out,
                             void* ws, size_t ws_bytes, const float** scales, const float** means, cudaStream_t st) {
   if (!fused_supported(c)) return srwn_fail(SRWN_ERR_UNSUPPORTED, "fused 16-bit path needs dilations <= %d, layers <= %d, pool_stride %% 128 == 0", kHalo, kMaxLayers);
+  if (int rc = fused_check_batch(c, B)) return rc;
   FusedWs w = carve_fused(c, B, T, ws, ws_bytes);
   if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
   const size_t n = (size_t)B * T;

@@ -204,6 +204,7 @@ int run_student_stream(srwn_ctx* h, void* state, long long t0, const float* z, N
                        size_t ws_bytes, cudaStream_t st) {
   int rc = check_state_args(h, B, precision, "srwn_student_forward_resume");
   if (rc) return rc;
+  if (precision == SRWN_FP16 && (rc = fused_check_batch(h, B))) return rc;
   int32_t sig[kSigLen];
   signature(h, B, precision, sig);
   rc = state_owner_check(h, state, sig, kSigLen, "srwn_student_state_reset");
