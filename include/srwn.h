@@ -129,8 +129,22 @@ int srwn_set_team_size(srwn_handle_t h, int32_t ctas_per_team);
  * second; every wait is bounded so that a lost signal surfaces as SRWN_ERR_CUDA instead of a hung GPU). */
 int srwn_set_wait_limit(srwn_handle_t h, int64_t clocks);
 int srwn_last_partition(srwn_handle_t h, int32_t* teams, int32_t* ctas_per_team);
-/* 1 if `op` (enum srwn_op) is built for `precision` with this handle's configuration, else 0. */
+/* 1 if `op` (enum srwn_op) is built for `precision` with this handle's configuration, else 0; srwn_last_error() is left
+ * as it was. */
 int srwn_supports(srwn_handle_t h, int32_t op, int32_t precision);
+/* Workspace of one call of `op` over B utterances of T samples at `precision`.  It refuses what that call would refuse of
+ * these arguments, with the same code, and sizes only what the call accepts (weights need not be committed yet).  Every
+ * call of the teacher, the student and their states refuses in this order:
+ *   1. a null required pointer: SRWN_ERR_INVALID;
+ *   2. a handle of the wrong kind for the op: SRWN_ERR_INVALID;
+ *   3. SRWN_BF16: SRWN_ERR_UNSUPPORTED;
+ *   4. a value that is not an enum srwn_precision: SRWN_ERR_INVALID;
+ *   5. SRWN_FP16 where the op's 16-bit kernel does not cover the configuration (srwn_supports == 0):
+ *      SRWN_ERR_UNSUPPORTED;
+ *   6. B < 1, T < 1 or T % pool_stride != 0: SRWN_ERR_INVALID; weights not committed: SRWN_ERR_WEIGHTS;
+ *   7. the batch limit of the fused 16-bit kernel (below): SRWN_ERR_UNSUPPORTED;
+ *   8. a state not reset on this handle for this B and precision: SRWN_ERR_INVALID;
+ *   9. a workspace smaller than this function reports: SRWN_ERR_WORKSPACE. */
 int srwn_workspace_bytes(srwn_handle_t h, int32_t op, int32_t B, int32_t T,
                          int32_t precision, size_t* bytes);
 
@@ -355,9 +369,10 @@ int srwn_encoder_supports(srwn_encoder_t e, int32_t precision);
 int srwn_encoder_workspace_bytes(srwn_encoder_t e, int32_t B, int32_t T, int32_t precision,
                                  size_t* bytes);
 /* encode(inputs) (model.py:250-255): x [B,T] audio -> encoding [B, T/pool_stride, latent].
- * SRWN_FP32: FFMA kernels (parity grade).  SRWN_FP16 / SRWN_BF16: tcgen05 kernels, one launch per
+ * SRWN_FP32: FFMA kernels (parity grade).  SRWN_FP16: tcgen05 kernels, one launch per
  * layer, 16-bit activations between layers (needs encoder_channels = 128, T % 128 == 0,
- * pool_stride % 128 == 0). */
+ * pool_stride % 128 == 0).  srwn_encoder_workspace_bytes refuses the precisions and lengths this
+ * call refuses, with the same code. */
 int srwn_teacher_encode(srwn_encoder_t e, const float* x, float* encoding, int32_t B, int32_t T,
                         int32_t precision, void* workspace, size_t workspace_bytes, void* stream);
 int srwn_encoder_check_async_error(srwn_encoder_t e, int32_t B, int32_t T, int32_t precision,

@@ -237,6 +237,26 @@ extern "C" int srwn_create(const srwn_config_t* cfg, srwn_handle_t* out) {
   return SRWN_OK;
 }
 
+// The abort words [flag, code, a, b] as a status: a fused launch whose pipeline wait expired (code, chunk, cta), or a
+// student stream call whose t0 disagreed with its state (kAbortStreamPosition, state t0, call t0).  `clear` lowers them.
+static int abort_status(const srwn_ctx* c, const char* fused_lead, const char* stream_lead, bool clear) {
+  volatile int* e = c->h_err;
+  if (!e || !e[0]) return SRWN_OK;
+  const int code = e[1], a = e[2], b = e[3];
+  if (clear) { e[0] = 0; e[1] = 0; e[2] = 0; e[3] = 0; }
+  if (code == kAbortStreamPosition)
+    return srwn_fail(SRWN_ERR_CUDA, "%s: the call passed t0=%d but its state was at t0=%d; results of that call are invalid",
+                     stream_lead, b, a);
+  return srwn_fail(SRWN_ERR_CUDA, "%s: pipeline wait timed out (code 0x%x, chunk %d, cta %d); results of that call are invalid",
+                   fused_lead, code, a, b);
+}
+
+// a fused launch or stream call that aborted leaves the abort words raised; every later fused launch and stream call on the
+// handle is refused until srwn_check_async_error has reported it
+int sticky_error(const srwn_ctx* c) {
+  return abort_status(c, "an earlier fused launch aborted", "an earlier call aborted", false);
+}
+
 extern "C" int srwn_destroy(srwn_handle_t h) {
   if (!h) return SRWN_OK;
   gen_state_forget(h);
@@ -328,9 +348,9 @@ extern "C" int srwn_commit_weights(srwn_handle_t h, void* stream) {
 }
 
 // ---- workspace sizing ---------------------------------------------------------------
-struct F32Ws { float *h0, *h1, *skip, *cond, *logits, *scales, *means, *xa, *xb, *z; size_t bytes; };
+struct F32Ws { float *h0, *h1, *skip, *cond, *logits, *scales, *means; size_t bytes; };
 
-static F32Ws carve_f32(const srwn_ctx* c, int op, int B, int T, void* ws, size_t cap, bool need_logits) {
+static F32Ws carve_f32(const srwn_ctx* c, int B, int T, void* ws, size_t cap, bool need_logits) {
   WsCarver w(ws, cap);
   F32Ws r{};
   const size_t n = (size_t)B * T;
@@ -344,21 +364,104 @@ static F32Ws carve_f32(const srwn_ctx* c, int op, int B, int T, void* ws, size_t
   } else {
     r.scales = w.take<float>(n * c->cfg.num_flows);
     r.means = w.take<float>(n * c->cfg.num_flows);
-    r.xa = w.take<float>(n);
-    r.xb = w.take<float>(n);
-    r.z = w.take<float>(n);                       // on-device noise of srwn_student_sample
   }
   r.bytes = w.used;
   return r;
 }
 
-int check_bt(const srwn_ctx* c, int B, int T) {
-  if (B < 1 || T < 1) return srwn_fail(SRWN_ERR_INVALID, "B and T must be positive");
-  if (T % c->cfg.pool_stride != 0)
-    return srwn_fail(SRWN_ERR_INVALID, "T=%d must be a multiple of pool_stride=%d (model.py:183)", T,
-                     c->cfg.pool_stride);
-  if (!c->committed) return srwn_fail(SRWN_ERR_WEIGHTS, "weights not committed (srwn_commit_weights)");
+size_t student_flows_workspace_bytes(const srwn_ctx* h, int precision, int B, int T) {
+  return precision == SRWN_FP16 ? fused_workspace_bytes(h, B, T) : carve_f32(h, B, T, nullptr, 0, false).bytes;
+}
+
+// one-call student forward: the flow chain's buffers, then the flows' own workspace
+struct StudentWs { float *xa, *xb, *z; void* flows; size_t flows_bytes, bytes; };
+
+static StudentWs carve_student(const srwn_ctx* h, int precision, int B, int T, void* ws, size_t cap) {
+  WsCarver w(ws, cap);
+  StudentWs r{};
+  const size_t n = (size_t)B * T;
+  r.xa = w.take<float>(n);
+  r.xb = w.take<float>(n);
+  if (precision == SRWN_FP32) r.z = w.take<float>(n);   // on-device noise of srwn_student_sample (fp16 draws it in flow 0)
+  r.flows_bytes = student_flows_workspace_bytes(h, precision, B, T);
+  r.flows = w.take<uint8_t>(r.flows_bytes);
+  r.bytes = w.used;
+  return r;
+}
+
+int check_workspace(const void* ws, size_t have, size_t need) {
+  if (!ws || have < need) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", need);
   return SRWN_OK;
+}
+
+// ---- which op runs at which precision on which handle ------------------------------------
+// The handle kind of each op (enum srwn_op) and the kernel that runs its SRWN_FP16 form; every op runs in SRWN_FP32.  The
+// fused kernel also limits the batch (fused_check_batch).
+enum Fp16Kernel { FP16_NONE, FP16_FUSED, FP16_AR_MMA };
+struct OpRule { int kind; Fp16Kernel fp16; };
+static const OpRule kOpRules[] = {
+    {SRWN_TEACHER, FP16_FUSED},     // SRWN_OP_TEACHER_LOGITS
+    {SRWN_TEACHER, FP16_FUSED},     // SRWN_OP_TEACHER_NLL
+    {SRWN_TEACHER, FP16_AR_MMA},    // SRWN_OP_TEACHER_GENERATE
+    {SRWN_STUDENT, FP16_FUSED},     // SRWN_OP_STUDENT_FORWARD
+    {SRWN_STUDENT, FP16_NONE},      // SRWN_OP_STUDENT_TRAIN
+    {SRWN_TEACHER, FP16_AR_MMA},    // SRWN_OP_TEACHER_PREFILL
+    {SRWN_STUDENT, FP16_FUSED},     // SRWN_OP_STUDENT_STREAM
+};
+constexpr int kNumOps = sizeof(kOpRules) / sizeof(kOpRules[0]);
+
+// bf16 MMA operands cannot meet the 2e-2 max-abs bound on logits for the 30-layer stack (exact arithmetic on bf16-rounded
+// operands already gives 2.45e-2, tools/bf16_emulation.py; the kernel measured 2.5e-2), so the 16-bit path is fp16
+// (same tensor rate, 8x finer mantissa, measured 3.6e-3) and SRWN_BF16 is refused rather than shipped with a looser bound.
+static int reject_bf16() {
+  return srwn_fail(SRWN_ERR_UNSUPPORTED, "SRWN_BF16 is not offered: bf16 operands miss the 2e-2 logit bound on this stack; use SRWN_FP16");
+}
+
+// The one rule of which op runs at which precision on which handle, in the refusal order of include/srwn.h: the op's handle
+// kind, SRWN_BF16, a value that is no precision, SRWN_FP16 where the op's 16-bit kernel does not cover the configuration
+static int check_op(const srwn_ctx* h, int op, int precision) {
+  if (op < 0 || op >= kNumOps) return srwn_fail(SRWN_ERR_INVALID, "unknown op %d", op);
+  const OpRule& r = kOpRules[op];
+  if (h->cfg.kind != r.kind)
+    return srwn_fail(SRWN_ERR_INVALID, r.kind == SRWN_TEACHER ? "not a teacher handle" : "not a student handle");
+  if (precision == SRWN_BF16) return reject_bf16();
+  if (precision != SRWN_FP32 && precision != SRWN_FP16) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
+  if (precision == SRWN_FP32) return SRWN_OK;
+  switch (r.fp16) {
+    case FP16_FUSED: return fused_check_config(h);
+    case FP16_AR_MMA: return ar_mma_check_config(h);
+    default: return srwn_fail(SRWN_ERR_UNSUPPORTED, "op %d runs in SRWN_FP32 only", op);
+  }
+}
+
+int check_state(const srwn_ctx* h, int op, int B, int precision) {
+  if (int rc = check_op(h, op, precision)) return rc;
+  if (B < 1) return srwn_fail(SRWN_ERR_INVALID, "B must be positive");
+  return SRWN_OK;
+}
+
+// check_op, then B and T, the weights (when `weights`) and the batch limit of the op's 16-bit kernel
+static int check_call(const srwn_ctx* h, int op, int B, int T, int precision, bool weights = true) {
+  if (int rc = check_op(h, op, precision)) return rc;
+  if (B < 1 || T < 1) return srwn_fail(SRWN_ERR_INVALID, "B and T must be positive");
+  if (T % h->cfg.pool_stride != 0)
+    return srwn_fail(SRWN_ERR_INVALID, "T=%d must be a multiple of pool_stride=%d (model.py:183)", T,
+                     h->cfg.pool_stride);
+  if (weights && !h->committed) return srwn_fail(SRWN_ERR_WEIGHTS, "weights not committed (srwn_commit_weights)");
+  if (precision == SRWN_FP16 && kOpRules[op].fp16 == FP16_FUSED) return fused_check_batch(h, B);
+  return SRWN_OK;
+}
+
+// check_op's answer without its message
+extern "C" int srwn_supports(srwn_handle_t h, int32_t op, int32_t precision) {
+  if (!h || op < 0 || op >= kNumOps || h->cfg.kind != kOpRules[op].kind) return 0;
+  if (precision == SRWN_FP32) return 1;
+  if (precision != SRWN_FP16) return 0;
+  switch (kOpRules[op].fp16) {
+    case FP16_FUSED: return fused_supported(h) ? 1 : 0;
+    case FP16_AR_MMA: return ar_mma_supported(h) ? 1 : 0;
+    default: return 0;
+  }
 }
 
 extern "C" int srwn_set_team_size(srwn_handle_t h, int32_t ctas_per_team) {
@@ -412,80 +515,33 @@ extern "C" int srwn_check_async_error(srwn_handle_t h, int32_t op, int32_t B, in
     return SRWN_OK;
   }
   if (op == SRWN_OP_TEACHER_GENERATE) return ar_mma_check_error(h, B, T, workspace, workspace_bytes, (cudaStream_t)stream);
-  return fused_check_error(workspace, workspace_bytes, h, B, T, (cudaStream_t)stream);
+  SRWN_CUDA(cudaStreamSynchronize((cudaStream_t)stream));
+  return abort_status(h, "fused kernel aborted", "student stream call aborted", true);
 }
 
 // The same check without the stream synchronisation, for callers that keep several launches in flight and have already
 // waited (on an event) for the launch they ask about: the abort words of the fused kernels live in pinned host memory.
 extern "C" int srwn_peek_async_error(srwn_handle_t h) {
   if (!h) return srwn_fail(SRWN_ERR_INVALID, "srwn_peek_async_error: null handle");
-  const volatile int* e = h->h_err;
-  if (e && e[0] && e[1] == kAbortStreamPosition) return stream_position_fail(e, "student stream call aborted");
-  if (e && e[0])
-    return srwn_fail(SRWN_ERR_CUDA, "fused kernel aborted: pipeline wait timed out (code 0x%x, chunk %d, cta %d)", e[1], e[2], e[3]);
-  return SRWN_OK;
-}
-
-// bf16 MMA operands cannot meet the 2e-2 max-abs bound on logits for the 30-layer stack (exact arithmetic on bf16-rounded
-// operands already gives 2.45e-2, tools/bf16_emulation.py; the kernel measured 2.5e-2), so the 16-bit path is fp16
-// (same tensor rate, 8x finer mantissa, measured 3.6e-3) and SRWN_BF16 is refused rather than shipped with a looser bound.
-int reject_bf16() {
-  return srwn_fail(SRWN_ERR_UNSUPPORTED, "SRWN_BF16 is not offered: bf16 operands miss the 2e-2 logit bound on this stack; use SRWN_FP16");
-}
-
-extern "C" int srwn_supports(srwn_handle_t h, int32_t op, int32_t precision) {
-  if (!h) return 0;
-  const bool teacher_op = op == SRWN_OP_TEACHER_LOGITS || op == SRWN_OP_TEACHER_NLL || op == SRWN_OP_TEACHER_GENERATE;
-  if (op == SRWN_OP_TEACHER_PREFILL)
-    return h->cfg.kind == SRWN_TEACHER && (precision == SRWN_FP32 || (precision == SRWN_FP16 && ar_mma_supported(h))) ? 1 : 0;
-  if (op == SRWN_OP_STUDENT_TRAIN) return h->cfg.kind == SRWN_STUDENT && precision == SRWN_FP32 ? 1 : 0;
-  if (op == SRWN_OP_STUDENT_STREAM)
-    return h->cfg.kind == SRWN_STUDENT && (precision == SRWN_FP32 || (precision == SRWN_FP16 && fused_supported(h))) ? 1 : 0;
-  if (teacher_op != (h->cfg.kind == SRWN_TEACHER) || op < 0 || op > SRWN_OP_STUDENT_FORWARD) return 0;
-  if (precision == SRWN_FP32) return 1;
-  if (op == SRWN_OP_TEACHER_GENERATE) return precision == SRWN_FP16 && ar_mma_supported(h) ? 1 : 0;
-  if (precision == SRWN_FP16) return fused_supported(h) ? 1 : 0;
-  return 0;   // SRWN_BF16: see reject_bf16
-
+  return abort_status(h, "fused kernel aborted", "student stream call aborted", false);
 }
 
 extern "C" int srwn_workspace_bytes(srwn_handle_t h, int32_t op, int32_t B, int32_t T,
                                     int32_t precision, size_t* bytes) {
   if (!h || !bytes) return srwn_fail(SRWN_ERR_INVALID, "srwn_workspace_bytes: null argument");
-  if (B < 1 || T < 1 || T % h->cfg.pool_stride) return srwn_fail(SRWN_ERR_INVALID, "bad B/T");
+  if (int rc = check_call(h, op, B, T, precision, false)) return rc;
+  const bool fp16 = precision == SRWN_FP16;
   switch (op) {
     case SRWN_OP_TEACHER_LOGITS:
     case SRWN_OP_TEACHER_NLL:
-      if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-      *bytes = precision != SRWN_FP32 ? fused_workspace_bytes(h, op, B, T)
-                                      : carve_f32(h, op, B, T, nullptr, 0, true).bytes;
-      return SRWN_OK;
-    case SRWN_OP_TEACHER_GENERATE:
-      if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-      *bytes = precision == SRWN_FP16 ? ar_mma_workspace_bytes(h, B, T) : ar_workspace_bytes(h, B, T);
-      return SRWN_OK;
-    case SRWN_OP_STUDENT_FORWARD:
-      if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-      *bytes = precision != SRWN_FP32 ? fused_workspace_bytes(h, op, B, T)
-                                      : carve_f32(h, op, B, T, nullptr, 0, false).bytes;
-      return SRWN_OK;
+      *bytes = fp16 ? fused_workspace_bytes(h, B, T) : carve_f32(h, B, T, nullptr, 0, true).bytes; break;
+    case SRWN_OP_TEACHER_GENERATE: *bytes = fp16 ? ar_mma_workspace_bytes(h, B, T) : ar_workspace_bytes(h, B, T); break;
+    case SRWN_OP_STUDENT_FORWARD: *bytes = carve_student(h, precision, B, T, nullptr, 0).bytes; break;
+    case SRWN_OP_STUDENT_TRAIN: *bytes = train_workspace_bytes(h, B, T); break;
+    case SRWN_OP_TEACHER_PREFILL: *bytes = prefill_workspace_bytes(h, B, T, precision); break;
+    case SRWN_OP_STUDENT_STREAM: *bytes = student_stream_workspace_bytes(h, B, T, precision); break;
   }
-  if (op == SRWN_OP_STUDENT_TRAIN) {
-    if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-    *bytes = train_workspace_bytes(h, B, T);
-    return SRWN_OK;
-  }
-  if (op == SRWN_OP_STUDENT_STREAM) {
-    if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-    *bytes = student_stream_workspace_bytes(h, B, T, precision == SRWN_FP16 ? SRWN_FP16 : SRWN_FP32);
-    return SRWN_OK;
-  }
-  if (op == SRWN_OP_TEACHER_PREFILL) {
-    if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-    *bytes = prefill_workspace_bytes(h, B, T, precision == SRWN_FP16 ? SRWN_FP16 : SRWN_FP32);
-    return SRWN_OK;
-  }
-  return srwn_fail(SRWN_ERR_INVALID, "unknown op %d", op);
+  return SRWN_OK;
 }
 
 // ---- teacher --------------------------------------------------------------------------
@@ -501,17 +557,12 @@ extern "C" int srwn_teacher_logits(srwn_handle_t h, const float* x, const float*
                                    int32_t B, int32_t T, int32_t precision, void* workspace,
                                    size_t workspace_bytes, void* stream) {
   if (!h || !x || !enc || !logits) return srwn_fail(SRWN_ERR_INVALID, "srwn_teacher_logits: null argument");
-  if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-  int rc = check_bt(h, B, T);
-  if (rc) return rc;
-  if (precision == SRWN_BF16) return reject_bf16();
+  if (int rc = check_call(h, SRWN_OP_TEACHER_LOGITS, B, T, precision)) return rc;
   if (precision == SRWN_FP16)
     return run_teacher_fused(h, x, enc, nullptr, nullptr, nullptr, logits, B, T,
                              workspace, workspace_bytes, (cudaStream_t)stream);
-  if (precision != SRWN_FP32) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
-  F32Ws w = carve_f32(h, SRWN_OP_TEACHER_LOGITS, B, T, workspace, workspace_bytes, false);
-  if (!workspace || w.bytes > workspace_bytes)
-    return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  F32Ws w = carve_f32(h, B, T, workspace, workspace_bytes, false);
+  if (int rc = check_workspace(workspace, workspace_bytes, w.bytes)) return rc;
   return teacher_f32(h, x, enc, logits, B, T, w, (cudaStream_t)stream);
 }
 
@@ -520,17 +571,13 @@ extern "C" int srwn_teacher_nll(srwn_handle_t h, const float* x_in, const float*
                                 float* logits_out, int32_t B, int32_t T, int32_t precision,
                                 void* workspace, size_t workspace_bytes, void* stream) {
   if (!h || !x_in || !enc || !x_scored) return srwn_fail(SRWN_ERR_INVALID, "srwn_teacher_nll: null argument");
-  if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-  int rc = check_bt(h, B, T);
+  int rc = check_call(h, SRWN_OP_TEACHER_NLL, B, T, precision);
   if (rc) return rc;
-  if (precision == SRWN_BF16) return reject_bf16();
   if (precision == SRWN_FP16)
     return run_teacher_fused(h, x_in, enc, x_scored, nll_out, nll_sum, logits_out, B, T,
                              workspace, workspace_bytes, (cudaStream_t)stream);
-  if (precision != SRWN_FP32) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
-  F32Ws w = carve_f32(h, SRWN_OP_TEACHER_NLL, B, T, workspace, workspace_bytes, logits_out == nullptr);
-  if (!workspace || w.bytes > workspace_bytes)
-    return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  F32Ws w = carve_f32(h, B, T, workspace, workspace_bytes, logits_out == nullptr);
+  if ((rc = check_workspace(workspace, workspace_bytes, w.bytes))) return rc;
   float* lg = logits_out ? logits_out : w.logits;
   rc = teacher_f32(h, x_in, enc, lg, B, T, w, (cudaStream_t)stream);
   if (rc) return rc;
@@ -542,14 +589,10 @@ extern "C" int srwn_teacher_generate(srwn_handle_t h, const float* enc, const fl
                                      int32_t T, int32_t precision, void* workspace, size_t workspace_bytes,
                                      void* stream) {
   if (!h || !enc || !u1 || !u2 || !x_out) return srwn_fail(SRWN_ERR_INVALID, "srwn_teacher_generate: null argument");
-  if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-  int rc = check_bt(h, B, T);
-  if (rc) return rc;
+  if (int rc = check_call(h, SRWN_OP_TEACHER_GENERATE, B, T, precision)) return rc;
   if (precision == SRWN_FP16)
     return run_ar_mma(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes, (cudaStream_t)stream, nullptr,
                       nullptr, 0);
-  if (precision != SRWN_FP32)
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "generation runs in fp32 (FFMA kernel) or fp16 (tensor-core kernel)");
   return run_ar_generate(h, enc, u1, u2, x_out, logits_out, B, T, workspace, workspace_bytes,
                          (cudaStream_t)stream, nullptr, nullptr, 0);
 }
@@ -562,7 +605,8 @@ extern "C" int srwn_teacher_generate_resume(srwn_handle_t h, void* state, const 
   if (!h || !state || !enc || !u1 || !u2 || !x_out)
     return srwn_fail(SRWN_ERR_INVALID, "srwn_teacher_generate_resume: null argument");
   GenState s;
-  int rc = gen_state_open(h, state, B, T, precision, &s);
+  int rc = check_call(h, SRWN_OP_TEACHER_GENERATE, B, T, precision);
+  if (!rc) rc = gen_state_open(h, state, B, precision, &s);
   if (rc) return rc;
   if (n_prefix < 0 || n_prefix > T || (n_prefix > 0 && !x_prefix))
     return srwn_fail(SRWN_ERR_INVALID, "n_prefix=%d must be in [0, T=%d], with x_prefix given when > 0", n_prefix, T);
@@ -579,29 +623,24 @@ extern "C" int srwn_generate_state_prefill(srwn_handle_t h, void* state, const f
                                            void* stream) {
   if (!h || !state || !x || !enc) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_prefill: null argument");
   GenState s;
-  int rc = gen_state_open(h, state, B, n, precision, &s);   // n % P == 0 keeps t0 on a frame boundary for later calls
+  int rc = check_call(h, SRWN_OP_TEACHER_PREFILL, B, n, precision);   // n % P == 0 keeps t0 on a frame boundary for later calls
+  if (!rc) rc = gen_state_open(h, state, B, precision, &s);
   if (rc) return rc;
   return run_prefill(h, s, x, enc, B, n, precision, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // ---- student --------------------------------------------------------------------------
 // z supplied (noise.on == 0) or drawn on the device (student.py:104); z_out optionally receives the draws
-static int student_forward_impl(srwn_handle_t h, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out,
-                                float* s_tot, float* mu_tot, float* x_last, int32_t B, int32_t T,
-                                int32_t precision, void* workspace, size_t workspace_bytes, cudaStream_t st) {
-  if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-  int rc = check_bt(h, B, T);
+static int student_forward(srwn_handle_t h, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out,
+                           float* s_tot, float* mu_tot, float* x_last, int32_t B, int32_t T, int32_t precision,
+                           void* workspace, size_t workspace_bytes, cudaStream_t st) {
+  int rc = check_call(h, SRWN_OP_STUDENT_FORWARD, B, T, precision);
   if (rc) return rc;
-  if (precision == SRWN_BF16) return reject_bf16();
-  if (precision == SRWN_FP16)
-    return run_student_fused(h, z, noise, z_out, enc, out, s_tot, mu_tot, x_last, B, T, workspace, workspace_bytes, st);
-  if (precision != SRWN_FP32) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
-  F32Ws w = carve_f32(h, SRWN_OP_STUDENT_FORWARD, B, T, workspace, workspace_bytes, false);
-  if (!workspace || w.bytes > workspace_bytes)
-    return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  const StudentWs w = carve_student(h, precision, B, T, workspace, workspace_bytes);
+  if ((rc = check_workspace(workspace, workspace_bytes, w.bytes))) return rc;
   const size_t n = (size_t)B * T;
   const int F = h->cfg.num_flows;
-  if (noise.on) {                                     // the layer-at-a-time path reads the noise as a tensor
+  if (noise.on && precision == SRWN_FP32) {           // the layer-at-a-time path reads the noise as a tensor
     float* zbuf = z_out ? z_out : w.z;
     rc = run_random_fill(zbuf, (int64_t)n, noise.seed, noise.stream, 1, 0.f, 1.f, st);
     if (rc) return rc;
@@ -610,15 +649,17 @@ static int student_forward_impl(srwn_handle_t h, const float* z, NoiseSpec noise
   float* x[17] = {const_cast<float*>(z)};            // flow f reads x[f] and writes x[f + 1] (num_flows <= 16, srwn_create)
   for (int f = 0; f < F; f++) x[f + 1] = (f == F - 1 && x_last) ? x_last : ((f & 1) ? w.xb : w.xa);
   const float *scales = nullptr, *means = nullptr;
-  rc = run_student_flows_f32(h, x, enc, B, T, 0, workspace, workspace_bytes, &scales, &means, st);
+  rc = run_student_flows(h, precision, x, noise, enc, B, T, 0, w.flows, w.flows_bytes, &scales, &means, st);
   if (rc) return rc;
   return run_flow_compose(z, noise, z_out, scales, means, F, out, s_tot, mu_tot, (int64_t)n, st);
 }
 
-int run_student_flows_f32(srwn_ctx* h, float* const* x, const float* enc, int B, int T, int t_out, void* ws, size_t ws_bytes,
-                          const float** scales, const float** means, cudaStream_t st) {
-  F32Ws w = carve_f32(h, SRWN_OP_STUDENT_FORWARD, B, T, ws, ws_bytes, false);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+int run_student_flows(srwn_ctx* h, int precision, float* const* x, NoiseSpec noise, const float* enc, int B, int T, int t_out,
+                      void* ws, size_t ws_bytes, const float** scales, const float** means, cudaStream_t st) {
+  if (precision == SRWN_FP16)
+    return run_student_flows_fused(h, x, noise, enc, B, T, t_out, ws, ws_bytes, scales, means, st);
+  F32Ws w = carve_f32(h, B, T, ws, ws_bytes, false);
+  if (int rc = check_workspace(ws, ws_bytes, w.bytes)) return rc;
   const size_t n = (size_t)B * T;
   for (int f = 0; f < h->cfg.num_flows; f++) {       // model.py:509-513, strictly sequential
     float* hf = nullptr;
@@ -631,25 +672,21 @@ int run_student_flows_f32(srwn_ctx* h, float* const* x, const float* enc, int B,
   return SRWN_OK;
 }
 
-size_t student_f32_workspace_bytes(const srwn_ctx* h, int B, int T) {
-  return carve_f32(h, SRWN_OP_STUDENT_FORWARD, B, T, nullptr, 0, false).bytes;
-}
-
 extern "C" int srwn_student_forward(srwn_handle_t h, const float* z, const float* enc, float* out,
                                     float* s_tot, float* mu_tot, float* x_last, int32_t B, int32_t T,
                                     int32_t precision, void* workspace, size_t workspace_bytes,
                                     void* stream) {
   if (!h || !z || !enc || !out) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_forward: null argument");
-  return student_forward_impl(h, z, NoiseSpec{0, 0, 0}, nullptr, enc, out, s_tot, mu_tot, x_last, B, T, precision,
-                              workspace, workspace_bytes, (cudaStream_t)stream);
+  return student_forward(h, z, NoiseSpec{0, 0, 0}, nullptr, enc, out, s_tot, mu_tot, x_last, B, T, precision,
+                         workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 extern "C" int srwn_student_sample(srwn_handle_t h, uint64_t seed, uint64_t stream_id, const float* enc, float* out,
                                    float* s_tot, float* mu_tot, float* x_last, float* z_out, int32_t B, int32_t T,
                                    int32_t precision, void* workspace, size_t workspace_bytes, void* stream) {
   if (!h || !enc || !out) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_sample: null argument");
-  return student_forward_impl(h, nullptr, NoiseSpec{seed, stream_id, 1}, z_out, enc, out, s_tot, mu_tot, x_last, B, T,
-                              precision, workspace, workspace_bytes, (cudaStream_t)stream);
+  return student_forward(h, nullptr, NoiseSpec{seed, stream_id, 1}, z_out, enc, out, s_tot, mu_tot, x_last, B, T,
+                         precision, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
 // ---- student synthesis in chunks through a carried flow state (state format and kernels: student_stream.cu) ----------
@@ -658,11 +695,7 @@ extern "C" int srwn_student_forward_resume(srwn_handle_t h, void* state, int64_t
                                            float* x_last, float* z_out, int32_t B, int32_t S, int32_t precision,
                                            void* workspace, size_t workspace_bytes, void* stream) {
   if (!h || !state || !enc || !out) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_forward_resume: null argument");
-  if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-  if (precision == SRWN_BF16) return reject_bf16();
-  if (precision != SRWN_FP32 && precision != SRWN_FP16) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
-  int rc = check_bt(h, B, S);
-  if (rc) return rc;
+  if (int rc = check_call(h, SRWN_OP_STUDENT_STREAM, B, S, precision)) return rc;
   if (t0 < 0 || t0 % h->cfg.pool_stride)
     return srwn_fail(SRWN_ERR_INVALID, "t0=%lld must be a non-negative multiple of pool_stride=%d", (long long)t0,
                      h->cfg.pool_stride);
@@ -695,9 +728,7 @@ extern "C" int srwn_student_forward_train(srwn_handle_t h, const float* z, const
                                           float* s_tot, float* mu_tot, int32_t B, int32_t T, void* workspace,
                                           size_t workspace_bytes, void* stream) {
   if (!h || !z || !enc || !out) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_forward_train: null argument");
-  if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-  int rc = check_bt(h, B, T);
-  if (rc) return rc;
+  if (int rc = check_call(h, SRWN_OP_STUDENT_TRAIN, B, T, SRWN_FP32)) return rc;
   return run_student_forward_train(h, z, enc, out, s_tot, mu_tot, B, T, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 
@@ -705,10 +736,7 @@ extern "C" int srwn_student_backward(srwn_handle_t h, const float* z, const floa
                                      const float* d_s_extra, float* grads, int32_t B, int32_t T, void* workspace,
                                      size_t workspace_bytes, void* stream) {
   if (!h || !z || !enc || !d_pre || !grads) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_backward: null argument");
-  if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-  if (h->cfg.num_flows > 16) return srwn_fail(SRWN_ERR_UNSUPPORTED, "backward supports up to 16 flows");
-  int rc = check_bt(h, B, T);
-  if (rc) return rc;
+  if (int rc = check_call(h, SRWN_OP_STUDENT_TRAIN, B, T, SRWN_FP32)) return rc;
   return run_student_backward(h, z, enc, d_pre, d_s_extra, grads, B, T, workspace, workspace_bytes, (cudaStream_t)stream);
 }
 

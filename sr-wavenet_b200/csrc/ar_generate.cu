@@ -208,8 +208,7 @@ size_t ar_workspace_bytes(const srwn_ctx* c, int B, int T) {
 int run_ar_generate(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
                     float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenState* rs,
                     const float* x_prefix, int n_prefix) {
-  if (!ws || ws_bytes < ar_workspace_bytes(c, B, T))
-    return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", ar_workspace_bytes(c, B, T));
+  if (int rc = check_workspace(ws, ws_bytes, ar_workspace_bytes(c, B, T))) return rc;
   WsCarver w(ws, ws_bytes);
   const int frames = T / c->cfg.pool_stride;
   const size_t queue_bytes = gen_queue_bytes(c, B, SRWN_FP32);

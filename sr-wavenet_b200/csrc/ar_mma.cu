@@ -593,6 +593,12 @@ bool ar_mma_supported(const srwn_ctx* c) {
          c->cfg.num_mixtures <= 8;
 }
 
+int ar_mma_check_config(const srwn_ctx* c) {
+  if (ar_mma_supported(c)) return SRWN_OK;
+  return srwn_fail(SRWN_ERR_UNSUPPORTED, "the fp16 generation kernel covers 3..%d or 20..%d layers and 1..6 mixtures; got %d layers, "
+                   "%d mixtures", armma::kMaxL - 16, armma::kMaxL, c->cfg.n_layers, c->cfg.num_mixtures);
+}
+
 static size_t ar_mma_image_bytes(const srwn_ctx* c) {
   return (size_t)c->cfg.n_layers * armma::kChainLayerBytes + (size_t)(c->cfg.n_layers + 5) * armma::kItemBytes + 352 * 4;
 }
@@ -666,10 +672,8 @@ size_t ar_mma_workspace_bytes(const srwn_ctx* c, int B, int T) { return carve_ar
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
                float* logits_out, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st, const GenState* rs,
                const float* x_prefix, int n_prefix) {
-  if (!ar_mma_supported(c) || !c->d_ar_packed)
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "fp16 generation kernel supports up to %d layers and 6 mixtures", armma::kMaxL);
   ArMmaWs w = carve_ar_mma(c, B, T, ws, ws_bytes);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  if (int rc = check_workspace(ws, ws_bytes, w.bytes)) return rc;
   const int L = c->cfg.n_layers, frames = T / c->cfg.pool_stride;
   if (!rs) SRWN_CUDA(cudaMemsetAsync(w.queues, 0, gen_queue_bytes(c, B, SRWN_FP16), st));   // zero padding of ops.py:9
   const GenState s = rs ? *rs : GenState{nullptr, nullptr, w.queues};   // one call from silence: the zeroed workspace queues

@@ -279,10 +279,8 @@ size_t prefill_workspace_bytes(const srwn_ctx* c, int B, int n, int precision) {
 int run_prefill(srwn_ctx* c, const GenState& s, const float* x, const float* enc, int B, int n, int precision, void* ws,
                 size_t ws_bytes, cudaStream_t st) {
   const bool fp16 = precision == SRWN_FP16;
-  if (fp16 && (!ar_mma_supported(c) || !c->d_ar_packed))
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "fp16 prefill needs the tensor-core generation kernel's configuration");
   const PrefillWs w = carve_prefill(c, B, n, precision, ws);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  if (int rc = check_workspace(ws, ws_bytes, w.bytes)) return rc;
   const int L = c->cfg.n_layers, P = c->cfg.pool_stride, C = c->cfg.cond_channels, sum_d = c->sum_dilation;
   const int Bp = fp16 ? (B + 7) / 8 * 8 : B;
   std::vector<int> D(L + 1, 0), qoff(L, 0);           // D[l] = d_l + ... + d_{L-1}

@@ -143,8 +143,12 @@ struct GenState {
 
 // ---- kernels and entry points implemented across translation units ------------------
 // api.cu
-int check_bt(const srwn_ctx* c, int B, int T);
 const float* srwn_host_weights(srwn_ctx* c);
+// the arguments of a state call for B utterances (srwn_generate_state_*: op SRWN_OP_TEACHER_GENERATE,
+// srwn_student_state_*: op SRWN_OP_STUDENT_STREAM): the op's handle kind and precision, then B
+int check_state(const srwn_ctx* h, int op, int B, int precision);
+int check_workspace(const void* ws, size_t have, size_t need);   // SRWN_ERR_WORKSPACE unless ws holds `need` bytes
+int sticky_error(const srwn_ctx* c);     // SRWN_ERR_CUDA while the handle's abort words are raised (no synchronisation)
 // stack_f32.cu
 __global__ void k_cond(const float* __restrict__ enc, const float* __restrict__ cond_k,
                        const float* __restrict__ cond_b, float* __restrict__ cond,
@@ -204,6 +208,7 @@ int run_adam(srwn_ctx* c, const float* grads, float* m, float* v, float* scratch
              float eps, int step, cudaStream_t st);
 // ar_mma.cu
 bool ar_mma_supported(const srwn_ctx* c);
+int ar_mma_check_config(const srwn_ctx* c);   // SRWN_ERR_UNSUPPORTED, naming what the kernel covers, where !ar_mma_supported
 int ar_mma_pack_weights(srwn_ctx* c, cudaStream_t st);
 size_t ar_mma_workspace_bytes(const srwn_ctx* c, int B, int T);
 int run_ar_mma(srwn_ctx* c, const float* enc, const float* u1, const float* u2, float* x_out,
@@ -214,15 +219,14 @@ int ar_mma_check_error(const srwn_ctx* c, int B, int T, void* ws, size_t ws_byte
 size_t prefill_workspace_bytes(const srwn_ctx* c, int B, int n, int precision);
 int run_prefill(srwn_ctx* c, const GenState& s, const float* x, const float* enc, int B, int n, int precision, void* ws,
                 size_t ws_bytes, cudaStream_t st);
-// api.cu: the F flows of the fp32 path over [B][T] rows: flow f reads x[f] and writes x[f+1] for rows t >= t_out;
-// *scales and *means ([F][B][T], in the workspace) receive every flow's affine parameters
-int run_student_flows_f32(srwn_ctx* h, float* const* x, const float* enc, int B, int T, int t_out, void* ws, size_t ws_bytes,
-                          const float** scales, const float** means, cudaStream_t st);
-size_t student_f32_workspace_bytes(const srwn_ctx* h, int B, int T);
-int reject_bf16();
+// api.cu: the F flows of the student over [B][T] rows in `precision`: flow f reads x[f] and writes x[f+1] for rows
+// t >= t_out; *scales and *means ([F][B][T], in the workspace) receive every flow's affine parameters.  Noise drawn in
+// place (fp16 only, flow 0) needs t_out == 0.
+int run_student_flows(srwn_ctx* h, int precision, float* const* x, NoiseSpec noise, const float* enc, int B, int T, int t_out,
+                      void* ws, size_t ws_bytes, const float** scales, const float** means, cudaStream_t st);
+size_t student_flows_workspace_bytes(const srwn_ctx* h, int precision, int B, int T);
 // student_stream.cu: chunked synthesis through a carried flow state (srwn_student_forward_resume)
 constexpr int kAbortStreamPosition = 0x5000000;     // abort code: the call's t0 disagreed with its state's
-int stream_position_fail(const volatile int* e, const char* lead);
 size_t student_stream_workspace_bytes(const srwn_ctx* h, int B, int S, int precision);
 int run_student_stream(srwn_ctx* h, void* state, long long t0, const float* z, NoiseSpec noise, const float* enc, float* out,
                        float* s_tot, float* mu_tot, float* x_last, float* z_out, int B, int S, int precision, void* ws,
@@ -233,22 +237,17 @@ __global__ void k_fold_bias(const float* __restrict__ cond, const float* __restr
                             const float* __restrict__ res_b, float* __restrict__ cb, int L);
 }
 bool fused_supported(const srwn_ctx* c);
+int fused_check_config(const srwn_ctx* c);         // SRWN_ERR_UNSUPPORTED, naming what the kernel covers, where !fused_supported
 int fused_check_batch(const srwn_ctx* c, int B);   // SRWN_ERR_UNSUPPORTED past sm_count * 8 utterances (srwn.h)
 size_t fused_packed_bytes(const srwn_ctx* c);
 int fused_pack_weights(srwn_ctx* c, cudaStream_t st);
-size_t fused_workspace_bytes(const srwn_ctx* c, int op, int B, int T);
+size_t fused_workspace_bytes(const srwn_ctx* c, int B, int T);
 int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc,
                       const float* x_scored, float* nll_out, float* nll_sum,
                       float* logits_out, int B, int T, void* ws, size_t ws_bytes,
                       cudaStream_t st);
-int run_student_fused(srwn_ctx* c, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out,
-                      float* s_tot, float* mu_tot, float* x_last, int B, int T,
-                      void* ws, size_t ws_bytes, cudaStream_t st);
-// the flows of run_student_fused as the stream call runs them: flow f reads x[f] and writes x[f+1] for rows t >= t_out
-// (the work partition starts every utterance at row 0 and its outputs at t_out); noise must be off when t_out > 0
+// run_student_flows in fp16 (the work partition starts every utterance at row 0 and its outputs at t_out)
 int run_student_flows_fused(srwn_ctx* c, float* const* x, NoiseSpec noise, const float* enc, int B, int T, int t_out,
                             void* ws, size_t ws_bytes, const float** scales, const float** means, cudaStream_t st);
-int fused_check_error(void* ws, size_t ws_bytes, const srwn_ctx* c, int B, int T, cudaStream_t st);
-int sticky_error(const srwn_ctx* c);     // SRWN_ERR_CUDA while the handle's abort words are raised (no synchronisation)
 size_t fused_partition_bytes(const srwn_ctx* c);
 void fused_last_partition(const srwn_ctx* c, int* teams, int* G);

@@ -661,8 +661,18 @@ static size_t enc_ws_bytes(const srwn_encoder* e, int B, int T, int precision) {
   return w.used;
 }
 
+// what srwn_teacher_encode refuses of a precision (srwn_encoder_workspace_bytes refuses the same)
+static int check_encode_precision(srwn_encoder_t e, int T, int precision) {
+  if (!srwn_encoder_supports(e, precision))
+    return srwn_fail(SRWN_ERR_UNSUPPORTED, "encoder precision %d needs encoder_channels=128, pool_stride %% 128 == 0, latent <= 64", precision);
+  if (precision != SRWN_FP32 && T % enc::kTile != 0)
+    return srwn_fail(SRWN_ERR_UNSUPPORTED, "the encoder's tensor-core path needs T %% 128 == 0 (got %d); use SRWN_FP32", T);
+  return SRWN_OK;
+}
+
 extern "C" int srwn_encoder_workspace_bytes(srwn_encoder_t e, int32_t B, int32_t T, int32_t precision, size_t* bytes) {
   if (!e || !bytes || B < 1 || T < 1) return srwn_fail(SRWN_ERR_INVALID, "srwn_encoder_workspace_bytes: bad argument");
+  if (int rc = check_encode_precision(e, T, precision)) return rc;
   *bytes = enc_ws_bytes(e, B, T, precision);
   return SRWN_OK;
 }
@@ -682,12 +692,8 @@ extern "C" int srwn_teacher_encode(srwn_encoder_t e, const float* x, float* enc_
   if (!e || !x || !enc_out) return srwn_fail(SRWN_ERR_INVALID, "srwn_teacher_encode: null argument");
   if (!e->committed) return srwn_fail(SRWN_ERR_WEIGHTS, "srwn_teacher_encode: weights not committed");
   if (B < 1 || T < e->P) return srwn_fail(SRWN_ERR_INVALID, "srwn_teacher_encode: need B >= 1 and T >= pool_stride");
-  if (!srwn_encoder_supports(e, precision))
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "srwn_teacher_encode: precision %d needs encoder_channels=128, pool_stride %% 128 == 0, latent <= 64", precision);
-  if (precision != SRWN_FP32 && T % enc::kTile != 0)
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "srwn_teacher_encode: the tensor-core path needs T %% 128 == 0 (got %d); use SRWN_FP32", T);
-  if (workspace_bytes < enc_ws_bytes(e, B, T, precision) || !workspace)
-    return srwn_fail(SRWN_ERR_WORKSPACE, "srwn_teacher_encode: workspace too small");
+  if (int rc = check_encode_precision(e, T, precision)) return rc;
+  if (int rc = check_workspace(workspace, workspace_bytes, enc_ws_bytes(e, B, T, precision))) return rc;
   cudaStream_t st = (cudaStream_t)stream;
   const int L = e->L, E = e->E, S = e->S, C = e->C, P = e->P, frames = T / P;
   const size_t rows = (size_t)B * T;

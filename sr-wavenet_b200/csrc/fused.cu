@@ -948,6 +948,12 @@ bool fused_supported(const srwn_ctx* c) {
   return true;
 }
 
+int fused_check_config(const srwn_ctx* c) {
+  if (fused_supported(c)) return SRWN_OK;
+  return srwn_fail(SRWN_ERR_UNSUPPORTED, "the fused 16-bit kernel needs at most %d layers, dilations <= %d and pool_stride %% %d == 0",
+                   kMaxLayers, kHalo, kTile);
+}
+
 // one fused launch gives every utterance a segment of its own: at most sm_count teams of kMaxSeg segments (partition.h)
 int fused_check_batch(const srwn_ctx* c, int B) {
   if (B > fused_max_batch(c->sm_count))
@@ -1026,7 +1032,7 @@ struct FusedWs {
 #ifdef SRWN_TUNING
   long long* trace;
 #endif
-  float *scales, *means, *xa, *xb;
+  float *scales, *means;
   size_t bytes;
 };
 
@@ -1046,8 +1052,6 @@ static FusedWs carve_fused(const srwn_ctx* c, int B, int T, void* ws, size_t cap
   if (c->cfg.kind == SRWN_STUDENT) {
     r.scales = w.take<float>(n * c->cfg.num_flows);
     r.means = w.take<float>(n * c->cfg.num_flows);
-    r.xa = w.take<float>(n);
-    r.xb = w.take<float>(n);
   }
   r.bytes = w.used;
   return r;
@@ -1059,7 +1063,7 @@ size_t fused_partition_bytes(const srwn_ctx* c) {
   return grid * kMaxSeg * sizeof(Seg) + grid * sizeof(int);
 }
 
-size_t fused_workspace_bytes(const srwn_ctx* c, int op, int B, int T) {
+size_t fused_workspace_bytes(const srwn_ctx* c, int B, int T) {
   return carve_fused(c, B, T, nullptr, 0).bytes;
 }
 
@@ -1077,21 +1081,9 @@ static int launch_fused(srwn_ctx* c, const Params& p, int grid, cudaStream_t st)
   return SRWN_OK;
 }
 
-// a fused launch that aborted (a bounded wait expired) leaves its error words in pinned host memory; every later call on
-// the handle is refused until srwn_check_async_error has reported it
-int sticky_error(const srwn_ctx* c) {
-  const volatile int* e = c->h_err;
-  if (e && e[0] && e[1] == kAbortStreamPosition) return stream_position_fail(e, "an earlier call aborted");
-  if (e && e[0])
-    return srwn_fail(SRWN_ERR_CUDA, "an earlier fused launch aborted: pipeline wait timed out (code 0x%x, chunk %d, cta %d); "
-                     "results of that call are invalid", e[1], e[2], e[3]);
-  return SRWN_OK;
-}
-
 static int prepare(srwn_ctx* c, int stack, const float* enc, int B, int T, int out0, const FusedWs& w, Params* p,
                    int* grid, bool first, cudaStream_t st) {
   const int L = c->cfg.n_layers, P = c->cfg.pool_stride, frames = T / P;
-  const float* sw = stack_w(c, stack);
   int rc = sticky_error(c);
   if (rc) return rc;
   // conditioning of every stack and the ring flags of every launch are prepared by the first call of a sequence (the
@@ -1106,7 +1098,6 @@ static int prepare(srwn_ctx* c, int stack, const float* enc, int B, int T, int o
     SRWN_LAUNCH_CHECK();
     SRWN_CUDA(cudaMemsetAsync(w.flags, 0, flag_stride * nst * sizeof(uint32_t), st));
   }
-  (void)sw;
   const size_t seg_bytes = (size_t)c->sm_count * kMaxSeg * sizeof(Seg), n_bytes = (size_t)c->sm_count * sizeof(int);
   if (first && (c->part_B != B || c->part_T != T || c->part_out0 != out0 || c->part_team_req != c->team_size)) {
     // the work partition depends on (B, T, out0) and the team size only: built once, kept on the device next to the handle.
@@ -1146,13 +1137,12 @@ static int prepare(srwn_ctx* c, int stack, const float* enc, int B, int T, int o
 int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc, const float* x_scored,
                       float* nll_out, float* nll_sum, float* logits_out, int B, int T,
                       void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fused_supported(c)) return srwn_fail(SRWN_ERR_UNSUPPORTED, "fused 16-bit path needs dilations <= %d, layers <= %d, pool_stride %% 128 == 0", kHalo, kMaxLayers);
-  if (int rc = fused_check_batch(c, B)) return rc;
   FusedWs w = carve_fused(c, B, T, ws, ws_bytes);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  int rc = check_workspace(ws, ws_bytes, w.bytes);
+  if (rc) return rc;
   Params p;
   int grid = 0;
-  int rc = prepare(c, 0, enc, B, T, 0, w, &p, &grid, true, st);
+  rc = prepare(c, 0, enc, B, T, 0, w, &p, &grid, true, st);
   if (rc) return rc;
   p.x_in = x_in; p.x_scored = x_scored; p.logits_out = logits_out; p.nll_out = nll_out;
   p.nll_partial = (x_scored && nll_sum) ? w.partial : nullptr;
@@ -1170,10 +1160,8 @@ int run_teacher_fused(srwn_ctx* c, const float* x_in, const float* enc, const fl
 
 int run_student_flows_fused(srwn_ctx* c, float* const* x, NoiseSpec noise, const float* enc, int B, int T, int t_out,
                             void* ws, size_t ws_bytes, const float** scales, const float** means, cudaStream_t st) {
-  if (!fused_supported(c)) return srwn_fail(SRWN_ERR_UNSUPPORTED, "fused 16-bit path needs dilations <= %d, layers <= %d, pool_stride %% 128 == 0", kHalo, kMaxLayers);
-  if (int rc = fused_check_batch(c, B)) return rc;
   FusedWs w = carve_fused(c, B, T, ws, ws_bytes);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  if (int rc = check_workspace(ws, ws_bytes, w.bytes)) return rc;
   const size_t n = (size_t)B * T;
   const int F = c->cfg.num_flows;
   int grid = 0;
@@ -1188,38 +1176,6 @@ int run_student_flows_fused(srwn_ctx* c, float* const* x, NoiseSpec noise, const
     if (rc) return rc;
   }
   *scales = w.scales; *means = w.means;
-  return SRWN_OK;
-}
-
-int run_student_fused(srwn_ctx* c, const float* z, NoiseSpec noise, float* z_out, const float* enc, float* out, float* s_tot,
-                      float* mu_tot, float* x_last, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
-  if (!fused_supported(c)) return srwn_fail(SRWN_ERR_UNSUPPORTED, "fused 16-bit path needs dilations <= %d, layers <= %d, pool_stride %% 128 == 0", kHalo, kMaxLayers);
-  FusedWs w = carve_fused(c, B, T, ws, ws_bytes);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
-  const int F = c->cfg.num_flows;
-  float* x[17] = {const_cast<float*>(z)};          // flow f reads x[f] and writes x[f + 1] (num_flows <= 16, srwn_create)
-  for (int f = 0; f < F; f++) x[f + 1] = (f == F - 1 && x_last) ? x_last : ((f & 1) ? w.xb : w.xa);
-  const float *scales = nullptr, *means = nullptr;
-  int rc = run_student_flows_fused(c, x, noise, enc, B, T, 0, ws, ws_bytes, &scales, &means, st);
-  if (rc) return rc;
-  return run_flow_compose(z, noise, z_out, scales, means, F, out, s_tot, mu_tot, (int64_t)B * T, st);
-}
-
-// reads (and clears) the abort words of the fused launches issued so far; synchronises the stream
-int fused_check_error(void* ws, size_t ws_bytes, const srwn_ctx* c, int B, int T, cudaStream_t st) {
-  (void)ws; (void)ws_bytes; (void)B; (void)T;
-  SRWN_CUDA(cudaStreamSynchronize(st));
-  volatile int* e = c->h_err;
-  if (e && e[0] && e[1] == kAbortStreamPosition) {
-    const int rc = stream_position_fail(e, "student stream call aborted");
-    e[0] = 0; e[1] = 0; e[2] = 0; e[3] = 0;
-    return rc;
-  }
-  if (e && e[0]) {
-    const int code = e[1], chunk = e[2], cta = e[3];
-    e[0] = 0; e[1] = 0; e[2] = 0; e[3] = 0;
-    return srwn_fail(SRWN_ERR_CUDA, "fused kernel aborted: pipeline wait timed out (code 0x%x, chunk %d, cta %d)", code, chunk, cta);
-  }
   return SRWN_OK;
 }
 

@@ -33,20 +33,9 @@ void state_signature(const srwn_ctx* c, int B, int precision, int32_t* sig) {
 struct StateOwner { const srwn_ctx* h; std::vector<int32_t> sig; };
 std::mutex g_states_mu;
 std::map<const void*, StateOwner> g_states;
+}  // namespace
 
-int check_state_args(const srwn_ctx* h, int B, int precision, const char* fn) {
-  if (!h) return srwn_fail(SRWN_ERR_INVALID, "%s: null handle", fn);
-  if (h->cfg.kind != SRWN_TEACHER) return srwn_fail(SRWN_ERR_INVALID, "not a teacher handle");
-  if (B < 1) return srwn_fail(SRWN_ERR_INVALID, "%s: B must be positive", fn);
-  if (precision == SRWN_FP16 && !ar_mma_supported(h))
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "fp16 generation kernel does not cover this configuration");
-  if (precision != SRWN_FP32 && precision != SRWN_FP16)
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "generation runs in fp32 (FFMA kernel) or fp16 (tensor-core kernel)");
-  return SRWN_OK;
-}
-
-// The owner check, then the state's parts (the layout of B utterances in `precision`).
-int open_owned(const srwn_ctx* h, void* state, int B, int precision, GenState* s) {
+int gen_state_open(const srwn_ctx* h, void* state, int B, int precision, GenState* s) {
   int32_t sig[6];
   state_signature(h, B, precision, sig);
   const int rc = state_owner_check(h, state, sig, 6, "srwn_generate_state_reset");
@@ -58,7 +47,6 @@ int open_owned(const srwn_ctx* h, void* state, int B, int precision, GenState* s
   s->queues = base + lay.queues;
   return SRWN_OK;
 }
-}  // namespace
 
 void state_owner_record(const srwn_ctx* h, const void* state, const int32_t* sig, int n) {
   std::lock_guard<std::mutex> lk(g_states_mu);
@@ -91,26 +79,16 @@ void gen_state_forget(const srwn_ctx* h) {
   for (auto it = g_states.begin(); it != g_states.end();) it = it->second.h == h ? g_states.erase(it) : std::next(it);
 }
 
-int gen_state_open(const srwn_ctx* h, void* state, int B, int T, int precision, GenState* s) {
-  int rc = check_state_args(h, B, precision, "generation state");
-  if (rc) return rc;
-  rc = check_bt(h, B, T);
-  if (rc) return rc;
-  return open_owned(h, state, B, precision, s);
-}
-
 extern "C" int srwn_generate_state_bytes(srwn_handle_t h, int32_t B, int32_t precision, size_t* bytes) {
-  if (!bytes) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_bytes: null argument");
-  int rc = check_state_args(h, B, precision, "srwn_generate_state_bytes");
-  if (rc) return rc;
+  if (!h || !bytes) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_bytes: null argument");
+  if (int rc = check_state(h, SRWN_OP_TEACHER_GENERATE, B, precision)) return rc;
   *bytes = gen_state_layout(h, B, precision).bytes;
   return SRWN_OK;
 }
 
 extern "C" int srwn_generate_state_reset(srwn_handle_t h, void* state, int32_t B, int32_t precision, void* stream) {
-  if (!state) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_reset: null state");
-  int rc = check_state_args(h, B, precision, "srwn_generate_state_reset");
-  if (rc) return rc;
+  if (!h || !state) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_reset: null argument");
+  if (int rc = check_state(h, SRWN_OP_TEACHER_GENERATE, B, precision)) return rc;
   GenStateHeader hdr{};
   state_signature(h, B, precision, hdr.sig);
   const cudaStream_t st = (cudaStream_t)stream;
@@ -175,18 +153,17 @@ __global__ void __launch_bounds__(kSpliceThreads) k_gen_state_splice(const __gri
 extern "C" int srwn_generate_state_splice(srwn_handle_t h, void* dst, int32_t dst_B, const int32_t* dst_rows,
                                           const void* src, int32_t src_B, const int32_t* src_rows, int32_t n,
                                           int32_t precision, void* stream) {
-  if (!dst || !src) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_splice: null state");
-  int rc = check_state_args(h, dst_B, precision, "srwn_generate_state_splice");
-  if (rc) return rc;
-  rc = check_state_args(h, src_B, precision, "srwn_generate_state_splice");
+  if (!h || !dst || !src) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_splice: null argument");
+  int rc = check_state(h, SRWN_OP_TEACHER_GENERATE, dst_B, precision);
+  if (!rc) rc = check_state(h, SRWN_OP_TEACHER_GENERATE, src_B, precision);
   if (rc) return rc;
   if (src == dst) return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_splice: src and dst are the same state");
   if (n < 0 || (n > 0 && (!dst_rows || !src_rows)))
     return srwn_fail(SRWN_ERR_INVALID, "srwn_generate_state_splice: n=%d must be >= 0, with both row arrays when > 0", n);
   GenState d, s;
-  rc = open_owned(h, dst, dst_B, precision, &d);
+  rc = gen_state_open(h, dst, dst_B, precision, &d);
   if (rc) return rc;
-  rc = open_owned(h, const_cast<void*>(src), src_B, precision, &s);
+  rc = gen_state_open(h, const_cast<void*>(src), src_B, precision, &s);
   if (rc) return rc;
   std::vector<uint8_t> named(dst_B, 0);
   for (int i = 0; i < n; i++) {

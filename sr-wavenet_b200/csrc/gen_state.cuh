@@ -20,9 +20,8 @@ constexpr int kGenSlotBytes = 512;    // fp16 queues: one slot of a group
 static_assert(kGenGroup == 8, "gen_f16_offset splits the utterance index with shifts");
 
 size_t gen_queue_bytes(const srwn_ctx* c, int B, int precision);
-// Checks the arguments of a call on `state` (the C entry points' order: handle, B, precision, then check_bt(B, T)), then
-// that the state was last reset on h for B and precision, without touching the device; fills *s with the state's parts.
-int gen_state_open(const srwn_ctx* h, void* state, int B, int T, int precision, GenState* s);
+// Checks that `state` was last reset on h for B and precision, without touching the device; fills *s with the state's parts.
+int gen_state_open(const srwn_ctx* h, void* state, int B, int precision, GenState* s);
 void gen_state_forget(const srwn_ctx* h);    // srwn_destroy: h's states (generation and synthesis) are no longer valid
 // host registry of state owners: the handle and signature a state buffer was last reset with
 void state_owner_record(const srwn_ctx* h, const void* state, const int32_t* sig, int n);

@@ -211,7 +211,7 @@ int run_stft_power(const float* x, float* power, int B, int T, int N, int step, 
   int lg, F;
   if (int rc = stft_shape(B, T, N, step, &lg, &F, "srwn_stft_power")) return rc;
   StftWs w = carve_stft(B, N, F, ws);
-  if (cap < w.bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "srwn_stft_power: workspace too small (%zu < %zu)", cap, w.bytes);
+  if (int rc = check_workspace(ws, cap, w.bytes)) return rc;
   const int K = N / 2 + 1, thr = N / 2 < 32 ? 32 : (N / 2 > 256 ? 256 : N / 2);
   const size_t smem = (size_t)(2 * N + N / 2) * sizeof(float2);
   if (smem > 48 * 1024) SRWN_CUDA(cudaFuncSetAttribute(stftk::k_frames, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -228,7 +228,7 @@ int run_stft_power_loss(const float* truth, const float* out, float gamma, doubl
   int lg, F;
   if (int rc = stft_shape(B, T, N, step, &lg, &F, "srwn_stft_power_loss")) return rc;
   StftWs w = carve_stft(B, N, F, ws);
-  if (cap < w.bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "srwn_stft_power_loss: workspace too small (%zu < %zu)", cap, w.bytes);
+  if (int rc = check_workspace(ws, cap, w.bytes)) return rc;
   const int K = N / 2 + 1, thr = N / 2 < 32 ? 32 : (N / 2 > 256 ? 256 : N / 2);
   const size_t smem = (size_t)(2 * N + N / 2) * sizeof(float2);
   if (smem > 48 * 1024) {

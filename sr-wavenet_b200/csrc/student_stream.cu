@@ -46,17 +46,6 @@ void signature(const srwn_ctx* c, int B, int precision, int32_t* sig) {
   memcpy(sig, v, sizeof(v));
 }
 
-int check_state_args(const srwn_ctx* h, int B, int precision, const char* fn) {
-  if (!h) return srwn_fail(SRWN_ERR_INVALID, "%s: null handle", fn);
-  if (h->cfg.kind != SRWN_STUDENT) return srwn_fail(SRWN_ERR_INVALID, "not a student handle");
-  if (B < 1) return srwn_fail(SRWN_ERR_INVALID, "%s: B must be positive", fn);
-  if (precision == SRWN_BF16) return reject_bf16();
-  if (precision != SRWN_FP32 && precision != SRWN_FP16) return srwn_fail(SRWN_ERR_INVALID, "unknown precision %d", precision);
-  if (precision == SRWN_FP16 && !fused_supported(h))
-    return srwn_fail(SRWN_ERR_UNSUPPORTED, "the fused fp16 flow kernel does not cover this configuration");
-  return SRWN_OK;
-}
-
 // one call: the flows' input buffers [B][N] (x[F] = the last flow's output), the frames of the buffer, the state
 struct StreamArgs {
   float* x[17];               // num_flows <= 16 (srwn_create)
@@ -160,35 +149,27 @@ StreamWs carve(const srwn_ctx* c, int B, int S, int precision, void* ws, size_t 
   for (int f = 0; f <= c->cfg.num_flows; f++) r.x[f] = w.take<float>((size_t)B * Nmax);
   r.ebuf = w.take<float>((size_t)B * (Nmax / c->cfg.pool_stride) * c->cfg.cond_channels);
   r.valid = w.take<int>(1);
-  r.inner = ws ? static_cast<uint8_t*>(ws) + w.used : nullptr;
-  r.inner_bytes = precision == SRWN_FP16 ? fused_workspace_bytes(c, SRWN_OP_STUDENT_FORWARD, B, Nmax)
-                                         : student_f32_workspace_bytes(c, B, Nmax);
-  r.bytes = w.used + r.inner_bytes;
+  r.inner_bytes = student_flows_workspace_bytes(c, precision, B, Nmax);
+  r.inner = w.take<uint8_t>(r.inner_bytes);
+  r.bytes = w.used;
   return r;
 }
 }  // namespace
-
-int stream_position_fail(const volatile int* e, const char* lead) {
-  return srwn_fail(SRWN_ERR_CUDA, "%s: the call passed t0=%d but its state was at t0=%d; results of that call are invalid",
-                   lead, e[3], e[2]);
-}
 
 size_t student_stream_workspace_bytes(const srwn_ctx* h, int B, int S, int precision) {
   return carve(h, B, S, precision, nullptr, 0).bytes;
 }
 
 extern "C" int srwn_student_state_bytes(srwn_handle_t h, int32_t B, int32_t precision, size_t* bytes) {
-  if (!bytes) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_state_bytes: null argument");
-  const int rc = check_state_args(h, B, precision, "srwn_student_state_bytes");
-  if (rc) return rc;
+  if (!h || !bytes) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_state_bytes: null argument");
+  if (int rc = check_state(h, SRWN_OP_STUDENT_STREAM, B, precision)) return rc;
   *bytes = layout(h, B).bytes;
   return SRWN_OK;
 }
 
 extern "C" int srwn_student_state_reset(srwn_handle_t h, void* state, int32_t B, int32_t precision, void* stream) {
-  if (!state) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_state_reset: null state");
-  const int rc = check_state_args(h, B, precision, "srwn_student_state_reset");
-  if (rc) return rc;
+  if (!h || !state) return srwn_fail(SRWN_ERR_INVALID, "srwn_student_state_reset: null argument");
+  if (int rc = check_state(h, SRWN_OP_STUDENT_STREAM, B, precision)) return rc;
   StreamHeader hdr{};
   signature(h, B, precision, hdr.sig);
   const cudaStream_t st = (cudaStream_t)stream;
@@ -202,15 +183,12 @@ extern "C" int srwn_student_state_reset(srwn_handle_t h, void* state, int32_t B,
 int run_student_stream(srwn_ctx* h, void* state, long long t0, const float* z, NoiseSpec noise, const float* enc, float* out,
                        float* s_tot, float* mu_tot, float* x_last, float* z_out, int B, int S, int precision, void* ws,
                        size_t ws_bytes, cudaStream_t st) {
-  int rc = check_state_args(h, B, precision, "srwn_student_forward_resume");
-  if (rc) return rc;
-  if (precision == SRWN_FP16 && (rc = fused_check_batch(h, B))) return rc;
   int32_t sig[kSigLen];
   signature(h, B, precision, sig);
-  rc = state_owner_check(h, state, sig, kSigLen, "srwn_student_state_reset");
+  int rc = state_owner_check(h, state, sig, kSigLen, "srwn_student_state_reset");
   if (rc) return rc;
   const StreamWs w = carve(h, B, S, precision, ws, ws_bytes);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  if ((rc = check_workspace(ws, ws_bytes, w.bytes))) return rc;
   rc = sticky_error(h);
   if (rc) return rc;
   StreamArgs a;
@@ -230,9 +208,7 @@ int run_student_stream(srwn_ctx* h, void* state, long long t0, const float* z, N
   k_stream_assemble<<<(unsigned)((n_in + kThreads - 1) / kThreads), kThreads, 0, st>>>(a, z, noise, enc);
   SRWN_LAUNCH_CHECK();
   const float *scales = nullptr, *means = nullptr;
-  rc = precision == SRWN_FP16
-           ? run_student_flows_fused(h, a.x, NoiseSpec{0, 0, 0}, a.ebuf, B, a.N, a.Heff, w.inner, w.inner_bytes, &scales, &means, st)
-           : run_student_flows_f32(h, a.x, a.ebuf, B, a.N, a.Heff, w.inner, w.inner_bytes, &scales, &means, st);
+  rc = run_student_flows(h, precision, a.x, NoiseSpec{0, 0, 0}, a.ebuf, B, a.N, a.Heff, w.inner, w.inner_bytes, &scales, &means, st);
   if (rc) return rc;
   const int64_t n_out = (int64_t)B * S;
   k_stream_compose<<<(unsigned)((n_out + kThreads - 1) / kThreads), kThreads, 0, st>>>(a, scales, means, out, s_tot, mu_tot,

@@ -336,7 +336,7 @@ size_t train_workspace_bytes(const srwn_ctx* c, int B, int T) { return carve_tra
 int run_student_forward_train(srwn_ctx* c, const float* z, const float* enc, float* out, float* s_tot,
                               float* mu_tot, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
   TrainWs w = carve_train(c, B, T, ws, ws_bytes);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  if (int rc = check_workspace(ws, ws_bytes, w.bytes)) return rc;
   const size_t n = (size_t)B * T;
   const int F = c->cfg.num_flows, L = c->cfg.n_layers;
   const float* xin = z;
@@ -357,7 +357,7 @@ int run_student_backward(srwn_ctx* c, const float* z, const float* enc, const fl
                          float* grads, int B, int T, void* ws, size_t ws_bytes, cudaStream_t st) {
   using namespace train;
   TrainWs w = carve_train(c, B, T, ws, ws_bytes);
-  if (!ws || w.bytes > ws_bytes) return srwn_fail(SRWN_ERR_WORKSPACE, "workspace too small: need %zu bytes", w.bytes);
+  if (int rc = check_workspace(ws, ws_bytes, w.bytes)) return rc;
   const size_t n = (size_t)B * T;
   const int F = c->cfg.num_flows, L = c->cfg.n_layers, P = c->cfg.pool_stride, frames = T / P, C = c->cfg.cond_channels;
   const int BF = B * frames;
